@@ -159,6 +159,18 @@ def ncu_traffic(kernel, units):
     return float(ent["dram_bytes"]) * units / float(ent["units"])
 
 
+def dump_outputs(out_dir, loss, model):
+    """Write what a training step hands its caller, as float32 .npy files: `loss` (this rank's shard loss), and per parameter
+    `param.<path>` (the values after the Adam update) and `grad.<path>` (the gradient the update applied), with the
+    parameter path's '/' written as '.'.  About 2.6 MB at CFG's shapes."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().cpu().numpy()}
+    for prefix, table in (("param", model.param_dict()), ("grad", model.grad_dict())):
+        arrays.update(("%s.%s" % (prefix, k.replace("/", ".")), v) for k, v in table.items())
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -213,6 +225,9 @@ def run_gpu(args):
         sampler.start()
     # ---- value: inputs resident in HBM ----
     ms, launches = timed(lambda: trainer.step(*resident, global_count=gcount), args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        # before the legs below train the same model further
+        dump_outputs(args.dump_outputs, trainer.loss_buf, model)
     ms_per_step = ms / args.steps
     value = args.pairs / (ms_per_step * 1e-3)
     # ---- e2e legs: host inputs, H2D inside the timed region, loss read back ----
@@ -584,7 +599,14 @@ def main():
     ap.add_argument("--no-fp32", action="store_true", help="skip the extra fp32-exact measurement")
     ap.add_argument("--sample", type=int, default=128, help="--impl reference: pairs per CPU step")
     ap.add_argument("--no-config-a", action="store_true", help="--impl reference: skip the config-A CPU figures")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, parameters and gradients of the last timed step to DIR/<name>.npy, so that two "
+                         "builds run with the same arguments can be compared array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         return run_reference(args)
     run_gpu(args)

@@ -25,6 +25,12 @@ def test_reference_arm_prints_the_contract_line_without_loading_the_product():
     assert line["e2e"] == dict(value=line["value"], unit="pairs/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0)
 
 
+def test_steps_below_one_are_rejected():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
 def test_other_ranks_of_the_reference_arm_exit_without_work():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], capture_output=True,

@@ -1,5 +1,6 @@
 import sys, os
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/gcn-bmp_b200")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "gcn-bmp_b200"))
 import torch, numpy as np, ctypes as C, gcnbmp
 from gcnbmp import _capi as K
 lib = K.lib

@@ -1,5 +1,5 @@
 import os, sys
-ROOT = "/root/repo"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "gcn-bmp_b200")):
     sys.path.insert(0, p)
 import numpy as np, torch, gcnbmp
