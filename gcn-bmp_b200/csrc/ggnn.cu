@@ -557,8 +557,7 @@ static int check_common(int mb, int N, int H, int E, int T, int mode, int nmax =
 using namespace bmp;
 
 int bmp_ggnn_forward_tc(const bmp_ggnn_fwd_t *a, void *stream);    // ggnn_tc.cu
-int bmp_ggnn_backward_tc(const bmp_ggnn_bwd_t *a, void *stream);   // ggnn_tc_bwd.cu
-int bmp_ggnn_backward_v2(const bmp_ggnn_bwd_t *a, void *stream);   // ggnn_tc_bwd.cu (bf16 panel stash)
+int bmp_ggnn_backward_tc(const bmp_ggnn_bwd_t *a, void *stream);   // ggnn_tc_bwd.cu (bf16 panel stash)
 // ggnn_x3.cu: BMP_MODE_F32 with the contractions on tcgen05 (bf16 hi/lo split, fp32-grade), when a workspace is given
 bool bmp_ggnn_x3_usable(int mb, int N, int H, int E, int T, const void *ws, size_t ws_bytes, const void *state_in, bool inference);
 int bmp_ggnn_forward_x3(const bmp_ggnn_fwd_t *a, void *stream);
@@ -622,12 +621,17 @@ extern "C" int bmp_ggnn_forward(const bmp_ggnn_fwd_t *a, void *stream) {
 }
 
 extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
-    if (a && a->stash2) {
-        if (a->mode != BMP_MODE_BF16 || (a->hidden != 64 && a->hidden != 128) || a->n_edge != 4 || a->state_in || !a->adj || !a->dHs) {
-            set_error("bmp_ggnn_backward: the panel stash needs BMP_MODE_BF16, hidden 64/128, 4 bond types and no external state");
+    if (a && (a->stash2 || a->mode == BMP_MODE_BF16)) {
+        if (!a->stash2 || a->mode != BMP_MODE_BF16) {
+            set_error("bmp_ggnn_backward: BMP_MODE_BF16 trains on the bf16 panel stash: stash2 (written by the forward) is required, "
+                      "and only in that mode");
             return BMP_EINVAL;
         }
-        return bmp_ggnn_backward_v2(a, stream);
+        if ((a->hidden != 64 && a->hidden != 128) || a->n_edge != 4 || a->state_in || !a->adj || !a->dHs) {
+            set_error("bmp_ggnn_backward: the panel stash needs hidden 64/128, 4 bond types and no external state");
+            return BMP_EINVAL;
+        }
+        return bmp_ggnn_backward_tc(a, stream);
     }
     if (!a || !a->adj || !a->Hs || !a->Ms || !a->Gs || !a->Ps || !a->dHs || !a->RSs) {
         set_error("bmp_ggnn_backward: null argument");
@@ -638,20 +642,16 @@ extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
     int rc = check_common(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, BMP_MODE_F32, x3_data ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
     if (rc) return rc;
     const int H = a->hidden, T = a->n_steps, E = a->n_edge;
-    // BMP_MODE_BF16: parameter-gradient contractions on tcgen05 (bias column sums fused in)
-    const bool tcw = a->mode == BMP_MODE_BF16 && (H == 64 || H == 128);
     const bool tc3 = a->mode == BMP_MODE_F32 && (H == 64 || H == 128 || H == 256);
     auto WG = [&](const float *A_, int lda, const float *B_, int ldb, float *C_, int ldc, long r_, float *db, int dbs) -> int {
-        if (tcw) return bmp_wgrad_tc(A_, lda, B_, ldb, C_, ldc, r_, H, H, db, dbs, stream);
-        // BMP_MODE_F32: the same tensor-core contraction with a bf16 hi/lo split (three UMMAs per product): fp32-grade accuracy
+        // parameter-gradient contractions on tcgen05 with a bf16 hi/lo split (three UMMAs per product): fp32-grade accuracy
         if (tc3) return bmp_wgrad_tc3(A_, lda, B_, ldb, C_, ldc, r_, H, H, db, dbs, stream);
         int e_ = bmp_wgrad(A_, lda, B_, ldb, C_, ldc, r_, H, H, stream);
         if (!e_ && db) e_ = bmp_colsum(A_, lda, db, dbs, r_, H, stream);
         return e_;
     };
-    const bool tc_data = tcw && E == 4 && !a->state_in;      // data part on tcgen05 as well
-    if (a->adj_u8 && !tc_data) { set_error("bmp_ggnn_backward: a byte adjacency needs the tcgen05 path"); return BMP_EINVAL; }
-    if (!tc_data && H > 128 && a->state_in) {
+    if (a->adj_u8) { set_error("bmp_ggnn_backward: a byte adjacency needs BMP_MODE_BF16"); return BMP_EINVAL; }
+    if (H > 128 && a->state_in) {
         set_error("bmp_ggnn_backward: an external GRU state needs hidden <= 128 (hidden=%d)", H);
         return BMP_ESHAPE;
     }
@@ -666,9 +666,7 @@ extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
         set_error("bmp_ggnn_backward: stash buffers must be 16-byte aligned");
         return BMP_EINVAL;
     }
-    if (tc_data) {
-        if ((rc = bmp_ggnn_backward_tc(a, stream))) return rc;
-    } else if (x3_data) {
+    if (x3_data) {
         if ((rc = bmp_ggnn_backward_x3(a, stream))) return rc;
     } else {
         size_t smem = bwd_smem_bytes(H);

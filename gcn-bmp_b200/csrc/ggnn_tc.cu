@@ -20,12 +20,11 @@
 namespace bmp {
 namespace tc {
 
-// LEAN = no fp32 per-step stash (inference, or the bf16 panel stash): no transposition staging, deeper weight ring
-template <int H, bool LEAN>
+template <int H>
 struct Cfg {
     static constexpr int KP = H / 64;
     static constexpr int TILE_BYTES = H * 128;            // weight tile: H rows (n) x 64 bf16 (k)
-    static constexpr int STAGES = (H == 128 && !LEAN) ? 2 : 4;
+    static constexpr int STAGES = 4;
     static constexpr int T_MSG = 4 * KP, T_GATE = 2 * KP, T_U = KP;
     static constexpr int TILES_STATEFUL = T_MSG + 3 * T_GATE + T_U;
     static constexpr int TILES_STATELESS = T_MSG + 2 * T_GATE;
@@ -34,8 +33,7 @@ struct Cfg {
     static constexpr int OFF_ADJ = OFF_H + KP * PANEL_BYTES;
     static constexpr int OFF_AH = OFF_ADJ + 8 * ADJ_TILE_BYTES;
     static constexpr int OFF_W = OFF_AH + 2 * KP * PANEL_BYTES;
-    static constexpr int OFF_STG = OFF_W + STAGES * TILE_BYTES;   // H/8 warps x 2 KB transposition staging
-    static constexpr int OFF_BAR = OFF_STG + (LEAN ? 0 : (H / 8) * 2048);
+    static constexpr int OFF_BAR = OFF_W + STAGES * TILE_BYTES;
     static constexpr int SMEM_BYTES = OFF_BAR + 256 + 1024;   // + alignment slack
 };
 
@@ -49,17 +47,17 @@ struct Args {
     const float *bias3[BMP_MAX_STEPS];     // [b_r | b_z | b_h] (U biases folded for stateful steps)
     const float *msg_b[BMP_MAX_STEPS];     // (H*4) as in the reference: b[c*4+e]
     int stateful[BMP_MAX_STEPS];
-    float *h_out, *h0_out, *Hs, *Ms, *Gs, *RSs;
+    float *h_out, *h0_out;
+    float *Hs;                   // optional (T+1, mb*N, H): h_t of every step (an output, not read back by the backward)
     long long *dbg;              // optional phase timestamps of CTA 0 (tools/tc_timeline.py)
-    Stash2 st;                   // bf16 panel stash (use2 != 0): replaces the fp32 Hs/Ms/Gs/RSs stores
-    int use2;
+    Stash2 st;                   // bf16 panel stash of the training forward (V2)
     const int32_t *midx;         // optional (mb,): atoms / adj are a drug table, molecule b = table row midx[b]
 };
 
-template <int H, bool V2, bool LEAN>
+// V2: training, dumps the bf16 panel stash; otherwise inference
+template <int H, bool V2>
 __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args a) {
-    static_assert(LEAN || !V2, "the panel stash implies LEAN");
-    using C = Cfg<H, LEAN>;
+    using C = Cfg<H>;
     constexpr int KP = C::KP;
     constexpr int EPW = H / 8;          // epilogue warps: 4 TMEM lane quarters x (H / 32) column groups
     constexpr int NE = 32 * EPW;
@@ -216,9 +214,10 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
         const uint32_t t_lane = tmem + ((uint32_t)(32 * q) << 16);
         const int molslot = row >> 6, atom = row & 63;
         float hreg[NC];
-        // transposition staging for coalesced fp32 stores: a dedicated block, or (LEAN) the AH buffer, which is idle at
-        // the only two moments LEAN stores anything (tile start: h_0; tile end: h_T)
-        float *stg = reinterpret_cast<float *>(smem + (LEAN ? C::OFF_AH : C::OFF_STG) + warp * 2048);
+        // transposition staging for coalesced fp32 stores: the AH buffer, idle at the only moments anything is stored -- tile
+        // start (h_0) and E4 (the new state): after B_ZH every MMA of the step has read AH and its panel dumps have left it
+        // (bulk_wait_read), and no warp writes it again before all of them have arrived on B_HREADY
+        float *stg = reinterpret_cast<float *>(smem + C::OFF_AH + warp * 2048);
         uint32_t it = 0;
 #define TSP(i) do { if (a.dbg && blockIdx.x == 0 && tid == 0 && it < 64) a.dbg[it * 16 + 8 + (i)] = clock64(); } while (0)
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -250,12 +249,6 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
                     *reinterpret_cast<uint4 *>(base + ((size_t)((cc >> 3) + g) * NE + tid) * 16) = pk;
                 }
             };
-            auto store_rows16 = [&](float *base, long ld, int col0, const float *vals) {
-                warp_store_rows<16>(stg, vals, lane, [&](int r) -> float * {
-                    const long g = wrow(r);
-                    return g >= 0 ? base + g * ld + col0 : nullptr;
-                });
-            };
             // ---- h_0: embedding gather (or h_in) -> fp32 registers (requested first: the latency overlaps the staging)
             {
                 const float *src = nullptr;
@@ -281,12 +274,8 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
             {
 #pragma unroll
                 for (int cc = 0; cc < NC; cc += 32) {
-                    if (LEAN) {
-                        if (a.h0_out) store_rows(a.h0_out, H, colbase + cc, &hreg[cc]);
-                    } else {
-                        if (a.h0_out) store_rows(a.h0_out, H, colbase + cc, &hreg[cc]);
-                        if (a.Hs) store_rows(a.Hs, H, colbase + cc, &hreg[cc]);
-                    }
+                    if (a.h0_out) store_rows(a.h0_out, H, colbase + cc, &hreg[cc]);
+                    if (V2 && a.Hs) store_rows(a.Hs, H, colbase + cc, &hreg[cc]);
                 }
             }
             auto store_h_operand = [&](int t_next) {
@@ -403,7 +392,6 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
                             float4 b4 = __ldg(reinterpret_cast<const float4 *>(mb_) + colbase + cc + x);
                             m[x] = __uint_as_float(v[x]) + deg[0] * b4.x + deg[1] * b4.y + deg[2] * b4.z + deg[3] * b4.w;
                         }
-                        if (!LEAN && a.Ms) store_rows(a.Ms + (long)t * rows_total * H, H, colbase + cc, m);
 #pragma unroll
                         for (int g = 0; g < 4; ++g) {
                             const int kk = colbase + cc + 8 * g;
@@ -437,10 +425,6 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
                             }
                         }
                         if (V2) store_native16(t, 2, cc, r);
-                        if (!LEAN && a.Gs) {
-                            store_rows16(a.Gs + (long)t * rows_total * 3 * H, 3 * H, colbase + cc, r);
-                            store_rows16(a.RSs + (long)t * rows_total * H, H, colbase + cc, rs);
-                        }
 #pragma unroll
                         for (int g = 0; g < 2; ++g) {
                             const int kk = colbase + cc + 8 * g;
@@ -448,15 +432,6 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
                                                   pack_bf16(rs[8 * g + 4], rs[8 * g + 5]), pack_bf16(rs[8 * g + 6], rs[8 * g + 7]));
                             *reinterpret_cast<uint4 *>(smem + C::OFF_AH + (KP + (kk >> 6)) * PANEL_BYTES + sw128(row, kk & 63)) = pk;
                         }
-                    }
-                } else if (!LEAN && a.Gs) {   // r / r*h slots of a stateless step: zeros (merged wgrad contractions stay exact)
-                    float zero[32];
-#pragma unroll
-                    for (int x = 0; x < 32; ++x) zero[x] = 0.f;
-#pragma unroll
-                    for (int cc = 0; cc < NC; cc += 32) {
-                        store_rows(a.Gs + (long)t * rows_total * 3 * H, 3 * H, colbase + cc, zero);
-                        store_rows(a.RSs + (long)t * rows_total * H, H, colbase + cc, zero);
                     }
                 }
                 warp_arrive(BAR(B_RSREADY), lane);
@@ -488,19 +463,11 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_kernel(const Args
                         store_native16(t, 0, cc, z);
                         store_native16(t, 1, cc, hb);
                     }
-                    if (!LEAN && a.Gs) {
-                        store_rows16(a.Gs + (long)t * rows_total * 3 * H, 3 * H, H + colbase + cc, z);
-                        store_rows16(a.Gs + (long)t * rows_total * 3 * H, 3 * H, 2 * H + colbase + cc, hb);
-                    }
                 }
 #pragma unroll
                 for (int cc = 0; cc < NC; cc += 32) {
-                    if (LEAN) {
-                        if (t == a.T - 1 && a.h_out) store_rows(a.h_out, H, colbase + cc, &hreg[cc]);
-                    } else {
-                        if (a.Hs) store_rows(a.Hs + (long)(t + 1) * rows_total * H, H, colbase + cc, &hreg[cc]);
-                        if (t == a.T - 1 && a.h_out) store_rows(a.h_out, H, colbase + cc, &hreg[cc]);
-                    }
+                    if (V2 && a.Hs) store_rows(a.Hs + (long)(t + 1) * rows_total * H, H, colbase + cc, &hreg[cc]);
+                    if (t == a.T - 1 && a.h_out) store_rows(a.h_out, H, colbase + cc, &hreg[cc]);
                 }
                 TSF(7);
                 if (t + 1 < a.T) {
@@ -605,11 +572,15 @@ int bmp_ggnn_forward_tc(const bmp_ggnn_fwd_t *a, void *stream) {
         return BMP_ESHAPE;
     }
     if (a->state_in) { set_error("BMP_MODE_BF16: an external GRU state is not supported (state must equal h)"); return BMP_ESHAPE; }
+    if (a->Ms || a->Gs || a->RSs || (a->Hs && !a->stash2)) {
+        set_error("BMP_MODE_BF16: the training tape is the bf16 panel stash (stash2); Ms / Gs / RSs must be NULL and Hs needs stash2");
+        return BMP_EINVAL;
+    }
     if (!a->tc_workspace || a->tc_workspace_bytes < bmp_ggnn_tc_workspace_bytes(H, T)) {
         set_error("BMP_MODE_BF16: tc_workspace of >= %zu bytes required", bmp_ggnn_tc_workspace_bytes(H, T));
         return BMP_EINVAL;
     }
-    if (!aligned16({a->h_in, a->embed_W, a->adj, a->h_out, a->h0_out, a->Hs, a->Ms, a->Gs, a->RSs, a->tc_workspace})) {
+    if (!aligned16({a->h_in, a->embed_W, a->adj, a->h_out, a->h0_out, a->Hs, a->tc_workspace})) {
         set_error("BMP_MODE_BF16: buffers must be 16-byte aligned");
         return BMP_EINVAL;
     }
@@ -617,12 +588,11 @@ int bmp_ggnn_forward_tc(const bmp_ggnn_fwd_t *a, void *stream) {
     tc::Args k = {};
     k.mb = a->mb; k.N = a->n_atoms; k.T = T; k.n_types = a->n_atom_types;
     k.atoms = a->atoms; k.embed_W = a->embed_W; k.h_in = a->h_in; k.adj = a->adj; k.adj_u8 = a->adj_u8;
-    k.h_out = a->h_out; k.h0_out = a->h0_out; k.Hs = a->Hs; k.Ms = a->Ms; k.Gs = a->Gs; k.RSs = a->RSs;
+    k.h_out = a->h_out; k.h0_out = a->h0_out; k.Hs = a->Hs;
     k.dbg = g_tc_dbg_fwd;
     k.midx = a->mol_index;
     if (a->mol_index && !a->atoms) { set_error("BMP_MODE_BF16: mol_index needs atom ids (a drug table), not h_in"); return BMP_EINVAL; }
-    k.use2 = a->stash2 != nullptr;
-    if (k.use2) k.st.carve(a->stash2, (a->mb + 1) / 2, H, T);
+    if (a->stash2) k.st.carve(a->stash2, (a->mb + 1) / 2, H, T);
     uint8_t *ws = (uint8_t *)(((uintptr_t)a->tc_workspace + 255) & ~(uintptr_t)255);
     const size_t ib = tc::image_bytes(H);
     int n_img = 0;
@@ -654,16 +624,14 @@ int bmp_ggnn_forward_tc(const bmp_ggnn_fwd_t *a, void *stream) {
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int n_tiles = (a->mb + 1) / 2;
     const int grid = n_tiles < sms ? n_tiles : sms;
-    const bool lean = !a->Hs && !a->Ms && !a->Gs && !a->RSs;
-    if (k.use2 && !lean) { set_error("BMP_MODE_BF16: the panel stash excludes the fp32 per-step stash"); return BMP_EINVAL; }
-#define LAUNCH_FWD(HH, VV, LL)                                                                                           \
+#define LAUNCH_FWD(HH, VV)                                                                                               \
     do {                                                                                                                 \
-        cudaFuncSetAttribute(tc::ggnn_tc_kernel<HH, VV, LL>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::Cfg<HH, LL>::SMEM_BYTES); \
-        tc::ggnn_tc_kernel<HH, VV, LL><<<grid, 32 * (HH / 8 + 2), tc::Cfg<HH, LL>::SMEM_BYTES, st>>>(k);                      \
+        cudaFuncSetAttribute(tc::ggnn_tc_kernel<HH, VV>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::Cfg<HH>::SMEM_BYTES); \
+        tc::ggnn_tc_kernel<HH, VV><<<grid, 32 * (HH / 8 + 2), tc::Cfg<HH>::SMEM_BYTES, st>>>(k);                          \
     } while (0)
     ProfScope prof(BMP_PROF_GGNN_FWD, st);
-    if (H == 64) { if (k.use2) LAUNCH_FWD(64, true, true); else if (lean) LAUNCH_FWD(64, false, true); else LAUNCH_FWD(64, false, false); }
-    else { if (k.use2) LAUNCH_FWD(128, true, true); else if (lean) LAUNCH_FWD(128, false, true); else LAUNCH_FWD(128, false, false); }
+    if (H == 64) { if (a->stash2) LAUNCH_FWD(64, true); else LAUNCH_FWD(64, false); }
+    else { if (a->stash2) LAUNCH_FWD(128, true); else LAUNCH_FWD(128, false); }
 #undef LAUNCH_FWD
     count_launch();
     return check_launch("ggnn_tc_kernel");

@@ -1,15 +1,15 @@
 // ggnn_tc_bwd.cu -- backward (data part) of the fused GGNN encoder on tcgen05 (BMP_MODE_BF16).
 //
 // Mirror of ggnn_tc.cu: persistent CTA per SM, a tile = two padded molecules = 128 rows, steps walked in
-// reverse over the forward stash.  The running gradient dL/dh_{t+1} lives in fp32 registers of the
+// reverse over the forward's bf16 panel stash.  The running gradient dL/dh_{t+1} lives in fp32 registers of the
 // epilogue threads; per step (SURVEY.md Appendix B, state == step input so U_r/U_z fold into W_r/W_z):
-//   phase A   dz, dhbar -> delta_z, delta_h (bf16 operand panels, fp32 into Gs for the wgrad contractions)
+//   phase A   dz, dhbar -> delta_z, delta_h (bf16 operand panels, dumped to the stash for the wgrad contractions)
 //   MMA-q     q = delta_h U                      -> phase B: delta_r = q*s*r(1-r), ds += q*r
 //   MMA-dx    [dh_x | dm] = [delta_r|delta_z|delta_h] [W_r+U_r ; W_z+U_z ; W]       K = 3H, N = 2H
 //   MMA-P     P[(e,j), c] = sum_i A_e[i,j] dm[i,c]   per (molecule, bond-type pair); A read MN-major
 //   MMA-dh    dh_x += Pcat Wcat                       K = 4H
 //   phase E   dh_t = dh_x + ds + external dHs[t]
-// Parameter gradients are the C += A^T B contractions of bmp_wgrad_tc over Gs / Ps / Hs / Ms / RSs.
+// Parameter gradients are C += A^T B contractions streamed from the stash panels (bmp_wgrad_panels_multi).
 #include "tc_common.cuh"
 
 namespace bmp {
@@ -35,14 +35,13 @@ struct Args {
     int mb, N, T;
     const void *adj;             // fp32 (mb,E,N,N), or bytes when adj_u8
     int adj_u8;
-    const float *Hs;
-    float *Gs, *Ps, *dHs;
+    float *dHs;
+    int every_step;              // dHs: (T+1) slices, an external gradient for every h_t; else two, [0] <-> h_0, [1] <-> h_T
     const uint8_t *img[BMP_MAX_STEPS];
     int stateful[BMP_MAX_STEPS];
     const int *ext_flags;        // [T+1]: != 0 where dHs[t] holds a non-zero external gradient
     long long *dbg;              // optional phase timestamps of CTA 0 (tools/tc_timeline.py)
-    Stash2 st;                   // bf16 panel stash (use2 != 0): gate values in, delta / P panels out
-    int use2;                    //   then dHs has two slices: [0] <-> h_0, [1] <-> h_T
+    Stash2 st;                   // bf16 panel stash: gate values in, delta / P panels out
     const int32_t *midx;         // optional (mb,): adj is a drug table, molecule b = table row midx[b]
 };
 
@@ -58,7 +57,7 @@ __global__ void nonzero_flags_kernel(const float *__restrict__ x, long n_per_t, 
     if (__syncthreads_or(nz) && threadIdx.x == 0) atomicOr(flags + t, 1);
 }
 
-template <int H, bool V2>
+template <int H>
 __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const Args a) {
     using C = Cfg<H>;
     constexpr int KP = C::KP;
@@ -147,9 +146,9 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                     const bool stateful = a.stateful[t] != 0;
                     mbar_wait(BAR(B_DRDY), par);
                     tc_fence_after();
-                    uint8_t *Dt = V2 ? a.st.Dp + ((size_t)t * n_tiles + tile) * 3 * KP * PANEL_BYTES : nullptr;
-                    uint8_t *Pt2 = V2 ? a.st.Pp + ((size_t)t * n_tiles + tile) * 4 * KP * PANEL_BYTES : nullptr;
-                    if (V2) {   // delta_z | delta_h panels (and the zeroed delta_r of a stateless step)
+                    uint8_t *Dt = a.st.Dp + ((size_t)t * n_tiles + tile) * 3 * KP * PANEL_BYTES;
+                    uint8_t *Pt2 = a.st.Pp + ((size_t)t * n_tiles + tile) * 4 * KP * PANEL_BYTES;
+                    {   // delta_z | delta_h panels (and the zeroed delta_r of a stateless step)
                         const uint32_t from = stateful ? KP : 0;
                         tma_bulk_s2g(Dt + (size_t)from * PANEL_BYTES, s_d + from * PANEL_BYTES, (3 * KP - from) * PANEL_BYTES);
                         bulk_commit();
@@ -164,14 +163,14 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                                 mma_wtile(s_d + (kb * KP + kp) * PANEL_BYTES, nb ? COL_DM : COL_DHX, kb == 1 && kp == 0);
                     mbar_wait(BAR(B_DRRDY), par);
                     tc_fence_after();
-                    if (V2 && stateful) {
+                    if (stateful) {
                         tma_bulk_s2g(Dt, s_d, KP * PANEL_BYTES);      // delta_r panels
                         bulk_commit();
                     }
                     if (stateful)
                         for (int nb = 0; nb < 2; ++nb)
                             for (int kp = 0; kp < KP; ++kp) mma_wtile(s_d + kp * PANEL_BYTES, nb ? COL_DM : COL_DHX, false);
-                    if (V2) bulk_wait_read();      // the delta panels are about to be reused (dm, Pcat)
+                    bulk_wait_read();      // the delta panels are about to be reused (dm, Pcat)
                     tc_commit(BAR(B_DX));
                     mbar_wait(BAR(B_DMRDY), par);
                     tc_fence_after();
@@ -180,22 +179,18 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                     mma_p(0, 1, 3 * H, B_P + 2);
                     mbar_wait(BAR(B_PRDY + 0), par);          // P(0,0) has left columns [0,H); Pcat half 0 is ready
                     tc_fence_after();
-                    if (V2) {
-                        tma_bulk_s2g(Pt2, s_d, 2 * KP * PANEL_BYTES);
-                        bulk_commit();
-                    }
+                    tma_bulk_s2g(Pt2, s_d, 2 * KP * PANEL_BYTES);
+                    bulk_commit();
                     mma_p(1, 1, 0 * H, B_P + 3);
                     for (int kp = 0; kp < 2 * KP; ++kp) mma_wtile(s_d + kp * PANEL_BYTES, COL_DHX, false);
-                    if (V2) bulk_wait_read();
+                    bulk_wait_read();
                     tc_commit(BAR(B_PFREE));
                     mbar_wait(BAR(B_PRDY + 1), par);
                     tc_fence_after();
-                    if (V2) {
-                        tma_bulk_s2g(Pt2 + (size_t)2 * KP * PANEL_BYTES, s_d, 2 * KP * PANEL_BYTES);
-                        bulk_commit();
-                    }
+                    tma_bulk_s2g(Pt2 + (size_t)2 * KP * PANEL_BYTES, s_d, 2 * KP * PANEL_BYTES);
+                    bulk_commit();
                     for (int kp = 0; kp < 2 * KP; ++kp) mma_wtile(s_d + kp * PANEL_BYTES, COL_DHX, false);
-                    if (V2) bulk_wait_read();
+                    bulk_wait_read();
                     tc_commit(BAR(B_DH));
                 }
         }
@@ -213,7 +208,7 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
             const long grow = (long)molg * a.N + atom;
             stage_adjacency<NE>(smem + C::OFF_ADJ, a.adj, a.adj_u8, tile, a.mb, a.N, tid, a.midx);
             {
-                const float *src = live ? a.dHs + ((long)(V2 ? 1 : a.T) * rows_total + grow) * H + colbase : nullptr;
+                const float *src = live ? a.dHs + ((long)(a.every_step ? a.T : 1) * rows_total + grow) * H + colbase : nullptr;
 #pragma unroll
                 for (int c = 0; c < NC; c += 4) {
                     float4 v = src ? *reinterpret_cast<const float4 *>(src + c) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -223,19 +218,16 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
             for (int t = a.T - 1; t >= 0; --t, ++it) {
                 const uint32_t par = it & 1;
                 const bool stateful = a.stateful[t] != 0;
-                float *Gt = a.Gs + ((long)t * rows_total + grow) * 3 * H + colbase;          // r | z | hbar slots of this row
-                const float *St = a.Hs + ((long)t * rows_total + grow) * H + colbase;        // state of the step = h_t
                 uint32_t v[32];
 #define TS(i) do { if (a.dbg && blockIdx.x == 0 && tid == 0 && it < 64) a.dbg[it * 16 + (i)] = clock64(); } while (0)
                 TS(0);
                 if (t == 0 && tile + (int)gridDim.x < n_tiles) prefetch_adjacency_l2<NE>(a.adj, a.adj_u8, tile + gridDim.x, a.mb, a.N, tid, a.midx);
                 // ---- phase A: gate derivatives ----
-                if (V2) {
-                    // gate values of the step: coalesced 16-byte loads in the thread-native bf16 order, two 16-column halves
-                    // (L2-resident: prefetched during the previous step) so the live set stays under the 96-register budget
-                    const uint8_t *bz = a.st.zn(t, tile, 0, H), *bh = a.st.zn(t, tile, 1, H), *bs = a.st.zn(t, tile, 3, H);
+                // gate values of the step: coalesced 16-byte loads in the thread-native bf16 order, two 16-column halves
+                // (L2-resident: prefetched during the previous step) so the live set stays under the 96-register budget
+                const uint8_t *bz = a.st.zn(t, tile, 0, H), *bh = a.st.zn(t, tile, 1, H), *bs = a.st.zn(t, tile, 3, H);
 #pragma unroll
-                    for (int half = 0; half < NC / 16; ++half) {
+                for (int half = 0; half < NC / 16; ++half) {
                     uint4 zp[2], hp[2], sp[2];
 #pragma unroll
                     for (int g = 0; g < 2; ++g) {
@@ -270,126 +262,20 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                         if (!stateful)   // delta_r panel of a stateless step: zeros (the merged W_r contraction reads it)
                             *reinterpret_cast<uint4 *>(smem + C::OFF_D + (kk >> 6) * PANEL_BYTES + sw128(row, kk & 63)) = make_uint4(0, 0, 0, 0);
                     }
-                    }
-                } else {
-                if (t > 0 && live && !V2) {   // pull the next step's stash lines towards L2 while this step computes
-                    const char *pg = reinterpret_cast<const char *>(a.Gs + ((long)(t - 1) * rows_total + grow) * 3 * H + colbase);
-                    const char *ps = reinterpret_cast<const char *>(a.Hs + ((long)(t - 1) * rows_total + grow) * H + colbase);
-                    const char *pe = reinterpret_cast<const char *>(a.dHs + ((long)(t - 1) * rows_total + grow) * H + colbase);
-#pragma unroll
-                    for (int b = 0; b < NC * 4; b += 128) {
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(pg + b));
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(pg + (long)H * 4 + b));
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(pg + (long)2 * H * 4 + b));
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(ps + b));
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(pe + b));
-                    }
-                }
-#pragma unroll
-                for (int cc = 0; cc < NC; cc += 32) {
-                    float dz[32], dh[32];
-#pragma unroll
-                    for (int x = 0; x < 32; x += 4) {
-                        float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f), h4 = z4, s4 = z4;
-                        if (live) {
-                            z4 = *reinterpret_cast<const float4 *>(Gt + H + cc + x);
-                            h4 = *reinterpret_cast<const float4 *>(Gt + 2 * H + cc + x);
-                            if (stateful) s4 = *reinterpret_cast<const float4 *>(St + cc + x);
-                        }
-                        const float zz[4] = {z4.x, z4.y, z4.z, z4.w}, hh[4] = {h4.x, h4.y, h4.z, h4.w}, ss[4] = {s4.x, s4.y, s4.z, s4.w};
-#pragma unroll
-                        for (int y = 0; y < 4; ++y) {
-                            const float g = acc[cc + x + y];
-                            dz[x + y] = g * (hh[y] - ss[y]) * zz[y] * (1.f - zz[y]);
-                            dh[x + y] = g * zz[y] * (1.f - hh[y] * hh[y]);
-                            acc[cc + x + y] = stateful ? g * (1.f - zz[y]) : 0.f;
-                        }
-                    }
-                    if (live) {
-#pragma unroll
-                        for (int x = 0; x < 32; x += 4) {
-                            *reinterpret_cast<float4 *>(Gt + H + cc + x) = make_float4(dz[x], dz[x + 1], dz[x + 2], dz[x + 3]);
-                            *reinterpret_cast<float4 *>(Gt + 2 * H + cc + x) = make_float4(dh[x], dh[x + 1], dh[x + 2], dh[x + 3]);
-                        }
-                    }
-#pragma unroll
-                    for (int g = 0; g < 4; ++g) {
-                        const int kk = colbase + cc + 8 * g;
-                        uint4 pz = make_uint4(pack_bf16(dz[8 * g], dz[8 * g + 1]), pack_bf16(dz[8 * g + 2], dz[8 * g + 3]),
-                                              pack_bf16(dz[8 * g + 4], dz[8 * g + 5]), pack_bf16(dz[8 * g + 6], dz[8 * g + 7]));
-                        uint4 ph = make_uint4(pack_bf16(dh[8 * g], dh[8 * g + 1]), pack_bf16(dh[8 * g + 2], dh[8 * g + 3]),
-                                              pack_bf16(dh[8 * g + 4], dh[8 * g + 5]), pack_bf16(dh[8 * g + 6], dh[8 * g + 7]));
-                        *reinterpret_cast<uint4 *>(smem + C::OFF_D + (KP + (kk >> 6)) * PANEL_BYTES + sw128(row, kk & 63)) = pz;
-                        *reinterpret_cast<uint4 *>(smem + C::OFF_D + (2 * KP + (kk >> 6)) * PANEL_BYTES + sw128(row, kk & 63)) = ph;
-                    }
-                }
                 }
                 warp_arrive(BAR(B_DRDY), lane);
                 TS(1);
                 // ---- phase B: through U and the reset gate ----
-                if (V2) {
-                    // 16-column halves keep the live set under the 96-register budget: r and (again, L2-resident) the state of
-                    // the first half are requested before waiting for q (the latency overlaps MMA-q), the second half's while
-                    // the first is consumed
-                    const uint8_t *br = a.st.zn(t, tile, 2, H), *bs = a.st.zn(t, tile, 3, H);
-                    uint4 rp[2], sp[2];
-                    auto load_rs = [&](int half) {
+                // 16-column halves keep the live set under the 96-register budget: r and (again, L2-resident) the state of
+                // the first half are requested before waiting for q (the latency overlaps MMA-q), the second half's while
+                // the first is consumed
+                const uint8_t *br = a.st.zn(t, tile, 2, H);
+                uint4 rp[2], sp[2];
+                auto load_rs = [&](int half) {
 #pragma unroll
-                        for (int j = 0; j < 2; ++j) {
-                            rp[j] = __ldg(reinterpret_cast<const uint4 *>(br + ((size_t)(2 * half + j) * NE + tid) * 16));
-                            sp[j] = __ldg(reinterpret_cast<const uint4 *>(bs + ((size_t)(2 * half + j) * NE + tid) * 16));
-                        }
-                    };
-                    if (stateful) load_rs(0);
-                    mbar_wait(BAR(B_Q), par);
-                    tc_fence_after();
-                    TS(2);
-                    if (stateful) {
-#pragma unroll
-                        for (int half = 0; half < 2; ++half) {
-                            uint32_t w[16];
-                            tc_ld16(t_lane + COL_Q + colbase + 16 * half, w);
-                            tc_wait_ld();
-                            float dr[16];
-#pragma unroll
-                            for (int g = 0; g < 2; ++g) {
-                                const int j = 2 * half + g;
-                                const __nv_bfloat162 *r2 = reinterpret_cast<const __nv_bfloat162 *>(&rp[g]);
-                                const __nv_bfloat162 *s2 = reinterpret_cast<const __nv_bfloat162 *>(&sp[g]);
-#pragma unroll
-                                for (int x = 0; x < 4; ++x) {
-                                    const float2 rr = __bfloat1622float2(r2[x]), ss = __bfloat1622float2(s2[x]);
-                                    const float q0 = live ? __uint_as_float(w[8 * g + 2 * x]) : 0.f, q1 = live ? __uint_as_float(w[8 * g + 2 * x + 1]) : 0.f;
-                                    acc[8 * j + 2 * x] += q0 * rr.x;
-                                    acc[8 * j + 2 * x + 1] += q1 * rr.y;
-                                    dr[8 * g + 2 * x] = q0 * ss.x * rr.x * (1.f - rr.x);
-                                    dr[8 * g + 2 * x + 1] = q1 * ss.y * rr.y * (1.f - rr.y);
-                                }
-                            }
-                            if (half == 0) load_rs(1);
-#pragma unroll
-                            for (int g = 0; g < 2; ++g) {
-                                const int kk = colbase + 8 * (2 * half + g);
-                                uint4 pr = make_uint4(pack_bf16(dr[8 * g], dr[8 * g + 1]), pack_bf16(dr[8 * g + 2], dr[8 * g + 3]),
-                                                      pack_bf16(dr[8 * g + 4], dr[8 * g + 5]), pack_bf16(dr[8 * g + 6], dr[8 * g + 7]));
-                                *reinterpret_cast<uint4 *>(smem + C::OFF_D + (kk >> 6) * PANEL_BYTES + sw128(row, kk & 63)) = pr;
-                            }
-                        }
-                    }
-                } else {
-                // r and the state of the first column chunk are requested BEFORE waiting for q, so their latency
-                // overlaps MMA-q; the second chunk is requested while the first is being consumed.
-                float rr[32], ss[32];
-                auto load_rs = [&](int cc) {
-#pragma unroll
-                    for (int x = 0; x < 32; x += 4) {
-                        float4 r4 = make_float4(0.f, 0.f, 0.f, 0.f), s4 = r4;
-                        if (live) {
-                            r4 = *reinterpret_cast<const float4 *>(Gt + cc + x);
-                            s4 = *reinterpret_cast<const float4 *>(St + cc + x);
-                        }
-                        rr[x] = r4.x; rr[x + 1] = r4.y; rr[x + 2] = r4.z; rr[x + 3] = r4.w;
-                        ss[x] = s4.x; ss[x + 1] = s4.y; ss[x + 2] = s4.z; ss[x + 3] = s4.w;
+                    for (int j = 0; j < 2; ++j) {
+                        rp[j] = __ldg(reinterpret_cast<const uint4 *>(br + ((size_t)(2 * half + j) * NE + tid) * 16));
+                        sp[j] = __ldg(reinterpret_cast<const uint4 *>(bs + ((size_t)(2 * half + j) * NE + tid) * 16));
                     }
                 };
                 if (stateful) load_rs(0);
@@ -398,30 +284,35 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                 TS(2);
                 if (stateful) {
 #pragma unroll
-                    for (int cc = 0; cc < NC; cc += 32) {
-                        tc_ld32(t_lane + COL_Q + colbase + cc, v);
+                    for (int half = 0; half < 2; ++half) {
+                        uint32_t w[16];
+                        tc_ld16(t_lane + COL_Q + colbase + 16 * half, w);
                         tc_wait_ld();
-                        float dr[32];
+                        float dr[16];
 #pragma unroll
-                        for (int x = 0; x < 32; ++x) {
-                            const float qv = __uint_as_float(v[x]);
-                            acc[cc + x] += qv * rr[x];
-                            dr[x] = qv * ss[x] * rr[x] * (1.f - rr[x]);
+                        for (int g = 0; g < 2; ++g) {
+                            const int j = 2 * half + g;
+                            const __nv_bfloat162 *r2 = reinterpret_cast<const __nv_bfloat162 *>(&rp[g]);
+                            const __nv_bfloat162 *s2 = reinterpret_cast<const __nv_bfloat162 *>(&sp[g]);
+#pragma unroll
+                            for (int x = 0; x < 4; ++x) {
+                                const float2 rr = __bfloat1622float2(r2[x]), ss = __bfloat1622float2(s2[x]);
+                                const float q0 = live ? __uint_as_float(w[8 * g + 2 * x]) : 0.f, q1 = live ? __uint_as_float(w[8 * g + 2 * x + 1]) : 0.f;
+                                acc[8 * j + 2 * x] += q0 * rr.x;
+                                acc[8 * j + 2 * x + 1] += q1 * rr.y;
+                                dr[8 * g + 2 * x] = q0 * ss.x * rr.x * (1.f - rr.x);
+                                dr[8 * g + 2 * x + 1] = q1 * ss.y * rr.y * (1.f - rr.y);
+                            }
                         }
-                        if (cc + 32 < NC) load_rs(cc + 32);
-                        if (live) {
+                        if (half == 0) load_rs(1);
 #pragma unroll
-                            for (int x = 0; x < 32; x += 4) *reinterpret_cast<float4 *>(Gt + cc + x) = make_float4(dr[x], dr[x + 1], dr[x + 2], dr[x + 3]);
-                        }
-#pragma unroll
-                        for (int g = 0; g < 4; ++g) {
-                            const int kk = colbase + cc + 8 * g;
+                        for (int g = 0; g < 2; ++g) {
+                            const int kk = colbase + 8 * (2 * half + g);
                             uint4 pr = make_uint4(pack_bf16(dr[8 * g], dr[8 * g + 1]), pack_bf16(dr[8 * g + 2], dr[8 * g + 3]),
                                                   pack_bf16(dr[8 * g + 4], dr[8 * g + 5]), pack_bf16(dr[8 * g + 6], dr[8 * g + 7]));
                             *reinterpret_cast<uint4 *>(smem + C::OFF_D + (kk >> 6) * PANEL_BYTES + sw128(row, kk & 63)) = pr;
                         }
                     }
-                }
                 }
                 warp_arrive(BAR(B_DRRDY), lane);
                 TS(3);
@@ -445,11 +336,11 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                 }
                 warp_arrive(BAR(B_DMRDY), lane);
                 TS(5);
-                if (V2 && t > 0) {      // while MMA-P runs: gate values of the NEXT step (t-1) towards L2 (four 128 x H bf16 blocks)
+                if (t > 0) {      // while MMA-P runs: gate values of the NEXT step (t-1) towards L2 (four 128 x H bf16 blocks)
                     const char *nx = reinterpret_cast<const char *>(a.st.zn(t - 1, tile, 0, H));
                     for (int off = tid * 128; off < 4 * 128 * H * 2; off += NE * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(nx + off));
                 }
-                // ---- phase D: P accumulators -> bf16 A-operand panels (two K halves) + fp32 stash ----
+                // ---- phase D: P accumulators -> bf16 A-operand panels (two K halves) ----
                 for (int p = 0; p < 2; ++p) {
                     if (p == 1) mbar_wait(BAR(B_PFREE), par);
                     for (int mol = 0; mol < 2; ++mol) {
@@ -460,19 +351,10 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                         TS(6 + pi);
                         const int orow = mol * 64 + atom;                   // row of (mol, atom j) in the tile
                         const int kbase = molslot * H + colbase;            // TMEM lane half = bond type within the pair
-                        const int omol = tile * 2 + mol;
-                        const bool olive = omol < a.mb && atom < a.N;
-                        float *Pt = a.Ps + (((long)t * rows_total + (long)omol * a.N + atom) * 4 + (2 * p + molslot)) * H + colbase;
 #pragma unroll
                         for (int cc = 0; cc < NC; cc += 32) {
                             tc_ld32(t_lane + pcol + colbase + cc, v);
                             tc_wait_ld();
-                            if (olive && !V2) {
-#pragma unroll
-                                for (int x = 0; x < 32; x += 4)
-                                    *reinterpret_cast<float4 *>(Pt + cc + x) = make_float4(__uint_as_float(v[x]), __uint_as_float(v[x + 1]),
-                                                                                           __uint_as_float(v[x + 2]), __uint_as_float(v[x + 3]));
-                            }
 #pragma unroll
                             for (int g = 0; g < 4; ++g) {
                                 const int kk = kbase + cc + 8 * g;
@@ -489,8 +371,8 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                 TS(10);
                 // ---- phase E: dh_t = dh_x (+ dh_msg) + ds + external gradient ----
                 {
-                    float *ext = a.dHs + ((long)(V2 ? 0 : t) * rows_total + grow) * H + colbase;
-                    const bool has_ext = live && (V2 ? t == 0 : a.ext_flags[t] != 0);
+                    const float *ext = a.dHs + ((long)(a.every_step ? t : 0) * rows_total + grow) * H + colbase;
+                    const bool has_ext = live && (a.every_step ? a.ext_flags[t] != 0 : t == 0);
                     if (has_ext) {      // requested and folded in before waiting for the accumulator: the latency overlaps MMA-dh
 #pragma unroll
                         for (int x = 0; x < NC; x += 4) {
@@ -512,7 +394,7 @@ __global__ void __launch_bounds__(32 * (H / 8 + 2), 1) ggnn_tc_bwd_kernel(const 
                         // dL/dh_0 of the tile: coalesced rows through a transposition block (the delta panels are idle:
                         // every MMA of the tile has completed)
                         float *stg = reinterpret_cast<float *>(smem + C::OFF_D + warp * 2048);
-                        float *out = a.dHs + colbase;      // slice 0 in both stash layouts
+                        float *out = a.dHs + colbase;      // slice 0 in both dHs layouts
 #pragma unroll
                         for (int h2 = 0; h2 < 2; ++h2)
                             warp_store_rows<16>(stg, acc + 16 * h2, lane, [&](int r) -> float * {
@@ -583,20 +465,23 @@ using namespace bmp;
 static long long *g_tc_dbg = nullptr;
 extern "C" void bmp_debug_set_buffer(void *p) { g_tc_dbg = (long long *)p; }
 
-// Data part of the backward on tcgen05; called by bmp_ggnn_backward when mode == BMP_MODE_BF16.
+int bmp_wgrad_panels_multi(bmp::w2::Args *list, int n, void *stream);   // wgrad_tc2.cu
+
+// BMP_MODE_BF16 backward over the bf16 panel stash; called by bmp_ggnn_backward.  The data kernel, then every parameter
+// gradient as a C += A^T B contraction whose operands are streamed straight from the dumped panels.
 int bmp_ggnn_backward_tc(const bmp_ggnn_bwd_t *a, void *stream) {
-    const int H = a->hidden, T = a->n_steps;
+    const int H = a->hidden, T = a->n_steps, KP = H / 64;
     if (!a->tc_workspace || a->tc_workspace_bytes < bmp_ggnn_tc_workspace_bytes(H, T)) {
         set_error("BMP_MODE_BF16 backward: tc_workspace of >= %zu bytes required", bmp_ggnn_tc_workspace_bytes(H, T));
         return BMP_EINVAL;
     }
     cudaStream_t st = (cudaStream_t)stream;
     tcb::Args k = {};
-    k.mb = a->mb; k.N = a->n_atoms; k.T = T; k.adj = a->adj; k.adj_u8 = a->adj_u8; k.Hs = a->Hs; k.Gs = a->Gs; k.Ps = a->Ps; k.dHs = a->dHs;
+    k.mb = a->mb; k.N = a->n_atoms; k.T = T; k.adj = a->adj; k.adj_u8 = a->adj_u8; k.dHs = a->dHs; k.every_step = a->dHs_every_step != 0;
     uint8_t *ws = (uint8_t *)(((uintptr_t)a->tc_workspace + 255) & ~(uintptr_t)255);
     int *flags = reinterpret_cast<int *>(ws);      // first 256 B of the workspace: per-step external-gradient flags
     ws += 256;
-    if (!a->stash2) {
+    if (k.every_step) {
         cudaMemsetAsync(flags, 0, (T + 1) * sizeof(int), st);
         tcb::nonzero_flags_kernel<<<dim3(64, T + 1), 256, 0, st>>>(a->dHs, (long)a->mb * a->n_atoms * H, flags);
         count_launch();
@@ -604,8 +489,8 @@ int bmp_ggnn_backward_tc(const bmp_ggnn_bwd_t *a, void *stream) {
     k.ext_flags = flags;
     k.dbg = g_tc_dbg;
     k.midx = a->mol_index;
-    k.use2 = a->stash2 != nullptr;
-    if (k.use2) k.st.carve(a->stash2, (a->mb + 1) / 2, H, T);
+    const int n_tiles = (a->mb + 1) / 2;
+    k.st.carve(a->stash2, n_tiles, H, T);
     const size_t ib = tcb::image_bytes(H);
     int n_img = 0;
     for (int t = 0; t < T; ++t) {
@@ -629,32 +514,21 @@ int bmp_ggnn_backward_tc(const bmp_ggnn_bwd_t *a, void *stream) {
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int n_tiles = (a->mb + 1) / 2;
     const int grid = n_tiles < sms ? n_tiles : sms;
-#define LAUNCH_BWD(HH, VV)                                                                                                   \
-    do {                                                                                                                      \
-        cudaFuncSetAttribute(tcb::ggnn_tc_bwd_kernel<HH, VV>, cudaFuncAttributeMaxDynamicSharedMemorySize, tcb::Cfg<HH>::SMEM_BYTES); \
-        tcb::ggnn_tc_bwd_kernel<HH, VV><<<grid, 32 * (HH / 8 + 2), tcb::Cfg<HH>::SMEM_BYTES, st>>>(k);                                  \
+#define LAUNCH_BWD(HH)                                                                                                     \
+    do {                                                                                                                   \
+        cudaFuncSetAttribute(tcb::ggnn_tc_bwd_kernel<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, tcb::Cfg<HH>::SMEM_BYTES); \
+        tcb::ggnn_tc_bwd_kernel<HH><<<grid, 32 * (HH / 8 + 2), tcb::Cfg<HH>::SMEM_BYTES, st>>>(k);                              \
     } while (0)
-    ProfScope prof(BMP_PROF_GGNN_BWD, st);
-    if (H == 64) { if (k.use2) LAUNCH_BWD(64, true); else LAUNCH_BWD(64, false); }
-    else { if (k.use2) LAUNCH_BWD(128, true); else LAUNCH_BWD(128, false); }
+    {
+        ProfScope prof(BMP_PROF_GGNN_BWD, st);
+        if (H == 64) LAUNCH_BWD(64);
+        else LAUNCH_BWD(128);
+    }
 #undef LAUNCH_BWD
     count_launch();
-    return check_launch("ggnn_tc_bwd_kernel");
-}
-
-int bmp_wgrad_panels_multi(bmp::w2::Args *list, int n, void *stream);   // wgrad_tc2.cu
-
-// Backward over the bf16 panel stash (stash v2): data kernel, then every parameter gradient as a
-// C += A^T B contraction whose operands are streamed straight from the dumped panels.
-int bmp_ggnn_backward_v2(const bmp_ggnn_bwd_t *a, void *stream) {
-    const int H = a->hidden, T = a->n_steps, KP = H / 64;
-    int rc = bmp_ggnn_backward_tc(a, stream);
-    if (rc) return rc;
-    tc::Stash2 S;
-    const int n_tiles = (a->mb + 1) / 2;
-    S.carve(a->stash2, n_tiles, H, T);
+    if ((rc = check_launch("ggnn_tc_bwd_kernel"))) return rc;
+    const tc::Stash2 &S = k.st;
     // Grouped contractions: every launch reads its A blocks and B blocks once (the kernel is HBM-bound), so the
     // launches are arranged for the fewest operand reads:
     //   per gate g and run of equal statefulness:  delta_g^T [h | m | r*h]  -> W_g (both halves) and U_g together

@@ -42,7 +42,7 @@ class GgnnBwd(C.Structure):
         ("stateful", C.c_int * MAX_STEPS), ("Hs", fp), ("Ms", fp), ("RSs", fp), ("Gs", fp), ("Ps", fp), ("dHs", fp),
         ("d_msg_W", _A()), ("d_msg_b", _A()), ("d_gru", GRU * MAX_STEPS), ("d_state_in", fp),
         ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("stash2", fp), ("tc_images_ready", C.c_int), ("adj_u8", C.c_int),
-        ("mol_index", fp)]
+        ("mol_index", fp), ("dHs_every_step", C.c_int)]
 
 
 class Pair(C.Structure):

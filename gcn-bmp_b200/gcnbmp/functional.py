@@ -180,7 +180,8 @@ def _grad_targets(params):
 class GGNNEncode(torch.autograd.Function):
     """embed -> T x GGNNUpdate.  `plan` = list of (msg_idx, gru_idx, stateful) per step;
     `params` = [embed_W or None] + n_msg*(W,b) + n_gru*12 tensors.
-    Returns Hs (T+1, mb, N, H) when a tape is needed, else a (2, mb, N, H) tensor [h_0, h_T]."""
+    Returns Hs (T+1, mb, N, H) when a tape is needed (BMP_MODE_BF16: only with `keep_steps`), else a (2, mb, N, H) tensor
+    [h_0, h_T]."""
 
     @staticmethod
     def forward(ctx, x, adj, state_in, plan, n_msg, n_gru, mode, want_stash, keep_steps, mol_index, *params):
@@ -225,15 +226,20 @@ class GGNNEncode(torch.autograd.Function):
                                  "or train in MODE_F32)")
             ws, a.tc_images_ready = _tc_images("ggnn_fwd", nbytes, dev, params)
             a.tc_workspace, a.tc_workspace_bytes = _p(ws), nbytes
-        if want_stash and mode == K.MODE_BF16 and not keep_steps:
-            # bf16 panel stash: the tape keeps operand panels + gate values; only [h_0, h_T] go back as fp32
-            out = torch.empty((2, mb, N, H), device=dev, dtype=torch.float32)
+        if want_stash and mode == K.MODE_BF16:
+            # bf16 panel stash: the tape keeps operand panels + gate values; only [h_0, h_T] (every h_t with keep_steps) go
+            # back as fp32
+            out = torch.empty((T + 1 if keep_steps else 2, mb, N, H), device=dev, dtype=torch.float32)
             stash2 = torch.empty((int(K.lib.bmp_ggnn_stash2_bytes(mb, H, T)),), device=dev, dtype=torch.uint8)
-            a.h0_out, a.h_out, a.stash2 = _p(out[0]), _p(out[1]), _p(stash2)
+            if keep_steps:
+                a.Hs = _p(out)
+            else:
+                a.h0_out, a.h_out = _p(out[0]), _p(out[1])
+            a.stash2 = _p(stash2)
             K.check(K.lib.bmp_ggnn_forward(C.byref(a), _stream()))
             ctx.save_for_backward(x, adj, state_in, stash2, None, None, None, *params)
             ctx.mol_index = mol_index
-            ctx.meta = (plan, n_msg, n_gru, mode, is_ids, (mb, N, H))
+            ctx.meta = (plan, n_msg, n_gru, mode, is_ids, keep_steps)
             return out
         x3ws = None
         if mode == K.MODE_F32 and state_in is None and mol_index is None and not adj_u8:
@@ -247,7 +253,7 @@ class GGNNEncode(torch.autograd.Function):
             K.check(K.lib.bmp_ggnn_forward(C.byref(a), _stream()))
             ctx.save_for_backward(x, adj, state_in, Hs, Ms, Gs, RSs, *params)
             ctx.mol_index = mol_index
-            ctx.meta = (plan, n_msg, n_gru, mode, is_ids, None)
+            ctx.meta = (plan, n_msg, n_gru, mode, is_ids, keep_steps)
             ctx.x3 = x3ws is not None
             return Hs
         out = torch.empty((2, mb, N, H), device=dev, dtype=torch.float32)   # [h_0, h_T]
@@ -259,15 +265,13 @@ class GGNNEncode(torch.autograd.Function):
     def backward(ctx, dHs):
         x, adj, state_in, Hs, Ms, Gs, RSs = ctx.saved_tensors[:7]
         params = ctx.saved_tensors[7:]
-        plan, n_msg, n_gru, mode, is_ids, v2shape = ctx.meta
+        plan, n_msg, n_gru, mode, is_ids, keep_steps = ctx.meta
         T = len(plan)
         E = adj.shape[1]
+        _, mb, N, H = dHs.shape
         stash2 = None
-        if v2shape is not None:
+        if mode == K.MODE_BF16:         # the tape is the bf16 panel stash, saved in the Hs slot
             stash2, Hs = Hs, None
-            mb, N, H = v2shape
-        else:
-            _, mb, N, H = Hs.shape
         rows = mb * N
         dHs = dHs.contiguous().clone()
         grads, rets = _grad_targets(params)
@@ -284,7 +288,7 @@ class GGNNEncode(torch.autograd.Function):
             a.d_msg_W[t], a.d_msg_b[t] = _p(grads[1 + 2 * mi]), _p(grads[2 + 2 * mi])
             _fill_gru(a.d_gru[t], grads[base + 12 * gi: base + 12 * (gi + 1)])
         a.Hs, a.Ms, a.RSs, a.Gs, a.Ps, a.dHs = _p(Hs), _p(Ms), _p(RSs), _p(Gs), _p(Ps), _p(dHs)
-        a.stash2 = _p(stash2)
+        a.stash2, a.dHs_every_step = _p(stash2), int(keep_steps)
         d_state = torch.zeros_like(state_in) if state_in is not None else None
         a.d_state_in = _p(d_state)
         if mode == K.MODE_BF16:

@@ -305,7 +305,7 @@ class _GRU(Link):
 
 def _encode(x, adj, state, plan, msgs, grus, embed_W, mode, keep_steps=False, mol_index=None):
     """Returns (states, last): states[0] = h_0, states[last] = h_T; every step is present only when
-    `keep_steps` (or in fp32 mode with a tape) -- BF16 mode otherwise keeps a bf16 panel stash internally."""
+    `keep_steps` (or in fp32 mode with a tape) -- BF16 mode trains on a bf16 panel stash it keeps internally."""
     want = torch.is_grad_enabled()
     H = msgs[0][0].shape[1]
     if mode == K.MODE_BF16 and adj.shape[-1] > Fn.MAX_KERNEL_ATOMS and mol_index is None:

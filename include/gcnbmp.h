@@ -70,9 +70,11 @@ typedef struct {                             /* gradients, same shapes; accumula
  * state at that call (the StatefulGRU "h is not None" branch); the state is
  * `state_in` for t == 0 and the step's own input h for t > 0 (which is what every
  * reference GGNN feeds it).  Tied weights = the same pointers at every t.
- * Stash buffers (needed by bmp_ggnn_backward, NULL for inference):
+ * Stash buffers (needed by the BMP_MODE_F32 bmp_ggnn_backward, NULL for inference):
  *   Hs (T+1, mb*N, H)  h_0 .. h_T           Ms (T, mb*N, H)   messages
- *   Gs (T, mb*N, 3H)   r | z | h_bar        RSs (T, mb*N, H)  r*state            */
+ *   Gs (T, mb*N, 3H)   r | z | h_bar        RSs (T, mb*N, H)  r*state
+ * BMP_MODE_BF16 trains on stash2 instead: Ms / Gs / RSs must be NULL there, and Hs
+ * (only with stash2) receives h_0 .. h_T as an output the backward does not read.   */
 typedef struct {
     int mb, n_atoms, hidden, n_edge, n_steps, n_atom_types, mode;
     const int32_t *atoms;        /* (mb,N) or NULL when h_in is given              */
@@ -86,11 +88,11 @@ typedef struct {
     int            stateful[BMP_MAX_STEPS];
     float *h_out;                /* (mb,N,H) final atom states (get_atom_array)     */
     float *h0_out;               /* (mb,N,H) copy of h_0 for the readout, or NULL   */
-    float *Hs, *Ms, *Gs, *RSs;   /* stash or NULL                                   */
+    float *Hs, *Ms, *Gs, *RSs;   /* stash or NULL (BMP_MODE_BF16: Hs only, see above) */
     void  *tc_workspace;         /* BMP_MODE_BF16 only: packed bf16 weight tiles    */
     size_t tc_workspace_bytes;   /* >= bmp_ggnn_tc_workspace_bytes(hidden, n_steps) */
     void  *stash2;               /* BMP_MODE_BF16 training: bf16 panel stash of      */
-                                 /* bmp_ggnn_stash2_bytes() bytes; replaces Hs..RSs  */
+                                 /* bmp_ggnn_stash2_bytes() bytes, the only tape     */
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
     int    adj_u8;               /* BMP_MODE_BF16 only, storage of `adj`: 0 = fp32 (mb,E,N,N) as the reference; 1 = the same
@@ -135,14 +137,17 @@ typedef struct {
     float *d_state_in;
     void  *tc_workspace;         /* BMP_MODE_BF16 only (same size rule as the forward) */
     size_t tc_workspace_bytes;
-    void  *stash2;               /* the forward's panel stash; then Hs/Ms/RSs/Gs/Ps may be NULL and dHs has TWO
-                                    slices: [0] = gradient w.r.t. h_0, [1] = gradient w.r.t. h_T               */
+    void  *stash2;               /* BMP_MODE_BF16: the forward's panel stash (required there); Hs/Ms/RSs/Gs/Ps are
+                                    unused and dHs is laid out as dHs_every_step says                          */
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
     int    adj_u8;               /* BMP_MODE_BF16 only, storage of `adj`: 0 = fp32 (mb,E,N,N) as the reference; 1 = the same
                                    array as bytes (exact for 0/1 bonds; 1/4 of the PCIe / HBM traffic); 2 = bit-packed rows
                                    (mb,E,N,ceil(N/8)), bit j&7 of byte j>>3 = adj[i][j] (numpy.packbits little; 1/32)  */
     const int32_t *mol_index;    /* the forward's mol_index: adjacency table rows, or NULL                          */
+    int    dHs_every_step;       /* BMP_MODE_BF16 only.  0: dHs has TWO slices, [0] = gradient w.r.t. h_0, [1] = gradient
+                                    w.r.t. h_T.  Nonzero: dHs (T+1, mb*N, H) as in BMP_MODE_F32, an external gradient for
+                                    every h_t.  Either way dHs[0] holds the total gradient w.r.t. h_0 on exit    */
 } bmp_ggnn_bwd_t;
 
 int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream);

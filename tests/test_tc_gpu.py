@@ -152,6 +152,45 @@ def test_tc_encoder_runs_other_hidden_sizes_zero_padded(H, T, tied, cls):
         assert _rms_rel(gd[k], ref) <= 5e-2, (k, _rms_rel(gd[k], ref))
 
 
+@pytest.mark.parametrize("cls,tied", [("ggnn", True), ("ggnn", False), ("mono", True), ("mono", False)])
+def test_tc_concat_hidden_training_matches_oracle(cls, tied):
+    """concat_hidden reads out every step's atom states, so the BF16 training forward hands back all T+1 states and the backward
+    takes a gradient for each of them: graph vectors and every parameter gradient vs the fp64 oracle within the BF16-mode bound."""
+    import gcnbmp
+    from gcnbmp import synthetic
+    from oracle import minichainer as F
+    H, T, O, mb, N = 64, 3, 32, 5, 40
+    rng = np.random.default_rng(17 + tied)
+    atoms, adj = synthetic.random_molecules(rng, mb, N)
+    if cls == "mono":
+        params = R.init_params(R.ggnn_mono_shapes(O, H, T, concat_hidden=True, weight_tying=tied), rng, dtype=np.float64)
+        tab = R.wrap_params(params)
+        onet = R.GGNNMono(R.P(tab), O, H, T, concat_hidden=True, weight_tying=tied)
+        net = gcnbmp.GGNNMono(O, H, T, concat_hidden=True, weight_tying=tied)
+    else:
+        params = R.init_params(R.ggnn_shapes(O, H, T, concat_hidden=True, weight_tying=tied), rng, dtype=np.float64)
+        tab = R.wrap_params(params)
+        onet = R.GGNN(R.P(tab), O, H, T, concat_hidden=True, weight_tying=tied)
+        net = gcnbmp.GGNN(O, hidden_dim=H, n_layers=T, concat_hidden=True, weight_tying=tied)
+    og = onet(atoms, adj.astype(np.float64))
+    w = rng.standard_normal(og.data.shape)
+    F.sum_(F.mul(og, F.const(w))).backward()
+    net.load_params(params)
+    net.mode = gcnbmp.MODE_BF16
+    g = net(atoms, adj)
+    assert tuple(g.shape) == og.data.shape
+    (g * torch.tensor(w, dtype=torch.float32, device="cuda")).sum().backward()
+    pg = g.detach().cpu().numpy()
+    assert rel_err(pg, og.data) <= MAX_TOL and _rms_rel(pg, og.data) <= RMS_TOL, (rel_err(pg, og.data), _rms_rel(pg, og.data))
+    gd = net.grad_dict()
+    for k in gd:
+        ref = tab[k].grad
+        if ref is None or np.abs(ref).max() < 1e-9:     # untied: the U matrices of a GRU that never has a state
+            continue
+        assert gd[k].shape == ref.shape and np.isfinite(gd[k]).all(), k
+        assert _rms_rel(gd[k], ref) <= MAX_TOL, (k, _rms_rel(gd[k], ref))
+
+
 @pytest.mark.parametrize("rows,M,N,lda_pad", [(5000, 128, 128, 0), (777, 192, 64, 64), (20000, 384, 256, 0), (64, 64, 128, 128)])
 def test_wgrad_tc_matches_fp64(rows, M, N, lda_pad):
     """C += A^T B on tcgen05 (bf16 operands) vs float64; bias = column sums of A (exact fp32 adds)."""

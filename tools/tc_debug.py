@@ -17,7 +17,7 @@ N = int(sys.argv[4]) if len(sys.argv) > 4 else 64
 rng = np.random.default_rng(0)
 atoms, adj = synthetic.random_molecules(rng, mb, N)
 net = gcnbmp.GGNNMono(H, H, T)
-net.keep_steps = True   # per-step states for the comparison (fp32 stash path)
+net.keep_steps = True   # per-step states for the comparison (every h_t written by the training forward)
 outs = {}
 for mode in (gcnbmp.MODE_F32, gcnbmp.MODE_BF16):
     net.mode = mode
