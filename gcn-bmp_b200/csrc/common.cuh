@@ -52,6 +52,24 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }
 
+// rescale_adj's column scale of one molecule (models/relgcn.py:20-28): inv[j] = 1 / sum_{e,i} adj[e][i][j], 1 where that sum is 0,
+// for j < N <= BMP_X3_MAX_ATOMS.  256 threads; per 64-column chunk four partial sums per column (rows r = p mod 4).
+__device__ __forceinline__ void column_inverse_degree(const float *__restrict__ adj, int E, int N, float (*part)[64], float *inv) {
+    const int j = threadIdx.x & 63, p = threadIdx.x >> 6;
+    for (int j0 = 0; j0 < N; j0 += 64) {
+        float s = 0.f;
+        if (j0 + j < N)
+            for (int r = p; r < E * N; r += 4) s += __ldg(adj + (long)r * N + j0 + j);
+        part[p][j] = s;
+        __syncthreads();
+        if (threadIdx.x < 64 && j0 + (int)threadIdx.x < N) {
+            const float t = (part[0][threadIdx.x] + part[1][threadIdx.x]) + (part[2][threadIdx.x] + part[3][threadIdx.x]);
+            inv[j0 + threadIdx.x] = t != 0.f ? 1.f / t : 1.f;
+        }
+        __syncthreads();
+    }
+}
+
 __device__ __forceinline__ float act_fwd(int act, float x) {
     switch (act) {
         case BMP_ACT_TANH: return tanhf(x);

@@ -22,6 +22,7 @@
 // 6 converter warps (fp32 rows, landed in a two-deep shared-memory ring by one cp.async.bulk copy per row, -> hi / lo
 // SW128 K-major panels), one producer warp (fp32 A rows and packed hi / lo weight k-tiles, cp.async.bulk + mbarrier), one MMA lane.  Two 128-column
 // TMEM accumulators alternate between consecutive items, so an item's epilogue overlaps the next item's MMAs.
+#include <cstdio>
 #include <cstring>
 #include <cuda.h>
 #include "tc_common.cuh"
@@ -30,7 +31,7 @@ namespace bmp {
 namespace x3 {
 using namespace tc;
 
-constexpr int MAXB = 5, MAXJ = 4;
+constexpr int MAXB = 6, MAXJ = 4;
 constexpr int STAGES = 2;
 constexpr int STAGE_BYTES = 2 * PANEL_BYTES;      // converted A operand: [A_hi | A_lo]
 constexpr int WDEPTH = 3;                         // packed weight k-tiles in flight (own ring: the L2 latency of a tile is hidden)
@@ -46,7 +47,7 @@ constexpr int OFF_F32 = OFF_WR + WDEPTH * 2 * PANEL_BYTES;
 constexpr int OFF_BAR = OFF_F32 + F32_DEPTH * F32_SLOT;
 constexpr int SMEM_BYTES = OFF_BAR + 256 + 1024;
 
-enum { EPI_MSG = 0, EPI_R, EPI_Z, EPI_HB, EPI_Q, EPI_DHX, EPI_DM, EPI_DHMSG, EPI_LIN /* accumulator + bias */ };
+enum { EPI_MSG = 0, EPI_R, EPI_Z, EPI_HB, EPI_Q, EPI_DHX, EPI_DM, EPI_DHMSG, EPI_LIN /* accumulator + bias */, EPI_TANH /* tanh(accumulator + bias) */ };
 
 struct Job {
     const float *A[MAXB];            // K-block b: (rows, 64 * kt[b]) fp32, leading dimension lda[b]
@@ -309,7 +310,7 @@ __global__ void __launch_bounds__(NT, 1) rowgemm3_kernel(const __grid_constant__
                     __syncwarp();
                     if (lane == 0) mbar_arrive(ACCE(buf));
                 }
-                if (epi == EPI_R || epi == EPI_Z || epi == EPI_HB || epi == EPI_LIN) {
+                if (epi == EPI_R || epi == EPI_Z || epi == EPI_HB || epi == EPI_LIN || epi == EPI_TANH) {
 #pragma unroll
                     for (int j = 0; j < 2; ++j) {
                         float2 b2 = make_float2(0.f, 0.f);
@@ -371,6 +372,11 @@ __global__ void __launch_bounds__(NT, 1) rowgemm3_kernel(const __grid_constant__
                     }
                     case EPI_DHMSG: {
                         X3_EACH(f[rr][j].x += x0[rr][j].x + x1[rr][j].x; f[rr][j].y += x0[rr][j].y + x1[rr][j].y)
+                        ST(J.out0, J.lo0, f);
+                        break;
+                    }
+                    case EPI_TANH: {
+                        X3_EACH(f[rr][j].x = tanh_x3(f[rr][j].x); f[rr][j].y = tanh_x3(f[rr][j].y))
                         ST(J.out0, J.lo0, f);
                         break;
                     }
@@ -501,10 +507,11 @@ __global__ void __launch_bounds__(256) adj_mask_kernel(const float *__restrict__
 // BWD = false: dst[row i][e*H + c] = sum_j A_e[i][j] src[j][c]  (A_e h; deg[row][e] = sum_j A_e[i][j] into rows of 64 floats, the A
 //              operand of the bias k-tile)
 // BWD = true : dst[row j][e*H + c] = sum_i A_e[i][j] src[i][c]  (A_e^T dm)                                    one CTA per molecule
+// cscale (mb, N) or NULL: every A_e[i][j] is taken times cscale[mol][j] (RelGCN's rescale_adj), deg included
 template <bool BWD>
 __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__restrict__ masks, const int *__restrict__ nonbinary,
                                                   const float *__restrict__ adj, const float *__restrict__ src, float *__restrict__ dst,
-                                                  float *__restrict__ deg, int mb, int N, int H) {
+                                                  float *__restrict__ deg, int mb, int N, int H, const float *__restrict__ cscale) {
     extern __shared__ __align__(16) float sh[];                  // [N][H]
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, HV = H / 4, W = (N + 63) >> 6, per = 4 * N * W;
     const bool general = *nonbinary != 0;
@@ -515,6 +522,7 @@ __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__re
         __syncthreads();
         const unsigned long long *mk = masks + (size_t)mol * 2 * per + (BWD ? per : 0);
         const float *am = adj + (long)mol * 4 * N * N;
+        const float *cs = cscale ? cscale + (long)mol * N : nullptr;
         for (int idx = warp; idx < 4 * N; idx += 8) {
             const int e = idx / N, x = idx - e * N;
             float4 acc0 = make_float4(0.f, 0.f, 0.f, 0.f), acc1 = acc0;
@@ -524,7 +532,8 @@ __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__re
                 while (m) {
                     const int y = 64 * w + __ffsll((long long)m) - 1;
                     m &= m - 1;
-                    const float v = general ? __ldg(am + ((long)e * N + (BWD ? y : x)) * N + (BWD ? x : y)) : 1.f;
+                    float v = general ? __ldg(am + ((long)e * N + (BWD ? y : x)) * N + (BWD ? x : y)) : 1.f;
+                    if (cs) v *= cs[BWD ? x : y];
                     d += v;
                     const float4 *hr = reinterpret_cast<const float4 *>(sh + y * H);
                     if (lane < HV) {
@@ -866,7 +875,7 @@ int bmp_ggnn_forward_x3(const bmp_ggnn_fwd_t *a, void *stream) {
         const uint8_t *img = ws + (size_t)img_of[t] * L.img_bytes;
         const bmp_gru_t &G = a->gru[t];
         float *h = Hs_at(t), *hn = Hs_at(t + 1), *m = Ms_at(t), *g = Gs_at(t), *rs = RS_at(t);
-        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, h, AH, t == 0 ? deg : nullptr, a->mb, N, H);
+        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, h, AH, t == 0 ? deg : nullptr, a->mb, N, H, nullptr);
         count_launch();
         if ((rc = check_launch("agg_kernel"))) return rc;
         Args ga;
@@ -1001,7 +1010,7 @@ int bmp_ggnn_backward_x3(const bmp_ggnn_bwd_t *a, void *stream) {
             }
         ga.njobs = nj;
         if ((rc = launch_gemm(ga, st))) return rc;
-        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, dm, a->Ps + (size_t)t * 4 * RH, nullptr, a->mb, N, H);
+        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, dm, a->Ps + (size_t)t * 4 * RH, nullptr, a->mb, N, H, nullptr);
         count_launch();
         if ((rc = check_launch("agg_kernel"))) return rc;
         // ---- dHs[t] += dh_x + sum_e P_e W_e
@@ -1018,6 +1027,356 @@ int bmp_ggnn_backward_x3(const bmp_ggnn_bwd_t *a, void *stream) {
             J.out0 = gout + nc * 128; J.lo0 = H;
         }
         if ((rc = launch_gemm(ga, st))) return rc;
+    }
+    return BMP_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ RelGCN encoder (BMP_MODE_F32, 65..256 atoms)
+// models/relgcn.py:61-73 and models/update/relgcn_update.py:24-44 for molecules the one-CTA-per-molecule FFMA kernels of relgcn.cu
+// cannot hold.  A layer is the GGNN message with a self term and no gate:
+//   forward layer l     agg        AH_e = A_e h_l, deg_e = A_e 1                       (rescale_adj: A_e[i][j] times cs[j])
+//                       rowgemm3   h_{l+1} = act([h_l | AH_0 .. AH_3 | deg] [W_s | W_0 .. W_3 | b_e]^T + b_s)
+//   backward layer l    delta      d = g * act'(h_{l+1})                               (pointwise)
+//                       agg        P_e = A_e^T d
+//                       rowgemm3   g <- [d | P_0 .. P_3] [W_s | W_0 .. W_3]             (the transposed packing)
+//                       dW_s += d^T h_l, db_s += sum d, dW_e += P_e^T h_l, db_e += sum P_e (bmp_wgrad_tc3 over the caller's Hs)
+// Every layer runs at one padded width Cp (the widest channel count rounded up to 64, 128 or 256): padded channels meet zero
+// weights and zero bias, so they stay exactly 0 under identity and tanh.  The caller's buffers (Hs, h_out, d_h0) keep the
+// unpadded widths of ch[]; batches of fewer than 128 rows run the GEMMs over one zero-padded 128-row tile.
+namespace bmp {
+namespace x3 {
+
+static int relgcn_cpad(int cmax) { return cmax <= 64 ? 64 : (cmax <= 128 ? 128 : (cmax <= 256 ? 256 : 0)); }
+static bool relgcn_shape_ok(int mb, int N, int cmax, int L) {
+    const int Cp = relgcn_cpad(cmax);
+    return mb > 0 && N > BMP_MAX_ATOMS && N <= BMP_X3_MAX_ATOMS && cmax > 0 && Cp > 0 && L > 0 && L <= BMP_MAX_STEPS &&
+           (size_t)N * Cp * sizeof(float) <= 160 * 1024;
+}
+__host__ __device__ inline int relgcn_ftiles(int Cp) { return ((Cp + 127) / 128) * (5 * (Cp / 64) + 1); }   // forward job: h, AH_0..3, deg (bias tile)
+__host__ __device__ inline int relgcn_btiles(int Cp) { return ((Cp + 127) / 128) * (5 * (Cp / 64)); }       // backward job: d, P_0..3
+
+struct RLayout {
+    size_t layer_img, bias_off, cs_off, mask_off, deg_off, ah_off, x_off, total;
+    long rg;                                   // GEMM rows: at least one full 128-row tile
+    RLayout(int mb, int N, int Cp, int L) {
+        auto up = [](size_t x) { return (x + 1023) & ~(size_t)1023; };
+        const long rows = (long)mb * N;
+        rg = rows > MIN_ROWS ? rows : MIN_ROWS;
+        layer_img = (size_t)(relgcn_ftiles(Cp) + relgcn_btiles(Cp)) * WSLOT;
+        bias_off = (size_t)L * layer_img;
+        cs_off = up(bias_off + (size_t)L * Cp * sizeof(float));
+        mask_off = up(cs_off + (size_t)rows * sizeof(float));
+        deg_off = up(mask_off + 256 + (size_t)mb * 64 * N * ((N + 63) / 64));
+        ah_off = up(deg_off + (size_t)rg * 64 * sizeof(float));
+        x_off = up(ah_off + (size_t)rg * 4 * Cp * sizeof(float));
+        total = x_off + 2 * (size_t)rg * Cp * sizeof(float) + 1024;
+    }
+};
+
+struct PackRelgcn {
+    const float *Ws, *bs, *We, *be;       // (Cout, Cin), (Cout), (Cout * 4, Cin) rows c * 4 + e, (Cout * 4)
+    int Cin, Cout, Cp, first;             // first: tile of blockIdx.x 0 (the backward packs only its own tiles)
+    uint8_t *img;
+    float *bias;                          // (Cp) b_s zero-padded
+};
+
+// One layer's image: the forward job's k-tiles per 128-column chunk (h, AH_0 .. AH_3, the bias tile of deg), then the backward job's
+// (d, P_0 .. P_3).  B element (n = output column, k = column inside K-block b):
+//   forward   W_s[n][k] ; W_e[n][k] = We[(n*4 + e)*Cin + k] ; b_e[n*4 + k] (k < 4)
+//   backward  W_s[k][n] ; W_e[k][n]
+__global__ void __launch_bounds__(256) pack_relgcn_kernel(const PackRelgcn p) {
+    const int Cp = p.Cp, kb = Cp / 64, hc = (Cp + 127) / 128, NC = Cp < 128 ? Cp : 128;
+    const int tile = blockIdx.x + p.first;
+    const bool bwd = tile >= relgcn_ftiles(Cp);
+    const int per = 5 * kb + (bwd ? 0 : 1), local = bwd ? tile - relgcn_ftiles(Cp) : tile;
+    const int nc = local / per, kk = local % per, b = kk / kb, kbase = (kk % kb) * 64;
+    (void)hc;
+    auto val = [&](int n, int k) -> float {
+        if (!bwd) {
+            if (n >= p.Cout) return 0.f;
+            if (b == 5) return k < 4 && p.be ? p.be[(long)n * 4 + k] : 0.f;
+            if (k >= p.Cin) return 0.f;
+            return b == 0 ? p.Ws[(long)n * p.Cin + k] : p.We[((long)n * 4 + b - 1) * p.Cin + k];
+        }
+        if (n >= p.Cin || k >= p.Cout) return 0.f;
+        return b == 0 ? p.Ws[(long)k * p.Cin + n] : p.We[((long)k * 4 + b - 1) * p.Cin + n];
+    };
+    uint8_t *dst = p.img + (size_t)tile * WSLOT;
+    for (int idx = threadIdx.x; idx < NC * 8; idx += 256) {
+        const int n = idx % NC, c8 = idx / NC;
+        float v[8];
+#pragma unroll
+        for (int x = 0; x < 8; ++x) v[x] = val(nc * 128 + n, kbase + c8 * 8 + x);
+        uint32_t h[4], l[4];
+#pragma unroll
+        for (int x = 0; x < 4; ++x) {
+            h[x] = pack_bf16(v[2 * x], v[2 * x + 1]);
+            l[x] = pack_bf16(v[2 * x] - __uint_as_float(h[x] << 16), v[2 * x + 1] - __uint_as_float(h[x] & 0xFFFF0000u));
+        }
+        const uint32_t off = sw128(n, c8 * 8);
+        *reinterpret_cast<uint4 *>(dst + off) = make_uint4(h[0], h[1], h[2], h[3]);
+        *reinterpret_cast<uint4 *>(dst + PANEL_BYTES + off) = make_uint4(l[0], l[1], l[2], l[3]);
+    }
+    if (tile == 0)
+        for (int i = threadIdx.x; i < Cp; i += 256) p.bias[i] = i < p.Cout && p.bs ? p.bs[i] : 0.f;
+}
+
+// x[r][c] = h_0[r][c] for c < C0, 0 for the padded channels; h_0 = embed_W[clamp(atoms[r])] or h_in[r]
+__global__ void __launch_bounds__(256) relgcn_input_kernel(const int32_t *__restrict__ atoms, const float *__restrict__ embed_W, int n_types,
+                                                           const float *__restrict__ h_in, float *__restrict__ x, long rows, int C0, int Cp) {
+    for (long idx = (long)blockIdx.x * 256 + threadIdx.x; idx < rows * Cp; idx += (long)gridDim.x * 256) {
+        const long r = idx / Cp;
+        const int c = (int)(idx - r * Cp);
+        float v = 0.f;
+        if (c < C0) {
+            if (atoms) {
+                int id = atoms[r];
+                id = id < 0 ? 0 : (id >= n_types ? n_types - 1 : id);
+                v = __ldg(embed_W + (long)id * C0 + c);
+            } else {
+                v = __ldg(h_in + r * C0 + c);
+            }
+        }
+        x[idx] = v;
+    }
+}
+
+// d[r][c] = g[r][c] * act'(y[r][c]) for c < C (y = the layer output, row stride C; g row stride ldg), 0 for the padded channels
+__global__ void __launch_bounds__(256) relgcn_delta_kernel(const float *__restrict__ g, int ldg, const float *__restrict__ y,
+                                                           float *__restrict__ d, long rows, int C, int Cp, int act) {
+    const int CV = Cp / 4;
+    for (long idx = (long)blockIdx.x * 256 + threadIdx.x; idx < rows * CV; idx += (long)gridDim.x * 256) {
+        const long r = idx / CV;
+        const int c = (int)(idx - r * CV) * 4;
+        float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (c < C) {
+            const float4 gv = __ldg(reinterpret_cast<const float4 *>(g + r * ldg + c));
+            const float4 yv = __ldg(reinterpret_cast<const float4 *>(y + r * C + c));
+            o = make_float4(gv.x * act_bwd(act, yv.x, yv.x), gv.y * act_bwd(act, yv.y, yv.y), gv.z * act_bwd(act, yv.z, yv.z),
+                            gv.w * act_bwd(act, yv.w, yv.w));
+        }
+        *reinterpret_cast<float4 *>(d + r * Cp + c) = o;
+    }
+}
+
+// cs[mol][j] = 1 / sum_{e,i} A[mol][e][i][j] (1 where the sum is 0)
+__global__ void __launch_bounds__(256) relgcn_colscale_kernel(const float *__restrict__ adj, float *__restrict__ cs, int mb, int N) {
+    __shared__ float part[4][64], inv[BMP_X3_MAX_ATOMS];
+    for (int mol = blockIdx.x; mol < mb; mol += gridDim.x) {
+        column_inverse_degree(adj + (long)mol * 4 * N * N, 4, N, part, inv);
+        for (int j = threadIdx.x; j < N; j += 256) cs[(long)mol * N + j] = inv[j];
+    }
+}
+
+static int relgcn_cmax(const int *ch, int L) {
+    int c = 0;
+    for (int l = 0; l <= L; ++l) c = ch[l] > c ? ch[l] : c;
+    return c;
+}
+
+// (rows, C) row-major <- the first C columns of (rows, Cp)
+static int copy_cols(float *dst, int C, const float *src, int Cp, long rows, cudaStream_t st) {
+    if (cudaMemcpy2DAsync(dst, (size_t)C * sizeof(float), src, (size_t)Cp * sizeof(float), (size_t)C * sizeof(float), (size_t)rows,
+                          cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+        set_error("relgcn x3: cudaMemcpy2DAsync failed");
+        return BMP_ECUDA;
+    }
+    return BMP_OK;
+}
+
+// the adjacency side shared by forward and backward: bit masks + general-weight flag, and the column scales of rescale_adj
+static int relgcn_adjacency(const float *adj, int mb, int N, bool scale, uint8_t *ws, const RLayout &R, cudaStream_t st) {
+    int *flag = reinterpret_cast<int *>(ws + R.mask_off);
+    const int grid = mb < 8 * sm_count() ? mb : 8 * sm_count();
+    cudaMemsetAsync(flag, 0, 256, st);
+    adj_mask_kernel<<<grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(adj, reinterpret_cast<unsigned long long *>(ws + R.mask_off + 256),
+                                                                         flag, mb, N);
+    count_launch();
+    int rc;
+    if ((rc = check_launch("adj_mask_kernel"))) return rc;
+    if (scale) {
+        relgcn_colscale_kernel<<<grid, 256, 0, st>>>(adj, reinterpret_cast<float *>(ws + R.cs_off), mb, N);
+        count_launch();
+        if ((rc = check_launch("relgcn_colscale_kernel"))) return rc;
+    }
+    return BMP_OK;
+}
+
+static int relgcn_pack(const float *const *Ws, const float *const *bs, const float *const *We, const float *const *be, const int *ch,
+                       int L, int Cp, bool backward, uint8_t *ws, const RLayout &R, cudaStream_t st) {
+    for (int l = 0; l < L; ++l) {
+        PackRelgcn p;
+        p.Ws = Ws[l]; p.bs = bs ? bs[l] : nullptr; p.We = We[l]; p.be = be ? be[l] : nullptr;
+        p.Cin = ch[l]; p.Cout = ch[l + 1]; p.Cp = Cp;
+        p.first = backward ? relgcn_ftiles(Cp) : 0;
+        p.img = ws + (size_t)l * R.layer_img;
+        p.bias = reinterpret_cast<float *>(ws + R.bias_off) + (size_t)l * Cp;
+        pack_relgcn_kernel<<<backward ? relgcn_btiles(Cp) : relgcn_ftiles(Cp), 256, 0, st>>>(p);
+        count_launch();
+    }
+    return check_launch("pack_relgcn_kernel");
+}
+
+static int pointwise_grid(long n) {
+    const long g = (n + 255) / 256;
+    return (int)(g < 16L * sm_count() ? g : 16L * sm_count());
+}
+
+}  // namespace x3
+}  // namespace bmp
+
+// Bytes of workspace the RelGCN encoder needs on the tensor-core path (weight images, adjacency masks, per-layer temporaries at the
+// padded width); 0 = shape not covered.  The size is the same for training and inference.
+extern "C" size_t bmp_relgcn_x3_workspace_bytes(int mb, int n_atoms, int ch_max, int n_layers, int inference) {
+    (void)inference;
+    if (!relgcn_shape_ok(mb, n_atoms, ch_max, n_layers)) return 0;
+    return RLayout(mb, n_atoms, relgcn_cpad(ch_max), n_layers).total;
+}
+
+// "" when the call can take the tensor-core path, else why not (n_atoms and the channel count named)
+const char *bmp_relgcn_x3_refusal(int mb, int N, int E, int L, const int *ch, int act, const void *ws, size_t ws_bytes) {
+    static thread_local char why[256];
+    const int cmax = L > 0 && L <= BMP_MAX_STEPS ? relgcn_cmax(ch, L) : 0;
+    if (!relgcn_shape_ok(mb, N, cmax, L) || E != 4) {
+        snprintf(why, sizeof(why), "n_atoms=%d with %d channels and %d bond types: above %d atoms only 4 bond types, n_atoms <= %d and "
+                 "n_atoms * channels (rounded up to 64/128/256) * 4 bytes <= 160 KB are covered", N, cmax, E, BMP_MAX_ATOMS, BMP_X3_MAX_ATOMS);
+        return why;
+    }
+    if (act != BMP_ACT_IDENTITY && act != BMP_ACT_TANH) {
+        snprintf(why, sizeof(why), "n_atoms=%d: above %d atoms the activation must be identity or tanh", N, BMP_MAX_ATOMS);
+        return why;
+    }
+    const size_t need = RLayout(mb, N, relgcn_cpad(cmax), L).total;
+    if (!ws || ws_bytes < need) {
+        snprintf(why, sizeof(why), "n_atoms=%d (> %d) needs tc_workspace of bmp_relgcn_x3_workspace_bytes() = %zu bytes (got %zu)", N,
+                 BMP_MAX_ATOMS, need, ws ? ws_bytes : (size_t)0);
+        return why;
+    }
+    return "";
+}
+
+int bmp_relgcn_forward_x3(const bmp_relgcn_fwd_t *a, void *stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    const int N = a->n_atoms, L = a->n_layers, Cp = relgcn_cpad(relgcn_cmax(a->ch, L)), kb = Cp / 64, hc = (Cp + 127) / 128;
+    const long rows = (long)a->mb * N;
+    uint8_t *ws = (uint8_t *)(((uintptr_t)a->tc_workspace + 1023) & ~(uintptr_t)1023);
+    const RLayout R(a->mb, N, Cp, L);
+    const long rg = R.rg;
+    int rc;
+    if ((rc = relgcn_pack(a->self_W, a->self_b, a->edge_W, a->edge_b, a->ch, L, Cp, false, ws, R, st))) return rc;
+    if ((rc = relgcn_adjacency(a->adj, a->mb, N, a->scale_adj != 0, ws, R, st))) return rc;
+    float *deg = reinterpret_cast<float *>(ws + R.deg_off), *AH = reinterpret_cast<float *>(ws + R.ah_off);
+    float *X[2] = {reinterpret_cast<float *>(ws + R.x_off), reinterpret_cast<float *>(ws + R.x_off) + (size_t)rg * Cp};
+    cudaMemsetAsync(deg, 0, (size_t)rg * 64 * sizeof(float), st);
+    if (rg > rows) {       // rows of the padded tile: zero inputs (their outputs are never read)
+        cudaMemsetAsync(X[0] + (size_t)rows * Cp, 0, (size_t)(rg - rows) * Cp * sizeof(float), st);
+        cudaMemsetAsync(AH + (size_t)rows * 4 * Cp, 0, (size_t)(rg - rows) * 4 * Cp * sizeof(float), st);
+    }
+    relgcn_input_kernel<<<pointwise_grid(rows * Cp), 256, 0, st>>>(a->atoms, a->embed_W, a->n_atom_types, a->h_in, X[0], rows, a->ch[0], Cp);
+    count_launch();
+    if ((rc = check_launch("relgcn_input_kernel"))) return rc;
+    if (a->Hs && (rc = copy_cols(a->Hs, a->ch[0], X[0], Cp, rows, st))) return rc;
+    const size_t agg_smem = (size_t)N * Cp * sizeof(float);
+    cudaFuncSetAttribute(agg_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)agg_smem);
+    const int agg_grid = a->mb < 8 * sm_count() ? a->mb : 8 * sm_count();
+    const int *flag = reinterpret_cast<const int *>(ws + R.mask_off);
+    const unsigned long long *masks = reinterpret_cast<const unsigned long long *>(ws + R.mask_off + 256);
+    const float *cs = a->scale_adj ? reinterpret_cast<const float *>(ws + R.cs_off) : nullptr;
+    size_t hs_off = (size_t)rows * a->ch[0];
+    for (int l = 0; l < L; ++l) {
+        float *h = X[l & 1], *hn = X[(l + 1) & 1];
+        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, h, AH, l == 0 ? deg : nullptr, a->mb, N, Cp, cs);
+        count_launch();
+        if ((rc = check_launch("agg_kernel"))) return rc;
+        const uint8_t *img = ws + (size_t)l * R.layer_img;
+        const float *bias = reinterpret_cast<const float *>(ws + R.bias_off) + (size_t)l * Cp;
+        Args ga;
+        memset(&ga, 0, sizeof(ga));
+        ga.rows = rg; ga.NC = Cp < 128 ? Cp : 128; ga.njobs = hc;
+        for (int nc = 0; nc < hc; ++nc) {
+            Job &J = ga.job[nc];
+            J.nblk = 6;
+            J.A[0] = h; J.lda[0] = Cp; J.kt[0] = kb;
+            for (int e = 0; e < 4; ++e) { J.A[1 + e] = AH + (size_t)e * Cp; J.lda[1 + e] = 4 * Cp; J.kt[1 + e] = kb; }
+            J.A[5] = deg; J.lda[5] = 64; J.kt[5] = 1;
+            J.wimg = img + (size_t)nc * (5 * kb + 1) * WSLOT;
+            J.epi = a->act == BMP_ACT_TANH ? EPI_TANH : EPI_LIN;
+            J.bias = bias + nc * 128;
+            J.out0 = hn + nc * 128; J.lo0 = Cp;
+        }
+        if ((rc = launch_gemm(ga, st))) return rc;
+        const int Cout = a->ch[l + 1];
+        if (a->Hs && (rc = copy_cols(a->Hs + hs_off, Cout, hn, Cp, rows, st))) return rc;
+        if (l == L - 1 && a->h_out && (rc = copy_cols(a->h_out, Cout, hn, Cp, rows, st))) return rc;
+        hs_off += (size_t)rows * Cout;
+    }
+    return BMP_OK;
+}
+
+int bmp_relgcn_backward_x3(const bmp_relgcn_bwd_t *a, void *stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    const int N = a->n_atoms, L = a->n_layers, E = a->n_edge, Cp = relgcn_cpad(relgcn_cmax(a->ch, L)), kb = Cp / 64, hc = (Cp + 127) / 128;
+    const long rows = (long)a->mb * N;
+    uint8_t *ws = (uint8_t *)(((uintptr_t)a->tc_workspace + 1023) & ~(uintptr_t)1023);
+    const RLayout R(a->mb, N, Cp, L);
+    const long rg = R.rg;
+    int rc;
+    if ((rc = relgcn_pack(a->self_W, nullptr, a->edge_W, nullptr, a->ch, L, Cp, true, ws, R, st))) return rc;
+    if ((rc = relgcn_adjacency(a->adj, a->mb, N, a->scale_adj != 0, ws, R, st))) return rc;
+    float *P = reinterpret_cast<float *>(ws + R.ah_off);
+    float *D = reinterpret_cast<float *>(ws + R.x_off), *G = D + (size_t)rg * Cp;     // delta, gradient w.r.t. the layer input
+    if (rg > rows) {
+        cudaMemsetAsync(D + (size_t)rows * Cp, 0, (size_t)(rg - rows) * Cp * sizeof(float), st);
+        cudaMemsetAsync(P + (size_t)rows * 4 * Cp, 0, (size_t)(rg - rows) * 4 * Cp * sizeof(float), st);
+    }
+    const size_t agg_smem = (size_t)N * Cp * sizeof(float);
+    cudaFuncSetAttribute(agg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)agg_smem);
+    const int agg_grid = a->mb < 8 * sm_count() ? a->mb : 8 * sm_count();
+    const int *flag = reinterpret_cast<const int *>(ws + R.mask_off);
+    const unsigned long long *masks = reinterpret_cast<const unsigned long long *>(ws + R.mask_off + 256);
+    const float *cs = a->scale_adj ? reinterpret_cast<const float *>(ws + R.cs_off) : nullptr;
+    size_t hs_off[BMP_MAX_STEPS + 2];
+    hs_off[0] = 0;
+    for (int l = 0; l < L; ++l) hs_off[l + 1] = hs_off[l] + (size_t)rows * a->ch[l];
+    // C (Cout, Cin; ldc) += A[:, :Cout]^T h_l, dbias += column sums of A[:, :Cout]
+    auto WG = [&](const float *A_, int lda, const float *Hl, int Cin, int Cout, float *C_, int ldc, float *db, int dbs) -> int {
+        if (C_ && (Cin == 64 || Cin == 128 || Cin == 256)) return bmp_wgrad_tc3(A_, lda, Hl, Cin, C_, ldc, rows, Cout, Cin, db, dbs, stream);
+        int e_ = C_ ? bmp_wgrad(A_, lda, Hl, Cin, C_, ldc, rows, Cout, Cin, stream) : BMP_OK;
+        if (!e_ && db) e_ = bmp_colsum(A_, lda, db, dbs, rows, Cout, stream);
+        return e_;
+    };
+    for (int l = L - 1; l >= 0; --l) {
+        const int Cin = a->ch[l], Cout = a->ch[l + 1];
+        const float *g = l == L - 1 ? a->d_h_out : G;
+        relgcn_delta_kernel<<<pointwise_grid(rows * (Cp / 4)), 256, 0, st>>>(g, l == L - 1 ? Cout : Cp, a->Hs + hs_off[l + 1], D, rows, Cout,
+                                                                             Cp, a->act);
+        count_launch();
+        if ((rc = check_launch("relgcn_delta_kernel"))) return rc;
+        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, D, P, nullptr, a->mb, N, Cp, cs);
+        count_launch();
+        if ((rc = check_launch("agg_kernel"))) return rc;
+        const float *Hl = a->Hs + hs_off[l];
+        if ((rc = WG(D, Cp, Hl, Cin, Cout, a->d_self_W[l], Cin, a->d_self_b[l], 1))) return rc;
+        for (int e = 0; e < E; ++e)
+            if ((rc = WG(P + (size_t)e * Cp, 4 * Cp, Hl, Cin, Cout, a->d_edge_W[l] ? a->d_edge_W[l] + (size_t)e * Cin : nullptr, E * Cin,
+                         a->d_edge_b[l] ? a->d_edge_b[l] + e : nullptr, E)))
+                return rc;
+        if (l == 0 && !a->d_h0) break;
+        const uint8_t *img = ws + (size_t)l * R.layer_img + (size_t)relgcn_ftiles(Cp) * WSLOT;
+        Args ga;
+        memset(&ga, 0, sizeof(ga));
+        ga.rows = rg; ga.NC = Cp < 128 ? Cp : 128; ga.njobs = hc;
+        for (int nc = 0; nc < hc; ++nc) {
+            Job &J = ga.job[nc];
+            J.nblk = 5;
+            J.A[0] = D; J.lda[0] = Cp; J.kt[0] = kb;
+            for (int e = 0; e < 4; ++e) { J.A[1 + e] = P + (size_t)e * Cp; J.lda[1 + e] = 4 * Cp; J.kt[1 + e] = kb; }
+            J.wimg = img + (size_t)nc * 5 * kb * WSLOT;
+            J.epi = EPI_LIN;
+            J.out0 = G + nc * 128; J.lo0 = Cp;
+        }
+        if ((rc = launch_gemm(ga, st))) return rc;
+        if (l == 0 && (rc = copy_cols(a->d_h0, Cin, G, Cp, rows, st))) return rc;
     }
     return BMP_OK;
 }

@@ -177,30 +177,34 @@ __global__ void atoms_pool_bwd_kernel(const float *__restrict__ a, int a_ch, con
 
 // ---------------------------------------------------------------- GIN aggregation (models/gin.py:88-94)
 // out[b,i,:] = h[b,i,:] + sum_e sum_j A[b,e,i,j] h[b,j,:]   (TRANS: A[b,e,j,i] -- the backward with respect to h).
-// One CTA per molecule: the bond types are summed into a 64 x 64 tile in shared memory once, then every thread owns
-// channels c, c + blockDim.x, ... of all atoms, reading h rows from shared memory.
+// One CTA per molecule: h is staged in shared memory, the bond types are summed into a tile of RB output rows x N (all N rows
+// when they fit, up to 64 atoms), then every thread owns channels c, c + blockDim.x, ... of the tile's atoms.
 template <bool TRANS>
 __global__ void __launch_bounds__(256) gin_aggregate_kernel(const float *__restrict__ adj, const float *__restrict__ h,
-                                                            float *__restrict__ out, int mb, int E, int N, int H) {
+                                                            float *__restrict__ out, int mb, int E, int N, int H, int RB) {
     extern __shared__ float sm[];
-    float *As = sm;                 // [N][N+1]
-    float *hs = sm + N * (N + 1);   // [N][H]
+    float *As = sm;                  // [RB][N+1]
+    float *hs = sm + RB * (N + 1);   // [N][H]
     for (int b = blockIdx.x; b < mb; b += gridDim.x) {
-        for (int idx = threadIdx.x; idx < N * N; idx += blockDim.x) {
-            const int i = idx / N, j = idx - i * N;
-            float s = 0.f;
-            for (int e = 0; e < E; ++e) s += adj[(((long)b * E + e) * N + (TRANS ? j : i)) * N + (TRANS ? i : j)];
-            As[i * (N + 1) + j] = s;
-        }
         for (int idx = threadIdx.x; idx < N * H; idx += blockDim.x) hs[idx] = h[(long)b * N * H + idx];
-        __syncthreads();
-        for (int idx = threadIdx.x; idx < N * H; idx += blockDim.x) {
-            const int i = idx / H, c = idx - i * H;
-            float s = hs[idx];
-            for (int j = 0; j < N; ++j) s = fmaf(As[i * (N + 1) + j], hs[j * H + c], s);
-            out[(long)b * N * H + idx] = s;
+        for (int i0 = 0; i0 < N; i0 += RB) {
+            const int rb = N - i0 < RB ? N - i0 : RB;
+            for (int idx = threadIdx.x; idx < rb * N; idx += blockDim.x) {
+                // consecutive threads read consecutive addresses of the adjacency
+                const int i = TRANS ? idx % rb : idx / N, j = TRANS ? idx / rb : idx % N;
+                float s = 0.f;
+                for (int e = 0; e < E; ++e) s += adj[(((long)b * E + e) * N + (TRANS ? j : i0 + i)) * N + (TRANS ? i0 + i : j)];
+                As[i * (N + 1) + j] = s;
+            }
+            __syncthreads();
+            for (int idx = threadIdx.x; idx < rb * H; idx += blockDim.x) {
+                const int i = idx / H, c = idx - i * H;
+                float s = hs[(i0 + i) * H + c];
+                for (int j = 0; j < N; ++j) s = fmaf(As[i * (N + 1) + j], hs[j * H + c], s);
+                out[(long)b * N * H + (long)(i0 + i) * H + c] = s;
+            }
+            __syncthreads();
         }
-        __syncthreads();
     }
 }
 
@@ -209,20 +213,20 @@ __global__ void __launch_bounds__(256) gin_aggregate_kernel(const float *__restr
 // degree[b,i] = sum_{i'} adj[b,i',i] (nfp.py:152: xp.sum(adj, axis=1)).  The D degree-specific GraphLinears of the reference,
 // each applied to where(deg == d, fv, 0), are then ONE Linear over X with the weights concatenated along the input axis (and
 // all D biases added to every atom, as the reference's zero-masked inputs still pick up every bias).
-// One CTA per molecule; adj (N x N) and h (N x C) staged in shared memory.  BWD: dfv = the degree block of dX, dh = adj^T dfv.
+// One CTA per molecule; h (N x C) staged in shared memory, adj (forward) or adj^T (backward) in tiles of RB output rows x N (all N
+// rows when they fit, up to 64 atoms).  BWD: dfv = the degree block of dX, dh = adj^T dfv.
 template <bool BWD>
 __global__ void __launch_bounds__(256) nfp_gather_kernel(const float *__restrict__ adj, const float *__restrict__ src,
-                                                         float *__restrict__ dst, int mb, int N, int C, int D) {
+                                                         float *__restrict__ dst, int mb, int N, int C, int D, int RB) {
     extern __shared__ float sm[];
-    float *As = sm;                       // [N][N+1]
-    float *hs = As + N * (N + 1);         // [N][C]   forward: h ; backward: dfv
+    float *As = sm;                       // [RB][N+1]  rows i0.. of adj (forward) or of adj^T (backward)
+    float *hs = As + RB * (N + 1);        // [N][C]   forward: h ; backward: dfv
     int *deg = reinterpret_cast<int *>(hs + N * C);   // [N] degree block index (0..D-1) or -1
     for (int b = blockIdx.x; b < mb; b += gridDim.x) {
-        for (int idx = threadIdx.x; idx < N * N; idx += blockDim.x) As[(idx / N) * (N + 1) + idx % N] = adj[(long)b * N * N + idx];
-        __syncthreads();
+        const float *Ab = adj + (long)b * N * N;
         for (int i = threadIdx.x; i < N; i += blockDim.x) {
             float s = 0.f;
-            for (int r = 0; r < N; ++r) s += As[r * (N + 1) + i];
+            for (int r = 0; r < N; ++r) s += Ab[(long)r * N + i];
             int d = -1;
             for (int k = 1; k <= D; ++k)
                 if (s - (float)k == 0.f) d = k - 1;
@@ -231,31 +235,47 @@ __global__ void __launch_bounds__(256) nfp_gather_kernel(const float *__restrict
         __syncthreads();
         if (!BWD) {
             for (int idx = threadIdx.x; idx < N * C; idx += blockDim.x) hs[idx] = src[(long)b * N * C + idx];
-            __syncthreads();
-            float *X = dst + (long)b * N * D * C;
-            for (int idx = threadIdx.x; idx < N * D * C; idx += blockDim.x) {
-                const int i = idx / (D * C), r = idx - i * D * C, d = r / C, c = r - d * C;
-                float v = 0.f;
-                if (d == deg[i])
-                    for (int j = 0; j < N; ++j) v = fmaf(As[i * (N + 1) + j], hs[j * C + c], v);
-                X[idx] = v;
-            }
         } else {
             const float *dX = src + (long)b * N * D * C;
             for (int idx = threadIdx.x; idx < N * C; idx += blockDim.x) {
                 const int i = idx / C, c = idx - i * C;
                 hs[idx] = deg[i] >= 0 ? dX[(long)i * D * C + deg[i] * C + c] : 0.f;
             }
-            __syncthreads();
-            for (int idx = threadIdx.x; idx < N * C; idx += blockDim.x) {
-                const int j = idx / C, c = idx - j * C;
-                float v = 0.f;
-                for (int i = 0; i < N; ++i) v = fmaf(As[i * (N + 1) + j], hs[i * C + c], v);
-                dst[(long)b * N * C + idx] = v;
-            }
         }
-        __syncthreads();
+        for (int i0 = 0; i0 < N; i0 += RB) {
+            const int rb = N - i0 < RB ? N - i0 : RB;
+            for (int idx = threadIdx.x; idx < rb * N; idx += blockDim.x) {
+                const int i = BWD ? idx % rb : idx / N, j = BWD ? idx / rb : idx % N;
+                As[i * (N + 1) + j] = BWD ? Ab[(long)j * N + i0 + i] : Ab[(long)(i0 + i) * N + j];
+            }
+            __syncthreads();
+            if (!BWD) {
+                float *X = dst + (long)b * N * D * C + (long)i0 * D * C;
+                for (int idx = threadIdx.x; idx < rb * D * C; idx += blockDim.x) {
+                    const int i = idx / (D * C), r = idx - i * D * C, d = r / C, c = r - d * C;
+                    float v = 0.f;
+                    if (d == deg[i0 + i])
+                        for (int j = 0; j < N; ++j) v = fmaf(As[i * (N + 1) + j], hs[j * C + c], v);
+                    X[idx] = v;
+                }
+            } else {
+                for (int idx = threadIdx.x; idx < rb * C; idx += blockDim.x) {
+                    const int jj = idx / C, c = idx - jj * C;
+                    float v = 0.f;
+                    for (int i = 0; i < N; ++i) v = fmaf(As[jj * (N + 1) + i], hs[i * C + c], v);
+                    dst[(long)b * N * C + (long)(i0 + jj) * C + c] = v;
+                }
+            }
+            __syncthreads();
+        }
     }
+}
+
+// rows of the adjacency tile that fit next to the `fixed` floats: all N when they fit, else as many as fit (0: none)
+static int adjacency_tile_rows(int N, size_t fixed) {
+    const size_t cap = 227 * 1024 / sizeof(float);
+    if (fixed + (size_t)N * (N + 1) <= cap) return N;
+    return fixed >= cap ? 0 : (int)((cap - fixed) / (N + 1) < (size_t)N ? (cap - fixed) / (N + 1) : N);
 }
 
 __global__ void embed_fwd_kernel(const int32_t *__restrict__ ids, const float *__restrict__ W, float *__restrict__ out, long rows,
@@ -431,17 +451,18 @@ extern "C" int bmp_gin_aggregate(const float *adj, const float *h, float *out, i
                                  int transpose, void *stream) {
     if (!adj || !h || !out) { set_error("bmp_gin_aggregate: null pointer"); return BMP_EINVAL; }
     if (mb <= 0) return BMP_OK;
-    if (n_atoms <= 0 || n_atoms > BMP_MAX_ATOMS || hidden <= 0 || n_edge <= 0) { set_error("bmp_gin_aggregate: bad shape N=%d H=%d E=%d", n_atoms, hidden, n_edge); return BMP_ESHAPE; }
-    const size_t smem = sizeof(float) * ((size_t)n_atoms * (n_atoms + 1) + (size_t)n_atoms * hidden);
-    if (smem > 227 * 1024) { set_error("bmp_gin_aggregate: hidden=%d needs %zu B of shared memory", hidden, smem); return BMP_ESHAPE; }
+    if (n_atoms <= 0 || n_atoms > BMP_X3_MAX_ATOMS || hidden <= 0 || n_edge <= 0) { set_error("bmp_gin_aggregate: bad shape n_atoms=%d H=%d E=%d", n_atoms, hidden, n_edge); return BMP_ESHAPE; }
+    const int RB = adjacency_tile_rows(n_atoms, (size_t)n_atoms * hidden);
+    if (RB < 8) { set_error("bmp_gin_aggregate: n_atoms=%d, hidden=%d do not fit in shared memory", n_atoms, hidden); return BMP_ESHAPE; }
+    const size_t smem = sizeof(float) * ((size_t)RB * (n_atoms + 1) + (size_t)n_atoms * hidden);
     const int grid = mb < 148 * 4 ? mb : 148 * 4;
     cudaStream_t st = (cudaStream_t)stream;
     if (transpose) {
         cudaFuncSetAttribute(gin_aggregate_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        gin_aggregate_kernel<true><<<grid, 256, smem, st>>>(adj, h, out, mb, n_edge, n_atoms, hidden);
+        gin_aggregate_kernel<true><<<grid, 256, smem, st>>>(adj, h, out, mb, n_edge, n_atoms, hidden, RB);
     } else {
         cudaFuncSetAttribute(gin_aggregate_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        gin_aggregate_kernel<false><<<grid, 256, smem, st>>>(adj, h, out, mb, n_edge, n_atoms, hidden);
+        gin_aggregate_kernel<false><<<grid, 256, smem, st>>>(adj, h, out, mb, n_edge, n_atoms, hidden, RB);
     }
     count_launch();
     return check_launch("gin_aggregate_kernel");
@@ -451,17 +472,18 @@ extern "C" int bmp_nfp_gather(const float *adj, const float *src, float *dst, in
                               int backward, void *stream) {
     if (!adj || !src || !dst) { set_error("bmp_nfp_gather: null pointer"); return BMP_EINVAL; }
     if (mb <= 0) return BMP_OK;
-    if (n_atoms <= 0 || n_atoms > BMP_MAX_ATOMS || ch <= 0 || n_degree <= 0) { set_error("bmp_nfp_gather: bad shape N=%d C=%d D=%d", n_atoms, ch, n_degree); return BMP_ESHAPE; }
-    const size_t smem = sizeof(float) * ((size_t)n_atoms * (n_atoms + 1) + (size_t)n_atoms * ch + n_atoms);
-    if (smem > 227 * 1024) { set_error("bmp_nfp_gather: channels=%d needs %zu B of shared memory", ch, smem); return BMP_ESHAPE; }
+    if (n_atoms <= 0 || n_atoms > BMP_X3_MAX_ATOMS || ch <= 0 || n_degree <= 0) { set_error("bmp_nfp_gather: bad shape n_atoms=%d C=%d D=%d", n_atoms, ch, n_degree); return BMP_ESHAPE; }
+    const int RB = adjacency_tile_rows(n_atoms, (size_t)n_atoms * ch + n_atoms);
+    if (RB < 8) { set_error("bmp_nfp_gather: n_atoms=%d, channels=%d do not fit in shared memory", n_atoms, ch); return BMP_ESHAPE; }
+    const size_t smem = sizeof(float) * ((size_t)RB * (n_atoms + 1) + (size_t)n_atoms * ch + n_atoms);
     const int grid = mb < 148 * 4 ? mb : 148 * 4;
     cudaStream_t st = (cudaStream_t)stream;
     if (backward) {
         cudaFuncSetAttribute(nfp_gather_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        nfp_gather_kernel<true><<<grid, 256, smem, st>>>(adj, src, dst, mb, n_atoms, ch, n_degree);
+        nfp_gather_kernel<true><<<grid, 256, smem, st>>>(adj, src, dst, mb, n_atoms, ch, n_degree, RB);
     } else {
         cudaFuncSetAttribute(nfp_gather_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        nfp_gather_kernel<false><<<grid, 256, smem, st>>>(adj, src, dst, mb, n_atoms, ch, n_degree);
+        nfp_gather_kernel<false><<<grid, 256, smem, st>>>(adj, src, dst, mb, n_atoms, ch, n_degree, RB);
     }
     count_launch();
     return check_launch("nfp_gather_kernel");

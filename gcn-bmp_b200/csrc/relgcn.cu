@@ -182,9 +182,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) relgcn_bwd_kernel(const bmp_relgc
     }
 }
 
-static int relgcn_check(int mb, int N, int E, int L, const int *ch, int *cmax) {
+static int relgcn_check(int mb, int N, int E, int L, const int *ch, int *cmax, int max_atoms) {
     if (mb <= 0 || L <= 0 || L > BMP_MAX_STEPS) { set_error("relgcn: bad mb=%d or n_layers=%d", mb, L); return BMP_ESHAPE; }
-    if (N <= 0 || N > BMP_MAX_ATOMS) { set_error("relgcn: n_atoms=%d outside 1..%d", N, BMP_MAX_ATOMS); return BMP_ESHAPE; }
+    if (N <= 0 || N > max_atoms) { set_error("relgcn: n_atoms=%d outside 1..%d", N, max_atoms); return BMP_ESHAPE; }
     if (E <= 0 || E > 8) { set_error("relgcn: n_edge=%d outside 1..8", E); return BMP_ESHAPE; }
     *cmax = 0;
     for (int l = 0; l <= L; ++l) {
@@ -204,14 +204,20 @@ using namespace bmp;
 bool bmp_relgcn_tc_supported(const int *ch, int n_layers, int n_edge);   // relgcn_tc.cu
 int bmp_relgcn_forward_tc(const bmp_relgcn_fwd_t *a, void *stream);
 int bmp_relgcn_backward_tc(const bmp_relgcn_bwd_t *a, void *stream);
+// ggnn_x3.cu: BMP_MODE_F32 above BMP_MAX_ATOMS atoms
+const char *bmp_relgcn_x3_refusal(int mb, int N, int E, int L, const int *ch, int act, const void *ws, size_t ws_bytes);
+int bmp_relgcn_forward_x3(const bmp_relgcn_fwd_t *a, void *stream);
+int bmp_relgcn_backward_x3(const bmp_relgcn_bwd_t *a, void *stream);
 
 extern "C" int bmp_relgcn_forward(const bmp_relgcn_fwd_t *a, void *stream) {
     if (!a || !a->adj || (!a->atoms && !a->h_in) || (a->atoms && !a->embed_W)) {
         set_error("bmp_relgcn_forward: null argument");
         return BMP_EINVAL;
     }
+    // BMP_MODE_F32 molecules with more than BMP_MAX_ATOMS atoms: the tensor-core row path of ggnn_x3.cu
+    const bool x3 = a->mode == BMP_MODE_F32 && a->n_atoms > BMP_MAX_ATOMS;
     int cmax = 0;
-    int rc = relgcn_check(a->mb, a->n_atoms, a->n_edge, a->n_layers, a->ch, &cmax);
+    int rc = relgcn_check(a->mb, a->n_atoms, a->n_edge, a->n_layers, a->ch, &cmax, x3 ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
     if (rc) return rc;
     for (int l = 0; l < a->n_layers; ++l)
         if (!a->self_W[l] || !a->edge_W[l] || !aligned16({a->self_W[l], a->edge_W[l]})) {
@@ -227,6 +233,11 @@ extern "C" int bmp_relgcn_forward(const bmp_relgcn_fwd_t *a, void *stream) {
         return bmp_relgcn_forward_tc(a, stream);
     }
     if (a->adj_u8) { set_error("bmp_relgcn_forward: a byte adjacency needs BMP_MODE_BF16"); return BMP_EINVAL; }
+    if (x3) {
+        const char *why = bmp_relgcn_x3_refusal(a->mb, a->n_atoms, a->n_edge, a->n_layers, a->ch, a->act, a->tc_workspace, a->tc_workspace_bytes);
+        if (*why) { set_error("relgcn: %s", why); return BMP_ESHAPE; }
+        return bmp_relgcn_forward_x3(a, stream);
+    }
     size_t smem = sizeof(float) * ((size_t)2 * cmax * AT + AT * AT + 8 * AT + AT + STAGE_FLOATS);
     int grid = a->mb < 148 ? a->mb : 148;
     cudaStream_t st = (cudaStream_t)stream;
@@ -253,12 +264,14 @@ extern "C" int bmp_relgcn_backward(const bmp_relgcn_bwd_t *a, void *stream) {
         return bmp_relgcn_backward_tc(a, stream);
     }
     if (a && a->adj_u8) { set_error("bmp_relgcn_backward: a byte adjacency needs BMP_MODE_BF16"); return BMP_EINVAL; }
-    if (!a || !a->adj || !a->Hs || !a->d_h_out || !a->Ds || !a->Ps) {
+    // the tensor-core path (more than BMP_MAX_ATOMS atoms) keeps its temporaries in tc_workspace: Ds and Ps are not used there
+    const bool x3 = a && a->mode == BMP_MODE_F32 && a->n_atoms > BMP_MAX_ATOMS;
+    if (!a || !a->adj || !a->Hs || !a->d_h_out || (!x3 && (!a->Ds || !a->Ps))) {
         set_error("bmp_relgcn_backward: null argument");
         return BMP_EINVAL;
     }
     int cmax = 0;
-    int rc = relgcn_check(a->mb, a->n_atoms, a->n_edge, a->n_layers, a->ch, &cmax);
+    int rc = relgcn_check(a->mb, a->n_atoms, a->n_edge, a->n_layers, a->ch, &cmax, x3 ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
     if (rc) return rc;
     const int L = a->n_layers, E = a->n_edge;
     for (int l = 0; l < L; ++l)
@@ -267,6 +280,11 @@ extern "C" int bmp_relgcn_backward(const bmp_relgcn_bwd_t *a, void *stream) {
             return BMP_EINVAL;
         }
     if (!aligned16({a->Hs, a->d_h_out, a->Ds, a->Ps, a->d_h0})) { set_error("bmp_relgcn_backward: buffers must be 16-byte aligned"); return BMP_EINVAL; }
+    if (x3) {
+        const char *why = bmp_relgcn_x3_refusal(a->mb, a->n_atoms, a->n_edge, a->n_layers, a->ch, a->act, a->tc_workspace, a->tc_workspace_bytes);
+        if (*why) { set_error("relgcn: %s", why); return BMP_ESHAPE; }
+        return bmp_relgcn_backward_x3(a, stream);
+    }
     size_t smem = sizeof(float) * ((size_t)2 * cmax * AT + AT * AT + AT + STAGE_FLOATS);
     int grid = a->mb < 148 ? a->mb : 148;
     cudaStream_t st = (cudaStream_t)stream;

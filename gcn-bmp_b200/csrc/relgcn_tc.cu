@@ -540,19 +540,9 @@ static size_t image_bytes(int H) { return (size_t)(5 * (H / 64)) * H * 128 + 256
 
 // adj_out[b,e,i,j] = adj[b,e,i,j] / max-safe(sum_{e',i'} adj[b,e',i',j])   (models/relgcn.py:20-28)
 __global__ void __launch_bounds__(256) rescale_adj_kernel(const float *__restrict__ adj, float *__restrict__ out, int E, int N) {
-    __shared__ float part[4][BMP_MAX_ATOMS], inv[BMP_MAX_ATOMS];
+    __shared__ float part[4][64], inv[BMP_X3_MAX_ATOMS];
     const long base = (long)blockIdx.x * E * N * N;
-    const int j = threadIdx.x & 63, p = threadIdx.x >> 6;
-    float s = 0.f;
-    if (j < N)
-        for (int r = p; r < E * N; r += 4) s += __ldg(adj + base + (long)r * N + j);
-    part[p][j] = s;
-    __syncthreads();
-    if (threadIdx.x < N) {
-        const float t = (part[0][threadIdx.x] + part[1][threadIdx.x]) + (part[2][threadIdx.x] + part[3][threadIdx.x]);
-        inv[threadIdx.x] = t != 0.f ? 1.f / t : 1.f;
-    }
-    __syncthreads();
+    column_inverse_degree(adj + base, E, N, part, inv);
     for (int i = threadIdx.x; i < E * N * N; i += blockDim.x) out[base + i] = __ldg(adj + base + i) * inv[i % N];
 }
 
@@ -564,7 +554,8 @@ using namespace bmp;
 int bmp_wgrad_panels(bmp::w2::Args &k, void *stream);   // wgrad_tc2.cu
 
 extern "C" int bmp_rescale_adj(const float *adj, float *adj_out, int mb, int n_edge, int n_atoms, void *stream) {
-    if (!adj || !adj_out || mb <= 0 || n_edge <= 0 || n_atoms <= 0 || n_atoms > BMP_MAX_ATOMS) { set_error("bmp_rescale_adj: bad arguments"); return BMP_EINVAL; }
+    if (!adj || !adj_out || mb <= 0 || n_edge <= 0 || n_atoms <= 0) { set_error("bmp_rescale_adj: bad arguments"); return BMP_EINVAL; }
+    if (n_atoms > BMP_X3_MAX_ATOMS) { set_error("bmp_rescale_adj: n_atoms=%d outside 1..%d", n_atoms, BMP_X3_MAX_ATOMS); return BMP_ESHAPE; }
     rgt::rescale_adj_kernel<<<mb, 256, 0, (cudaStream_t)stream>>>(adj, adj_out, n_edge, n_atoms);
     count_launch();
     return check_launch("rescale_adj_kernel");

@@ -165,6 +165,7 @@ def _load():
     lib.bmp_readout_x3_workspace_bytes.argtypes, lib.bmp_readout_x3_workspace_bytes.restype = [i] * 6, C.c_size_t
     lib.bmp_coattn_tc_workspace_bytes.argtypes, lib.bmp_coattn_tc_workspace_bytes.restype = [i], C.c_size_t
     lib.bmp_relgcn_tc_workspace_bytes.argtypes, lib.bmp_relgcn_tc_workspace_bytes.restype = [i, i], C.c_size_t
+    lib.bmp_relgcn_x3_workspace_bytes.argtypes, lib.bmp_relgcn_x3_workspace_bytes.restype = [i] * 5, C.c_size_t
     lib.bmp_bimpm_workspace_bytes.argtypes, lib.bmp_bimpm_workspace_bytes.restype = [i, i, i, i, i], C.c_size_t
     lib.bmp_last_error.restype = C.c_char_p
     lib.bmp_version.restype = C.c_int
@@ -178,7 +179,7 @@ def _load():
 
 lib = _load()
 EXPORTS = ["bmp_ggnn_forward", "bmp_ggnn_backward", "bmp_embed_backward", "bmp_relgcn_forward",
-           "bmp_relgcn_backward", "bmp_relgcn_tc_workspace_bytes", "bmp_rescale_adj", "bmp_readout_forward", "bmp_readout_backward", "bmp_readout_tc_workspace_bytes", "bmp_coattn_forward",
+           "bmp_relgcn_backward", "bmp_relgcn_tc_workspace_bytes", "bmp_relgcn_x3_workspace_bytes", "bmp_rescale_adj", "bmp_readout_forward", "bmp_readout_backward", "bmp_readout_tc_workspace_bytes", "bmp_coattn_forward",
            "bmp_coattn_backward", "bmp_coattn_tc_workspace_bytes", "bmp_hole_corr_forward", "bmp_hole_corr_backward", "bmp_linear_forward",
            "bmp_linear_backward", "bmp_ggnn_tc_workspace_bytes", "bmp_ggnn_stash2_bytes", "bmp_ggnn_x3_workspace_bytes", "bmp_pair_workspace_bytes", "bmp_pair_forward_backward", "bmp_readout_x3_workspace_bytes", "bmp_wgrad", "bmp_wgrad_tc", "bmp_wgrad_tc3", "bmp_colsum", "bmp_sigmoid_ce", "bmp_adam_step",
            "bmp_pair_features_forward", "bmp_pair_features_backward", "bmp_bilinear_forward", "bmp_bilinear_backward", "bmp_grad_hooks",

@@ -309,9 +309,21 @@ class GGNNEncode(torch.autograd.Function):
         return (dx, None, d_state, None, None, None, None, None, None, None) + tuple(rets)
 
 
+def _relgcn_x3_workspace(a, mb, N, ch, dev):
+    """MODE_F32 with more than 64 atoms: the tensor-core row path's workspace (weight images + per-layer temporaries).  Shapes it
+    does not cover get none, and the library's error names n_atoms and the channel count."""
+    nbytes = int(K.lib.bmp_relgcn_x3_workspace_bytes(mb, N, max(ch), len(ch) - 1, 0))
+    if nbytes == 0:
+        return None
+    ws = torch.empty((nbytes,), device=dev, dtype=torch.uint8)
+    a.tc_workspace, a.tc_workspace_bytes = _p(ws), nbytes
+    return ws
+
+
 class RelGCNEncode(torch.autograd.Function):
     """embed -> [rescale_adj] -> L x tanh(RelGCNUpdate).  params = [embed_W or None] + L*(Ws,bs,We,be).
-    Returns the final atom states (mb, N, ch[L])."""
+    Returns the final atom states (mb, N, ch[L]).  In MODE_F32 molecules of 65..256 atoms run on the tensor-core row path
+    (csrc/ggnn_x3.cu), at most 64 on the one-CTA-per-molecule FFMA kernels."""
 
     @staticmethod
     def forward(ctx, x, adj, ch, scale_adj, act, want_stash, mode, *params):
@@ -352,29 +364,34 @@ class RelGCNEncode(torch.autograd.Function):
         elif want_stash:
             Hs = torch.empty((rows * sum(ch),), device=adj.device, dtype=torch.float32)
             a.Hs = _p(Hs)
+        x3 = mode == K.MODE_F32 and N > MAX_KERNEL_ATOMS
+        if x3:
+            ws = _relgcn_x3_workspace(a, mb, N, ch, adj.device)     # noqa: F841  (kept alive across the launch)
         K.check(K.lib.bmp_relgcn_forward(C.byref(a), _stream()))
         if want_stash:
             ctx.save_for_backward(x, adj, Hs, *params)
-            ctx.meta = (tuple(ch), int(bool(scale_adj)), act, is_ids, tc)
+            ctx.meta = (tuple(ch), int(bool(scale_adj)), act, is_ids, tc, x3)
         return h_out
 
     @staticmethod
     def backward(ctx, d_out):
         x, adj, Hs = ctx.saved_tensors[:3]
         params = ctx.saved_tensors[3:]
-        ch, scale_adj, act, is_ids, tc = ctx.meta
+        ch, scale_adj, act, is_ids, tc, x3 = ctx.meta
         mb, E, N, _ = adj.shape
         L = len(ch) - 1
         rows = mb * N
         dev = adj.device
         d_out = _f32(d_out)
         grads, rets = _grad_targets(params)
-        Ds = Ps = None
-        if not tc:
+        Ds = Ps = ws = None
+        if not tc and not x3:
             Ds = torch.empty((rows * sum(ch[1:]),), device=dev, dtype=torch.float32)
             Ps = torch.empty((rows * E * sum(ch[1:]),), device=dev, dtype=torch.float32)
         d_h0 = torch.empty((mb, N, ch[0]), device=dev, dtype=torch.float32)
         a = K.RelgcnBwd()
+        if x3:
+            ws = _relgcn_x3_workspace(a, mb, N, ch, dev)      # noqa: F841
         if tc:
             nbytes = int(K.lib.bmp_relgcn_tc_workspace_bytes(ch[0], L))
             ws, a.tc_images_ready = _tc_images("relgcn_bwd", nbytes, dev, params)

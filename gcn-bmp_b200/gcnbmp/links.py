@@ -303,6 +303,16 @@ class _GRU(Link):
                 c["U_z"].W, c["U_z"].b, c["W"].W, c["W"].b, c["U"].W, c["U"].b]
 
 
+def _relgcn_mode(mode, adj, n_atoms):
+    """(mode, adjacency) for a RelGCN encoder call: in BF16 mode a batch padded past 64 atoms runs the fp32 tensor-core row path
+    instead (the fused tcgen05 RelGCN kernels hold at most 64 atoms per molecule) -- more accurate, slower, same interface."""
+    if mode != K.MODE_BF16 or n_atoms <= Fn.MAX_KERNEL_ATOMS:
+        return mode, adj
+    if adj.dtype != torch.float32:
+        adj = Fn.unpack_adjacency(adj, n_atoms) if Fn.adj_format(adj) == 2 else adj.to(torch.float32)
+    return K.MODE_F32, adj
+
+
 def _encode(x, adj, state, plan, msgs, grus, embed_W, mode, keep_steps=False, mol_index=None):
     """Returns (states, last): states[0] = h_0, states[last] = h_T; every step is present only when
     `keep_steps` (or in fp32 mode with a tape) -- BF16 mode trains on a bf16 panel stash it keeps internally."""
@@ -368,7 +378,8 @@ class GGNNUpdate(Link):
 
 
 class RelGCNUpdate(Link):
-    """models/update/relgcn_update.py:12-44 -- one relational-GCN layer (no activation)."""
+    """models/update/relgcn_update.py:12-44 -- one relational-GCN layer (no activation).  In BF16 mode a batch wider than 64
+    atoms runs the fp32 tensor-core row path."""
 
     def __init__(self, in_channels, out_channels, num_edge_type=4):
         Link.__init__(self)
@@ -383,8 +394,9 @@ class RelGCNUpdate(Link):
     def __call__(self, h, adj):
         # the bare link has no activation (the tanh lives in models/relgcn.py:70-71)
         h, adj = _as_device(h, torch.float32), _adj_device(adj, self.__dict__.get("mode", K.MODE_F32))
+        mode, adj = _relgcn_mode(self.__dict__.get("mode", K.MODE_F32), adj, h.shape[1])
         return Fn.RelGCNEncode.apply(h, adj, (self.in_channels, self.out_channels), 0, K.ACT["identity"],
-                                     torch.is_grad_enabled(), self.__dict__.get("mode", K.MODE_F32), None, *self.tensors())
+                                     torch.is_grad_enabled(), mode, None, *self.tensors())
 
 
 class GGNNReadout(Link):
@@ -542,7 +554,8 @@ class GGNNMono(Link):
 
 class RelGCN(Link):
     """models/relgcn.py:31-73 -- embed -> (rescale_adj) -> [tanh(RelGCNUpdate)] x L ->
-    GGNNReadout(nobias, tanh) with h0=None."""
+    GGNNReadout(nobias, tanh) with h0=None.  Molecules of up to 64 atoms run on the fused per-molecule kernels, 65..256 on the
+    fp32 tensor-core row path (csrc/ggnn_x3.cu); in BF16 mode a batch padded past 64 atoms is routed to that fp32 path."""
 
     def __init__(self, out_channels=64, num_edge_type=4, ch_list=None,
                  n_atom_types=MAX_ATOMIC_NUM, input_type='int', scale_adj=None):
@@ -576,6 +589,7 @@ class RelGCN(Link):
         for c in self.rgcn_convs:
             params += c.tensors()
         mode, ch = self.__dict__.get("mode", K.MODE_F32), tuple(self.ch_list)
+        mode, adj = _relgcn_mode(mode, adj, x.shape[1])
         if mode == K.MODE_BF16 and len(set(ch)) > 1 and max(ch) <= 128 and self.num_edge_type == 4:
             # The tcgen05 RelGCN kernels take ONE channel count (64 or 128) for all layers; a non-uniform list such as the reference's
             # default [16, 128, 64] runs on them zero-padded to the widest layer (parameter re-packing: padded input columns meet zero

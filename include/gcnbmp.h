@@ -34,8 +34,9 @@ extern "C" {
 
 #define BMP_MAX_STEPS   16
 #define BMP_MAX_ATOMS   64   /* padded atoms per molecule handled by one CTA */
-#define BMP_X3_MAX_ATOMS 256 /* GGNN encoder in BMP_MODE_F32 with the tensor-core workspace (bmp_ggnn_x3_workspace_bytes): its
-                               row GEMMs never see molecule boundaries; n_atoms * hidden * 4 bytes <= 160 KB */
+#define BMP_X3_MAX_ATOMS 256 /* GGNN and RelGCN encoders in BMP_MODE_F32 with the tensor-core workspace (bmp_ggnn_x3_workspace_bytes,
+                               bmp_relgcn_x3_workspace_bytes): their row GEMMs never see molecule boundaries; n_atoms * hidden * 4
+                               bytes <= 160 KB.  Also the limit of bmp_rescale_adj, bmp_gin_aggregate and bmp_nfp_gather */
 #define BMP_MAX_HIDDEN 256
 
 /* activations (chainer.functions.{identity,tanh,relu,sigmoid}) */
@@ -186,6 +187,14 @@ typedef struct {
 
 int bmp_relgcn_forward(const bmp_relgcn_fwd_t *a, void *stream);
 size_t bmp_relgcn_tc_workspace_bytes(int channels, int n_layers);   /* 0 = channel count not on the tcgen05 path */
+/* BMP_MODE_F32 with 65 <= n_atoms <= BMP_X3_MAX_ATOMS (csrc/ggnn_x3.cu): bmp_relgcn_forward / bmp_relgcn_backward take the
+ * tensor-core row path -- per layer one adjacency product over bit masks and one split-bf16 GEMM (three UMMAs per product, fp32
+ * accumulate: the <= 1e-4 parity of the mode is kept) -- when tc_workspace / tc_workspace_bytes hold at least this many bytes.
+ * ch_max = the largest ch[l]: every layer runs zero-padded to it rounded up to 64, 128 or 256, which with n_atoms must satisfy
+ * n_atoms * padded channels * 4 bytes <= 160 KB; n_edge must be 4 and act identity or tanh.  Same Hs stash as the FFMA kernels;
+ * the backward takes a workspace of the same size (its contents need not be the forward's) and leaves Ds / Ps unused (they may
+ * be NULL).  Host-only; the size does not depend on `inference`.  0 = shape not covered (the FFMA kernels take n_atoms <= 64). */
+size_t bmp_relgcn_x3_workspace_bytes(int mb, int n_atoms, int ch_max, int n_layers, int inference);
 /* adj_out[b,e,i,j] = adj[b,e,i,j] / (sum_{e',i'} adj[b,e',i',j] or 1)   (rescale_adj, models/relgcn.py:20-28) */
 int bmp_rescale_adj(const float *adj, float *adj_out, int mb, int n_edge, int n_atoms, void *stream);
 
@@ -416,7 +425,8 @@ int bmp_atoms_pool_backward(const float *a, int a_ch, const float *z, const floa
                             int mb, int n_atoms, int ch, void *stream);
 
 /* GIN aggregation, models/gin.py:88-94: out[b,i,:] = h[b,i,:] + sum_e sum_j adj[b,e,i,j] h[b,j,:]; `transpose` != 0 uses
- * adj[b,e,j,i] instead -- the same call is the backward with respect to h (pass d_out as h).  fp32, N <= 64.            */
+ * adj[b,e,j,i] instead -- the same call is the backward with respect to h (pass d_out as h).  fp32, N <= 256 with
+ * N * hidden * 4 bytes well inside the 227 KB of shared memory of a block.                                              */
 int bmp_gin_aggregate(const float *adj, const float *h, float *out, int mb, int n_edge, int n_atoms, int hidden,
                       int transpose, void *stream);
 
@@ -460,7 +470,7 @@ int bmp_bimpm_backward(const bmp_bimpm_t *a, void *stream);
  *   forward  (backward == 0): src = h (mb,N,C) -> dst = X (mb,N,D*C), X[b,i,(d-1)C+c] = (adj[b] h[b])[i,c] if degree(b,i) == d
  *            (degree = column sums of adj, nfp.py:152; d = 1..D), else 0; the D degree-specific GraphLinears are then one
  *            Linear over X with their weights concatenated along the input axis and their biases summed;
- *   backward (backward != 0): src = dX -> dst = dh = adj[b]^T (degree block of dX).  fp32, N <= 64.                        */
+ *   backward (backward != 0): src = dX -> dst = dh = adj[b]^T (degree block of dX).  fp32, N <= 256.                       */
 int bmp_embed_forward(const int32_t *atoms, const float *embed_W, float *out, int rows, int hidden, int n_atom_types, void *stream);
 int bmp_nfp_gather(const float *adj, const float *src, float *dst, int mb, int n_atoms, int ch, int n_degree, int backward,
                    void *stream);
