@@ -515,14 +515,27 @@ __global__ void __launch_bounds__(NTHREADS, 1) coattn_bwd_kernel(const CoArgs A,
     if (tid == 0 && B.d_b) atomicAdd(B.d_b, gb[0]);
 }
 
-static int co_check(int mb, int n1, int n2, int H, int O, int head, int variant) {
+static int co_check(int mb, int n1, int n2, int H, int O, int head, int variant, const void *ws, size_t ws_bytes) {
     if (mb <= 0) return BMP_ESHAPE;
-    if (n1 <= 0 || n1 > BMP_MAX_ATOMS || n2 <= 0 || n2 > BMP_MAX_ATOMS) {
-        set_error("coattn: n1=%d n2=%d outside 1..%d", n1, n2, BMP_MAX_ATOMS);
+    if (n1 <= 0 || n1 > BMP_X3_MAX_ATOMS || n2 <= 0 || n2 > BMP_X3_MAX_ATOMS) {
+        set_error("coattn: n1=%d n2=%d outside 1..%d", n1, n2, BMP_X3_MAX_ATOMS);
         return BMP_ESHAPE;
     }
     if (H <= 0 || (H & 3) || O <= 0) { set_error("coattn: hidden=%d must be a positive multiple of 4, out_dim=%d > 0", H, O); return BMP_ESHAPE; }
     if (variant == BMP_COATTN_FINE && (head <= 0 || head > MAXHEAD)) { set_error("coattn: head=%d outside 1..%d", head, MAXHEAD); return BMP_ESHAPE; }
+    if (n1 > BMP_MAX_ATOMS || n2 > BMP_MAX_ATOMS) {     // coattn_big.cu: C^T and S in a per-CTA slice of the caller's workspace
+        const size_t need = bmp_coattn_large_workspace_bytes(n1, n2, H, variant == BMP_COATTN_FINE ? head : 0);
+        if (!need) {
+            set_error("coattn: n1=%d n2=%d hidden=%d: above %d atoms hidden must be a multiple of 4 <= 192", n1, n2, H, BMP_MAX_ATOMS);
+            return BMP_ESHAPE;
+        }
+        if (!ws || ws_bytes < need) {
+            set_error("coattn: n1=%d n2=%d hidden=%d needs a tc_workspace of %zu bytes (bmp_coattn_large_workspace_bytes), %zu given",
+                      n1, n2, H, need, ws ? ws_bytes : (size_t)0);
+            return BMP_ESHAPE;
+        }
+        return BMP_OK;
+    }
     if (co_smem_floats(H, head > 0 ? head : 1) * sizeof(float) > 227 * 1024) {
         set_error("coattn: hidden=%d does not fit the shared-memory resident kernel", H);
         return BMP_ESHAPE;
@@ -537,6 +550,7 @@ using namespace bmp;
 bool bmp_coattn_tc_supported(int H, int head, int variant, bool bwd);
 int bmp_coattn_forward_tc(const bmp_coattn_fwd_t *a, void *stream);
 int bmp_coattn_backward_tc(const bmp_coattn_bwd_t *a, void *stream);
+int bmp_coattn_big(const bmp_coattn_fwd_t *f, const bmp_coattn_bwd_t *bw, void *stream);   // coattn_big.cu: 65..256 atoms
 
 static long long *g_co_dbg = nullptr;
 extern "C" void bmp_debug_set_buffer_co(void *p) { g_co_dbg = (long long *)p; }
@@ -563,9 +577,10 @@ extern "C" int bmp_coattn_forward(const bmp_coattn_fwd_t *a, void *stream) {
         set_error("bmp_coattn_forward: null head parameters");
         return BMP_EINVAL;
     }
-    int rc = co_check(a->mb, a->n1, a->n2, a->hidden, a->out_dim, a->head, a->variant);
+    int rc = co_check(a->mb, a->n1, a->n2, a->hidden, a->out_dim, a->head, a->variant, a->tc_workspace, a->tc_workspace_bytes);
     if (rc) return rc;
     if (!aligned16({a->atoms_1, a->atoms_2, a->W})) { set_error("bmp_coattn_forward: atoms_1, atoms_2, W must be 16-byte aligned"); return BMP_EINVAL; }
+    if (a->n1 > BMP_MAX_ATOMS || a->n2 > BMP_MAX_ATOMS) return bmp_coattn_big(a, nullptr, stream);     // fp32 in either mode
     if (a->mode == BMP_MODE_BF16 && bmp_coattn_tc_supported(a->hidden, a->head, a->variant, false)) return bmp_coattn_forward_tc(a, stream);
     CoArgs A = make_args(a->mb, a->n1, a->n2, a->hidden, a->out_dim, a->head, a->variant, a->act, a->atoms_1, a->atoms_2,
                          a->W, a->V1, a->V2, a->b, a->lt_1, a->lt_2, a->wa_1, a->wa_2, a->W_j, a->b_j);
@@ -588,13 +603,16 @@ extern "C" int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream) {
         set_error("bmp_coattn_backward: null head parameters / workspaces");
         return BMP_EINVAL;
     }
-    int rc = co_check(a->mb, a->n1, a->n2, a->hidden, a->out_dim, a->head, a->variant);
+    int rc = co_check(a->mb, a->n1, a->n2, a->hidden, a->out_dim, a->head, a->variant, a->tc_workspace, a->tc_workspace_bytes);
     if (rc) return rc;
     if (a->hidden > BMP_MAX_HIDDEN) { set_error("coattn backward: hidden > %d", BMP_MAX_HIDDEN); return BMP_ESHAPE; }
     if (!aligned16({a->atoms_1, a->atoms_2, a->W, a->R, a->d_atoms_1, a->d_atoms_2})) { set_error("bmp_coattn_backward: buffers must be 16-byte aligned"); return BMP_EINVAL; }
-    const bool tc_data = a->mode == BMP_MODE_BF16 && bmp_coattn_tc_supported(a->hidden, a->head, a->variant, true);
+    const bool big = a->n1 > BMP_MAX_ATOMS || a->n2 > BMP_MAX_ATOMS;     // fp32 kernel and fp32 weight gradients in either mode
+    const bool tc_data = !big && a->mode == BMP_MODE_BF16 && bmp_coattn_tc_supported(a->hidden, a->head, a->variant, true);
     if (tc_data) {     // also accumulates d W, d lt_k, d V_k, d wa_k, d b inside the kernel
         if ((rc = bmp_coattn_backward_tc(a, stream))) return rc;
+    } else if (big) {
+        if ((rc = bmp_coattn_big(nullptr, a, stream))) return rc;
     } else {
         CoArgs A = make_args(a->mb, a->n1, a->n2, a->hidden, a->out_dim, a->head, a->variant, a->act, a->atoms_1, a->atoms_2,
                              a->W, a->V1, a->V2, a->b, a->lt_1, a->lt_2, a->wa_1, a->wa_2, a->W_j, a->b_j);
@@ -612,7 +630,7 @@ extern "C" int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream) {
     const int H = a->hidden, O = a->out_dim, hd = a->head;
     const long rows1 = (long)a->mb * a->n1, rows2 = (long)a->mb * a->n2;
     // d W[h][k] += sum_{pairs,j} a1[j][h] R[j][k]
-    const bool tcw = a->mode == BMP_MODE_BF16 && (H == 64 || H == 128 || H == 256);
+    const bool tcw = !big && a->mode == BMP_MODE_BF16 && (H == 64 || H == 128 || H == 256);
     auto WG = [&](const float *A_, int lda, const float *B_, float *C_, long r_, int M_) -> int {
         if (tcw && (M_ & 3) == 0) return bmp_wgrad_tc(A_, lda, B_, H, C_, H, r_, M_, H, nullptr, 1, stream);
         return bmp_wgrad(A_, lda, B_, H, C_, H, r_, M_, H, stream);

@@ -76,6 +76,8 @@ Plan make_plan(void *base, int mb, int n1, int n2, int H, int O, int head, int K
         const size_t b1 = bmp_ggnn_x3_workspace_bytes(mb, n1, H, 4, T, 0), b2 = bmp_ggnn_x3_workspace_bytes(mb, n2, H, 4, T, 0);
         pl.x3_bytes = (b1 && b2) ? (b1 > b2 ? b1 : b2) : 0;          // both drugs or neither: one image set serves both
         pl.x3_ws = pl.x3_bytes ? c.take<uint8_t>(pl.x3_bytes) : nullptr;
+        pl.co_bytes = bmp_coattn_large_workspace_bytes(n1, n2, H, head);     // 0 unless a molecule has more than 64 atoms
+        pl.co_ws = pl.co_bytes ? c.take<uint8_t>(pl.co_bytes) : nullptr;
     }
     pl.c1 = c.take<float>((size_t)mb * O); pl.c2 = c.take<float>((size_t)mb * O);
     pl.dc1 = c.take<float>((size_t)mb * O); pl.dc2 = c.take<float>((size_t)mb * O);

@@ -3,6 +3,10 @@
 // models/ggnn_dev.py:113-122; SUM: models/ggnn_dev.py:167.
 // One CTA per molecule; [h | h0] channel-major in shared memory; the two linears
 // run as 64x64 register tiles; the sum over atoms is a 16-lane shuffle reduction.
+// Molecules of up to BMP_X3_MAX_ATOMS atoms are walked in 64-atom chunks: the forward
+// carries the per-molecule sum across chunks in g, the backward needs no cross-chunk
+// state (an atom's gradient depends on dg and its own row only).  Up to 64 atoms there
+// is one chunk and the arithmetic is that of the single-tile kernel.
 #include "common.cuh"
 
 namespace bmp {
@@ -34,74 +38,82 @@ __global__ void __launch_bounds__(NTHREADS, 1) readout_kernel(const bmp_readout_
     float *stage = dv_s + (BWD ? O * AT : 0);
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4, i0 = tx * 4;
 
+    const int nchunks = (N + AT - 1) / AT;
     for (int mol = blockIdx.x; mol < mb; mol += gridDim.x) {
-        const long row0 = (long)mol * N;
-        __syncthreads();
-        load_cm(hcat, h + row0 * H, N, H);
-        if (h0) load_cm(hcat + H * AT, h0 + row0 * H, N, H);
-        __syncthreads();
-        float mk[4];
+        for (int ch = 0; ch < nchunks; ++ch) {
+            const long row0 = (long)mol * N + ch * AT;
+            const int n = min(AT, N - ch * AT);
+            __syncthreads();
+            load_cm(hcat, h + row0 * H, n, H);
+            if (h0) load_cm(hcat + H * AT, h0 + row0 * H, n, H);
+            __syncthreads();
+            float mk[4];
 #pragma unroll
-        for (int b = 0; b < 4; ++b) mk[b] = (i0 + b < N) ? (mask ? mask[row0 + i0 + b] : 1.f) : 0.f;
+            for (int b = 0; b < 4; ++b) mk[b] = (i0 + b < n) ? (mask ? mask[row0 + i0 + b] : 1.f) : 0.f;
 
-        for (int oc = 0; oc * 64 < O; ++oc) {
-            float au[4][4], av[4][4];
-            zero_acc(au);
-            zero_acc(av);
-            gemm64_g<false>(au, W_i, Ki, oc * 64, O, Ki, hcat, stage);
-            gemm64_g<false>(av, W_j, Kj, oc * 64, O, Kj, hcat, stage);
-            const int o0 = oc * 64 + ty * 4;
+            for (int oc = 0; oc * 64 < O; ++oc) {
+                float au[4][4], av[4][4];
+                zero_acc(au);
+                zero_acc(av);
+                gemm64_g<false>(au, W_i, Ki, oc * 64, O, Ki, hcat, stage);
+                gemm64_g<false>(av, W_j, Kj, oc * 64, O, Kj, hcat, stage);
+                const int o0 = oc * 64 + ty * 4;
 #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const bool live = o0 + q < O;
-                const float bi = (live && b_i) ? b_i[o0 + q] : 0.f, bj = (live && b_j) ? b_j[o0 + q] : 0.f;
-                if (!BWD) {
-                    float s = 0.f;
+                for (int q = 0; q < 4; ++q) {
+                    const bool live = o0 + q < O;
+                    const float bi = (live && b_i) ? b_i[o0 + q] : 0.f, bj = (live && b_j) ? b_j[o0 + q] : 0.f;
+                    if (!BWD) {
+                        float s = 0.f;
 #pragma unroll
-                    for (int b = 0; b < 4; ++b) s += mk[b] * sigmoidf_(au[q][b] + bi) * act_fwd(act, av[q][b] + bj);
-                    s = reduce16(s);
-                    if (tx == 0 && live) f.g[(long)mol * O + o0 + q] = act_fwd(act_agg, s);
-                } else {
-                    float dsum = 0.f;
-                    if (live) {
-                        float gout = bw.g[(long)mol * O + o0 + q];
-                        dsum = bw.dg[(long)mol * O + o0 + q] * act_bwd(act_agg, gout, gout);
-                        // relu on the aggregate: derivative through the output sign is exact (y>0 <=> x>0)
-                    }
+                        for (int b = 0; b < 4; ++b) s += mk[b] * sigmoidf_(au[q][b] + bi) * act_fwd(act, av[q][b] + bj);
+                        s = reduce16(s);
+                        if (tx == 0 && live) {     // partial sums of earlier chunks wait in g (same thread)
+                            float *gp = f.g + (long)mol * O + o0 + q;
+                            if (ch) s += *gp;
+                            *gp = ch + 1 == nchunks ? act_fwd(act_agg, s) : s;
+                        }
+                    } else {
+                        float dsum = 0.f;
+                        if (live) {
+                            float gout = bw.g[(long)mol * O + o0 + q];
+                            dsum = bw.dg[(long)mol * O + o0 + q] * act_bwd(act_agg, gout, gout);
+                            // relu on the aggregate: derivative through the output sign is exact (y>0 <=> x>0)
+                        }
 #pragma unroll
-                    for (int b = 0; b < 4; ++b) {
-                        float u = au[q][b] + bi, v = av[q][b] + bj;
-                        float su = sigmoidf_(u), av_ = act_fwd(act, v);
-                        au[q][b] = dsum * mk[b] * av_ * su * (1.f - su);
-                        av[q][b] = dsum * mk[b] * su * act_bwd(act, v, av_);
+                        for (int b = 0; b < 4; ++b) {
+                            float u = au[q][b] + bi, v = av[q][b] + bj;
+                            float su = sigmoidf_(u), av_ = act_fwd(act, v);
+                            au[q][b] = dsum * mk[b] * av_ * su * (1.f - su);
+                            av[q][b] = dsum * mk[b] * su * act_bwd(act, v, av_);
+                        }
                     }
                 }
+                if (BWD && o0 < O) {
+                    tile_store_s(du_s, oc * 64, au);
+                    tile_store_s(dv_s, oc * 64, av);
+                    tile_store_g(bw.DU + row0 * O, O, oc * 64, O, n, au);
+                    tile_store_g(bw.DV + row0 * O, O, oc * 64, O, n, av);
+                }
             }
-            if (BWD && o0 < O) {
-                tile_store_s(du_s, oc * 64, au);
-                tile_store_s(dv_s, oc * 64, av);
-                tile_store_g(bw.DU + row0 * O, O, oc * 64, O, N, au);
-                tile_store_g(bw.DV + row0 * O, O, oc * 64, O, N, av);
-            }
-        }
-        if (BWD) {
-            __syncthreads();
-            for (int kc = 0; kc * 64 < Kcat; ++kc) {
-                float d[4][4];
-                zero_acc(d);
-                gemm64_g<true>(d, W_i, Ki, kc * 64, Ki, O, du_s, stage);
-                if (kc * 64 < Kj) gemm64_g<true>(d, W_j, Kj, kc * 64, Kj, O, dv_s, stage);
-                // accumulate into dh (k < H) / dh0 (k >= H); a 64-chunk never straddles H unless H % 64 != 0
-                const int k0 = kc * 64 + ty * 4;
+            if (BWD) {
+                __syncthreads();
+                for (int kc = 0; kc * 64 < Kcat; ++kc) {
+                    float d[4][4];
+                    zero_acc(d);
+                    gemm64_g<true>(d, W_i, Ki, kc * 64, Ki, O, du_s, stage);
+                    if (kc * 64 < Kj) gemm64_g<true>(d, W_j, Kj, kc * 64, Kj, O, dv_s, stage);
+                    // accumulate into dh (k < H) / dh0 (k >= H); a 64-chunk never straddles H unless H % 64 != 0
+                    const int k0 = kc * 64 + ty * 4;
 #pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    if (i0 + b >= N) continue;
+                    for (int b = 0; b < 4; ++b) {
+                        if (i0 + b >= n) continue;
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        int k = k0 + q;
-                        if (k >= Kcat) continue;
-                        float *dst = (k < H) ? bw.dh : bw.dh0;
-                        if (dst) dst[(row0 + i0 + b) * H + (k < H ? k : k - H)] += d[q][b];
+                        for (int q = 0; q < 4; ++q) {
+                            int k = k0 + q;
+                            if (k >= Kcat) continue;
+                            float *dst = (k < H) ? bw.dh : bw.dh0;
+                            if (dst) dst[(row0 + i0 + b) * H + (k < H ? k : k - H)] += d[q][b];
+                        }
                     }
                 }
             }
@@ -132,7 +144,7 @@ __global__ void __launch_bounds__(NTHREADS) readout_sum_bwd_kernel(const float *
 static int readout_check(int mb, int N, int H, int O, int variant, const float *h) {
     if (!h) { set_error("readout: null h"); return BMP_EINVAL; }
     if (mb <= 0) return BMP_ESHAPE;
-    if (N <= 0 || N > BMP_MAX_ATOMS) { set_error("readout: n_atoms=%d outside 1..%d", N, BMP_MAX_ATOMS); return BMP_ESHAPE; }
+    if (N <= 0 || N > BMP_X3_MAX_ATOMS) { set_error("readout: n_atoms=%d outside 1..%d", N, BMP_X3_MAX_ATOMS); return BMP_ESHAPE; }
     if (H <= 0 || (H & 3) || H > BMP_MAX_HIDDEN) { set_error("readout: hidden=%d must be a multiple of 4 <= %d", H, BMP_MAX_HIDDEN); return BMP_ESHAPE; }
     if (variant != BMP_READOUT_SUM && (O <= 0 || (O & 3))) { set_error("readout: out_dim=%d must be a positive multiple of 4", O); return BMP_ESHAPE; }
     return BMP_OK;
@@ -163,7 +175,8 @@ extern "C" int bmp_readout_forward(const bmp_readout_fwd_t *a, void *stream) {
     }
     if (!a->W_i || !a->W_j) { set_error("bmp_readout_forward: null weights"); return BMP_EINVAL; }
     if (!aligned16({a->W_i, a->W_j, a->h, a->h0})) { set_error("bmp_readout_forward: h, h0, W_i, W_j must be 16-byte aligned"); return BMP_EINVAL; }
-    if (a->mode == BMP_MODE_BF16 && bmp_readout_tc_workspace_bytes(a->hidden, a->out_dim)) {
+    // BF16 mode above 64 atoms: the fp32 kernels (the tcgen05 read-out maps one molecule onto a 64-row tile)
+    if (a->mode == BMP_MODE_BF16 && a->n_atoms <= BMP_MAX_ATOMS && bmp_readout_tc_workspace_bytes(a->hidden, a->out_dim)) {
         return bmp_readout_tc(a->mb, a->n_atoms, a->hidden, a->out_dim, a->variant, a->act, a->act_agg, a->h, a->h0,
                               a->is_real_node, a->W_i, a->b_i, a->W_j, a->b_j, a->g, nullptr, nullptr, nullptr, nullptr, nullptr,
                               a->tc_workspace, a->tc_workspace_bytes, a->tc_images_ready != 0, false, stream);
@@ -197,7 +210,7 @@ extern "C" int bmp_readout_backward(const bmp_readout_bwd_t *a, void *stream) {
     if (!aligned16({a->W_i, a->W_j, a->h, a->h0, a->DU, a->DV, a->dh, a->dh0})) { set_error("bmp_readout_backward: buffers must be 16-byte aligned"); return BMP_EINVAL; }
     const int Kcat = a->h0 ? 2 * H : H;
     const int Kj = a->variant == BMP_READOUT_R2 ? H : Kcat;
-    const bool tc = a->mode == BMP_MODE_BF16 && H <= 128 && O <= 128 && bmp_readout_tc_workspace_bytes(H, O) != 0;   // 256: forward-only
+    const bool tc = a->mode == BMP_MODE_BF16 && a->n_atoms <= BMP_MAX_ATOMS && H <= 128 && O <= 128 && bmp_readout_tc_workspace_bytes(H, O) != 0;   // 256: forward-only
     if (tc) {
         if ((rc = bmp_readout_tc(a->mb, a->n_atoms, H, O, a->variant, a->act, a->act_agg, a->h, a->h0, a->is_real_node,
                                  a->W_i, a->b_i, a->W_j, a->b_j, const_cast<float *>(a->g), a->dg, a->DU, a->DV, a->dh, a->dh0,

@@ -437,11 +437,10 @@ def _readout_ws(a, mode, H, O, variant, dev, params):
 
 
 # ---- molecules with more than 64 atoms ---------------------------------------------------------------------------------
-# The hand-written read-out / co-attention kernels map one padded molecule (pair) of <= 64 atoms onto a CTA.  Larger molecules
-# (the reference pads to the batch maximum, ggnn_preprocessor.py:41 has no cap) take the same formulas composed from library
-# GEMMs (torch.matmul -> cuBLAS) with autograd; the GGNN encoder itself runs them on the fp32 tensor-core path (row GEMMs, any N
-# up to 256).  The same compositions take the widths the shared-memory-resident kernels cannot hold (co-attention hidden > 192,
-# read-out backward at hidden = out_dim = 256).  A functional path for real data, not a tuned one.
+# The reference pads to the batch maximum (ggnn_preprocessor.py:41 has no cap).  Above MAX_KERNEL_ATOMS the read-out kernels walk
+# a molecule in 64-atom chunks and the co-attention runs csrc/coattn_big.cu (fp32 in either mode, energy in a per-CTA workspace
+# slice), both up to 256 atoms.  The compositions below (torch.matmul -> cuBLAS, with autograd) remain only for the widths the
+# kernels do not hold: co-attention atoms wider than 192 (first_last_atoms) and the read-out backward at hidden = out_dim = 256.
 MAX_KERNEL_ATOMS = 64
 _TORCH_ACT = {0: (lambda x: x), 1: torch.tanh, 2: torch.relu, 3: torch.sigmoid}
 
@@ -459,11 +458,12 @@ def _readout_large(h, h0, mask, variant, act, act_agg, W_i, b_i, W_j, b_j):
 
 
 def readout(h, h0, mask, variant, act, act_agg, W_i, b_i, W_j, b_j, mode=0):
-    """GGNNReadout variants R1 / R2 / SUM: the CUDA kernels, or the library composition above 64 atoms."""
+    """GGNNReadout variants R1 / R2 / SUM: the CUDA kernels (up to 256 atoms), or the library composition for a training step at
+    hidden = out_dim = 256."""
     kcat = h.shape[2] * (2 if h0 is not None else 1)
     # the fp32 backward kernel keeps [h | h0] and both gate tiles in shared memory: (Kcat + 2 O) * 64 floats + staging <= 227 KB
     too_wide = variant != K.READOUT_SUM and torch.is_grad_enabled() and kcat + 2 * W_i.shape[0] > 836
-    if h.shape[1] > MAX_KERNEL_ATOMS or too_wide:
+    if too_wide:
         return _readout_large(_f32(h), _f32(h0), _f32(mask), variant, act, act_agg, W_i, b_i, W_j, b_j)
     return Readout.apply(h, h0, mask, variant, act, act_agg, W_i, b_i, W_j, b_j, mode)
 
@@ -491,10 +491,11 @@ def _coattention_large(a1, a2, variant, act, W, V1, V2, b, lt_1, lt_2, wa_1, wa_
 
 
 def coattention(atoms_1, atoms_2, variant, act, W, V1, V2, b, lt_1, lt_2, wa_1, wa_2, W_j, b_j, mode=0):
-    """Fine-grained co-attention (Nie / VQA / Pooling): the CUDA kernels, or the library composition above 64 atoms."""
+    """Fine-grained co-attention (Nie / VQA / Pooling): the CUDA kernels (up to 256 atoms), or the library composition for atoms
+    wider than 192."""
     # hidden > 192 (e.g. the [h_first | h_last] atoms of train_ddi_modify_eval3.py:110-134 at GGNN hidden 128): the three 64 x H fp32
     # panels of the CUDA kernel no longer fit shared memory
-    if max(atoms_1.shape[1], atoms_2.shape[1]) > MAX_KERNEL_ATOMS or atoms_1.shape[2] > 192:
+    if atoms_1.shape[2] > 192:
         return _coattention_large(_f32(atoms_1), _f32(atoms_2), variant, act, W, V1, V2, b, lt_1, lt_2, wa_1, wa_2, W_j, b_j)
     return Coattention.apply(atoms_1, atoms_2, variant, act, W, V1, V2, b, lt_1, lt_2, wa_1, wa_2, W_j, b_j, mode)
 
@@ -546,7 +547,15 @@ class Readout(torch.autograd.Function):
 
 
 def _coattn_workspace(a, mode, H, dev, params):
-    """Packed bf16 weight images of the tcgen05 co-attention (None when that path does not apply)."""
+    """Packed bf16 weight images of the tcgen05 co-attention, or above 64 atoms (either mode) the scratch of the fp32 kernel for
+    that size; None when neither applies."""
+    if max(a.n1, a.n2) > MAX_KERNEL_ATOMS:
+        n = int(K.lib.bmp_coattn_large_workspace_bytes(a.n1, a.n2, H, a.head))
+        if not n:
+            return None         # not covered: the call reports the shape
+        ws = torch.empty((n,), device=dev, dtype=torch.uint8)
+        a.tc_workspace, a.tc_workspace_bytes = _p(ws), n
+        return ws
     if mode != K.MODE_BF16:
         return None
     n = int(K.lib.bmp_coattn_tc_workspace_bytes(H))

@@ -277,7 +277,8 @@ typedef struct {
     const float *W, *V1, *V2, *b, *lt_1, *lt_2, *wa_1, *wa_2, *W_j, *b_j;
     float *compact_1, *compact_2;      /* (mb,O) */
     int    mode;                       /* BMP_MODE_BF16: contractions on tcgen05 (FINE variant, hidden 64/128, head <= 15) */
-    void  *tc_workspace;               /* BMP_MODE_BF16: >= bmp_coattn_tc_workspace_bytes(hidden) bytes, 16-byte aligned */
+    void  *tc_workspace;               /* BMP_MODE_BF16: >= bmp_coattn_tc_workspace_bytes(hidden) bytes, 16-byte aligned;
+                                          n1 or n2 > 64 (either mode): >= bmp_coattn_large_workspace_bytes(n1, n2, hidden, head) */
     size_t tc_workspace_bytes;
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
@@ -307,6 +308,11 @@ typedef struct {
 int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream);
 /* packed bf16 weight images of the tcgen05 co-attention kernels; 0 when hidden is not 64 or 128 */
 size_t bmp_coattn_tc_workspace_bytes(int hidden);
+/* Pairs where a molecule has 65..BMP_X3_MAX_ATOMS atoms (csrc/coattn_big.cu): bmp_coattn_forward / bmp_coattn_backward run an fp32
+ * kernel in either mode that keeps the N1 x N2 energy in per-CTA slices of tc_workspace, which must hold at least this many bytes.
+ * Covers FINE and POOL, every activation, head <= 16, hidden a multiple of 4 <= 192.  0 when both molecules have <= 64 atoms or the
+ * shape is not covered (the call then fails with BMP_ESHAPE).  Host-only.                                                          */
+size_t bmp_coattn_large_workspace_bytes(int n1, int n2, int hidden, int head);
 
 /* ---- HolE circular correlation ----------------------------------------------
  * replaces models/link_prediction/hole.py:28-50 (= models/mlp.py:128-151):
