@@ -552,6 +552,24 @@ static int check_common(int mb, int N, int H, int E, int T, int mode, int nmax =
     return BMP_OK;
 }
 
+// BMP_MODE_F32: a drug table (mol_index) and byte / bit-packed storage (adj_u8 = 1 / 2) are read by the tensor-core row path's
+// adjacency kernels only; the FFMA kernels take the gathered fp32 (mb,E,N,N) array
+static int check_table_args(const char *fn, const int32_t *mol_index, int adj_u8, bool x3) {
+    if (adj_u8 < 0 || adj_u8 > 2) { set_error("%s: adj_u8=%d is not a storage code (0 fp32, 1 bytes, 2 bit-packed rows)", fn, adj_u8); return BMP_EINVAL; }
+    if (x3) return BMP_OK;
+    if (mol_index) {
+        set_error("%s: mol_index in BMP_MODE_F32 needs the tensor-core row path: tc_workspace of bmp_ggnn_x3_workspace_bytes() bytes "
+                  "and no state_in (else gather the rows first)", fn);
+        return BMP_ESHAPE;
+    }
+    if (adj_u8) {
+        set_error("%s: adj_u8=%d in BMP_MODE_F32 needs the tensor-core row path: tc_workspace of bmp_ggnn_x3_workspace_bytes() bytes "
+                  "and no state_in (else pass fp32)", fn, adj_u8);
+        return BMP_EINVAL;
+    }
+    return BMP_OK;
+}
+
 }  // namespace bmp
 
 using namespace bmp;
@@ -563,21 +581,29 @@ bool bmp_ggnn_x3_usable(int mb, int N, int H, int E, int T, const void *ws, size
 int bmp_ggnn_forward_x3(const bmp_ggnn_fwd_t *a, void *stream);
 int bmp_ggnn_backward_x3(const bmp_ggnn_bwd_t *a, void *stream);
 
+// The one place that decides whether a BMP_MODE_F32 forward runs on the tensor-core row path (callers size the workspace with it and
+// know up front whether a drug table / byte storage is read in place): shape, no external state, 16-byte aligned bias vectors.
+extern "C" size_t bmp_ggnn_x3_forward_bytes(const bmp_ggnn_fwd_t *a, int inference) {
+    if (!a || a->state_in || a->n_steps <= 0 || a->n_steps > BMP_MAX_STEPS) return 0;
+    for (int t = 0; t < a->n_steps; ++t) {
+        const bmp_gru_t &g = a->gru[t];
+        if (!aligned16({a->msg_b[t], g.b_Wr, g.b_Ur, g.b_Wz, g.b_Uz, g.b_W, g.b_U})) return 0;
+    }
+    return bmp_ggnn_x3_workspace_bytes(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, inference);
+}
+
 extern "C" int bmp_ggnn_forward(const bmp_ggnn_fwd_t *a, void *stream) {
     if (!a || !a->adj || (!a->atoms && !a->h_in) || (a->atoms && !a->embed_W)) {
         set_error("bmp_ggnn_forward: null argument");
         return BMP_EINVAL;
     }
     if (a->mode == BMP_MODE_BF16) return bmp_ggnn_forward_tc(a, stream);
-    if (a->mol_index) { set_error("bmp_ggnn_forward: mol_index (table indirection) is a BMP_MODE_BF16 feature; gather the rows first"); return BMP_ESHAPE; }
-    if (a->adj_u8) { set_error("bmp_ggnn_forward: a byte adjacency needs BMP_MODE_BF16"); return BMP_EINVAL; }
-    bool x3 = a->n_steps > 0 && a->n_steps <= BMP_MAX_STEPS &&
-              bmp_ggnn_x3_usable(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, a->tc_workspace, a->tc_workspace_bytes, a->state_in, a->Hs == nullptr);
-    for (int t = 0; x3 && t < a->n_steps; ++t) {
-        const bmp_gru_t &g = a->gru[t];
-        x3 = aligned16({a->msg_b[t], g.b_Wr, g.b_Ur, g.b_Wz, g.b_Uz, g.b_W, g.b_U});
-    }
-    int rc = check_common(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, a->mode, x3 ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
+    const size_t x3_need = bmp_ggnn_x3_forward_bytes(a, a->Hs == nullptr);
+    const bool x3 = x3_need && a->tc_workspace && a->tc_workspace_bytes >= x3_need;
+    int rc = check_table_args("bmp_ggnn_forward", a->mol_index, a->adj_u8, x3);
+    if (rc) return rc;
+    if (a->mol_index && !a->atoms) { set_error("bmp_ggnn_forward: mol_index needs atom ids (a drug table), not h_in"); return BMP_EINVAL; }
+    rc = check_common(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, a->mode, x3 ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
     if (rc) return rc;
     for (int t = 0; t < a->n_steps; ++t) {
         const bmp_gru_t &g = a->gru[t];
@@ -639,7 +665,9 @@ extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
     }
     const bool x3_data = a->mode == BMP_MODE_F32 && a->n_steps > 0 && a->n_steps <= BMP_MAX_STEPS &&
                          bmp_ggnn_x3_usable(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, a->tc_workspace, a->tc_workspace_bytes, a->state_in, false);
-    int rc = check_common(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, BMP_MODE_F32, x3_data ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
+    int rc = check_table_args("bmp_ggnn_backward", a->mol_index, a->adj_u8, x3_data);
+    if (rc) return rc;
+    rc = check_common(a->mb, a->n_atoms, a->hidden, a->n_edge, a->n_steps, BMP_MODE_F32, x3_data ? BMP_X3_MAX_ATOMS : BMP_MAX_ATOMS);
     if (rc) return rc;
     const int H = a->hidden, T = a->n_steps, E = a->n_edge;
     const bool tc3 = a->mode == BMP_MODE_F32 && (H == 64 || H == 128 || H == 256);
@@ -650,7 +678,6 @@ extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
         if (!e_ && db) e_ = bmp_colsum(A_, lda, db, dbs, r_, H, stream);
         return e_;
     };
-    if (a->adj_u8) { set_error("bmp_ggnn_backward: a byte adjacency needs BMP_MODE_BF16"); return BMP_EINVAL; }
     if (H > 128 && a->state_in) {
         set_error("bmp_ggnn_backward: an external GRU state needs hidden <= 128 (hidden=%d)", H);
         return BMP_ESHAPE;

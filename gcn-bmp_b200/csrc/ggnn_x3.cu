@@ -469,27 +469,41 @@ __global__ void __launch_bounds__(256) pack_x3_kernel(const PackArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------------ adjacency products
-// The adjacency is the reference's dense fp32 (mb,E,N,N) array, > 97 % zeros.  It is scanned ONCE per encoder call into bit masks
-// (64 bits per row and per column of every bond type, 4 KB per molecule instead of 64 KB) plus a flag "some non-zero entry is not
-// 1.0"; the per-step products then walk the set bits in ascending order -- the dense sum with the zeros skipped -- and touch the
-// dense array again only when that flag is set (general fp32 weights).
-// masks[mol][0][e][i][w] bit b = (A_e[i][64 w + b] != 0) ; masks[mol][1][e][j][w] bit b = (A_e[64 w + b][j] != 0) ; W = ceil(N / 64) words
-__global__ void __launch_bounds__(256) adj_mask_kernel(const float *__restrict__ adj, unsigned long long *__restrict__ masks, int *nonbinary,
-                                                       int mb, int N) {
+// The adjacency (> 97 % zeros) is scanned ONCE per encoder call into bit masks (64 bits per row and per column of every bond type,
+// 4 KB per molecule at N = 64 instead of 64 KB of fp32) plus a flag "some non-zero entry is not 1.0"; the per-step products then walk
+// the set bits in ascending order -- the dense sum with the zeros skipped -- and touch the adjacency again only when that flag is set
+// (general weights).  Storage `fmt` (bmp_ggnn_fwd_t.adj_u8): 0 = fp32 (U,E,N,N) as the reference, 1 = the same as bytes, 2 = bit-packed
+// rows (U,E,N,ceil(N/8)), bit j&7 of byte j>>3 (never sets the flag).  Molecule b is row mol_index[b] of that array (NULL: row b), so
+// a drug table is read in place: no gathered or widened copy.  The masks stay indexed by b.
+// masks[b][0][e][i][w] bit k = (A_e[i][64 w + k] != 0) ; masks[b][1][e][j][w] bit k = (A_e[64 w + k][j] != 0) ; W = ceil(N / 64) words
+__device__ __forceinline__ const void *adj_mol(const void *adj, const int32_t *mol_index, int mol, int fmt, int N) {
+    const long row = mol_index ? (long)__ldg(mol_index + mol) : (long)mol;
+    const long per = 4L * N * (fmt == 2 ? (N + 7) / 8 : N);         // entries (bytes for fmt 1 / 2) of one molecule
+    return fmt == 0 ? (const void *)((const float *)adj + row * per) : (const void *)((const uint8_t *)adj + row * per);
+}
+// entry (i, j) of bond type e of one molecule's adjacency, as a weight
+__device__ __forceinline__ float adj_at(const void *am, int fmt, int N, int e, int i, int j) {
+    if (fmt == 0) return __ldg((const float *)am + ((long)e * N + i) * N + j);
+    if (fmt == 1) return (float)__ldg((const uint8_t *)am + ((long)e * N + i) * N + j);
+    return (float)((__ldg((const uint8_t *)am + ((long)e * N + i) * ((N + 7) >> 3) + (j >> 3)) >> (j & 7)) & 1);
+}
+
+__global__ void __launch_bounds__(256) adj_mask_kernel(const void *__restrict__ adj, const int32_t *__restrict__ mol_index, int fmt,
+                                                       unsigned long long *__restrict__ masks, int *nonbinary, int mb, int N) {
     extern __shared__ unsigned long long cm[];                   // [4][N][W] column masks
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, W = (N + 63) >> 6, per = 4 * N * W;
     for (int mol = blockIdx.x; mol < mb; mol += gridDim.x) {
         __syncthreads();
         for (int idx = tid; idx < per; idx += 256) cm[idx] = 0ull;
         unsigned long long *out = masks + (size_t)mol * 2 * per;
+        const void *am = adj_mol(adj, mol_index, mol, fmt, N);
         __syncthreads();
         bool odd = false;
         for (int idx = warp; idx < 4 * N; idx += 8) {
             const int e = idx / N, i = idx - e * N;
-            const float *arow = adj + (((long)mol * 4 + e) * N + i) * N;
             for (int w = 0; w < W; ++w) {
                 const int j0 = 64 * w + lane, j1 = j0 + 32;
-                const float a0 = j0 < N ? __ldg(arow + j0) : 0.f, a1 = j1 < N ? __ldg(arow + j1) : 0.f;
+                const float a0 = j0 < N ? adj_at(am, fmt, N, e, i, j0) : 0.f, a1 = j1 < N ? adj_at(am, fmt, N, e, i, j1) : 0.f;
                 const unsigned long long m = (unsigned long long)__ballot_sync(0xffffffffu, a0 != 0.f) |
                                              ((unsigned long long)__ballot_sync(0xffffffffu, a1 != 0.f) << 32);
                 if (lane == 0) out[(e * N + i) * W + w] = m;
@@ -508,10 +522,12 @@ __global__ void __launch_bounds__(256) adj_mask_kernel(const float *__restrict__
 //              operand of the bias k-tile)
 // BWD = true : dst[row j][e*H + c] = sum_i A_e[i][j] src[i][c]  (A_e^T dm)                                    one CTA per molecule
 // cscale (mb, N) or NULL: every A_e[i][j] is taken times cscale[mol][j] (RelGCN's rescale_adj), deg included
+// adj / mol_index / fmt as for adj_mask_kernel: read only when the flag says some weight is not 0/1 (fmt 0 or 1)
 template <bool BWD>
 __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__restrict__ masks, const int *__restrict__ nonbinary,
-                                                  const float *__restrict__ adj, const float *__restrict__ src, float *__restrict__ dst,
-                                                  float *__restrict__ deg, int mb, int N, int H, const float *__restrict__ cscale) {
+                                                  const void *__restrict__ adj, const int32_t *__restrict__ mol_index, int fmt,
+                                                  const float *__restrict__ src, float *__restrict__ dst, float *__restrict__ deg, int mb,
+                                                  int N, int H, const float *__restrict__ cscale) {
     extern __shared__ __align__(16) float sh[];                  // [N][H]
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, HV = H / 4, W = (N + 63) >> 6, per = 4 * N * W;
     const bool general = *nonbinary != 0;
@@ -521,7 +537,7 @@ __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__re
         for (int idx = tid; idx < N * HV; idx += 256) reinterpret_cast<float4 *>(sh)[idx] = __ldg(s4 + idx);
         __syncthreads();
         const unsigned long long *mk = masks + (size_t)mol * 2 * per + (BWD ? per : 0);
-        const float *am = adj + (long)mol * 4 * N * N;
+        const void *am = general ? adj_mol(adj, mol_index, mol, fmt, N) : nullptr;
         const float *cs = cscale ? cscale + (long)mol * N : nullptr;
         for (int idx = warp; idx < 4 * N; idx += 8) {
             const int e = idx / N, x = idx - e * N;
@@ -532,7 +548,7 @@ __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__re
                 while (m) {
                     const int y = 64 * w + __ffsll((long long)m) - 1;
                     m &= m - 1;
-                    float v = general ? __ldg(am + ((long)e * N + (BWD ? y : x)) * N + (BWD ? x : y)) : 1.f;
+                    float v = general ? adj_at(am, fmt, N, e, BWD ? y : x, BWD ? x : y) : 1.f;
                     if (cs) v *= cs[BWD ? x : y];
                     d += v;
                     const float4 *hr = reinterpret_cast<const float4 *>(sh + y * H);
@@ -551,6 +567,15 @@ __global__ void __launch_bounds__(256) agg_kernel(const unsigned long long *__re
             if (lane + 32 < HV) out[lane + 32] = acc1;
             if (!BWD && deg && lane == 0) deg[((long)mol * N + x) * 64 + e] = d;
         }
+    }
+}
+
+// dst[b][n] = table[mol_index[b]][n] for the (mb, N) atom ids of a drug table
+__global__ void __launch_bounds__(256) gather_rows_kernel(const int32_t *__restrict__ table, const int32_t *__restrict__ mol_index,
+                                                          int32_t *__restrict__ dst, int mb, int N) {
+    for (long idx = (long)blockIdx.x * 256 + threadIdx.x; idx < (long)mb * N; idx += (long)gridDim.x * 256) {
+        const long b = idx / N;
+        dst[idx] = __ldg(table + (long)__ldg(mol_index + b) * N + (idx - b * N));
     }
 }
 
@@ -590,6 +615,11 @@ static int sm_count() {
         if (sms <= 0) sms = 148;
     }
     return sms;
+}
+
+static int pointwise_grid(long n) {
+    const long g = (n + 255) / 256;
+    return (int)(g < 16L * sm_count() ? g : 16L * sm_count());
 }
 
 // the row GEMMs never see molecule boundaries; the per-molecule adjacency products keep an N x H fp32 tile in shared memory
@@ -854,7 +884,15 @@ int bmp_ggnn_forward_x3(const bmp_ggnn_fwd_t *a, void *stream) {
     auto RS_at = [&](int t) { return inference ? mini + 6 * RH : a->RSs + (size_t)t * RH; };
 
     if (a->atoms) {
-        if ((rc = bmp_embed_forward(a->atoms, a->embed_W, Hs_at(0), (int)rows, H, a->n_atom_types, stream))) return rc;
+        const int32_t *ids = a->atoms;
+        if (a->mol_index) {            // table rows: gather the (mb, N) ids into the deg slice, which is zeroed right after
+            int32_t *g = reinterpret_cast<int32_t *>(ws + L.deg_off);
+            gather_rows_kernel<<<pointwise_grid(rows), 256, 0, st>>>(a->atoms, a->mol_index, g, a->mb, N);
+            count_launch();
+            if ((rc = check_launch("gather_rows_kernel"))) return rc;
+            ids = g;
+        }
+        if ((rc = bmp_embed_forward(ids, a->embed_W, Hs_at(0), (int)rows, H, a->n_atom_types, stream))) return rc;
     } else {
         cudaMemcpyAsync(Hs_at(0), a->h_in, RH * sizeof(float), cudaMemcpyDeviceToDevice, st);
     }
@@ -867,7 +905,7 @@ int bmp_ggnn_forward_x3(const bmp_ggnn_fwd_t *a, void *stream) {
     cudaFuncSetAttribute(agg_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)agg_smem);
     const int agg_grid = a->mb < 8 * sm_count() ? a->mb : 8 * sm_count();
     cudaMemsetAsync(flag, 0, 256, st);
-    adj_mask_kernel<<<agg_grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(a->adj, masks, flag, a->mb, N);
+    adj_mask_kernel<<<agg_grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(a->adj, a->mol_index, a->adj_u8, masks, flag, a->mb, N);
     count_launch();
     if ((rc = check_launch("adj_mask_kernel"))) return rc;
     for (int t = 0; t < T; ++t) {
@@ -875,7 +913,8 @@ int bmp_ggnn_forward_x3(const bmp_ggnn_fwd_t *a, void *stream) {
         const uint8_t *img = ws + (size_t)img_of[t] * L.img_bytes;
         const bmp_gru_t &G = a->gru[t];
         float *h = Hs_at(t), *hn = Hs_at(t + 1), *m = Ms_at(t), *g = Gs_at(t), *rs = RS_at(t);
-        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, h, AH, t == 0 ? deg : nullptr, a->mb, N, H, nullptr);
+        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, a->mol_index, a->adj_u8, h, AH, t == 0 ? deg : nullptr, a->mb,
+                                                            N, H, nullptr);
         count_launch();
         if ((rc = check_launch("agg_kernel"))) return rc;
         Args ga;
@@ -960,7 +999,7 @@ int bmp_ggnn_backward_x3(const bmp_ggnn_bwd_t *a, void *stream) {
     cudaFuncSetAttribute(agg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)agg_smem);
     const int agg_grid = a->mb < 8 * sm_count() ? a->mb : 8 * sm_count();
     cudaMemsetAsync(flag, 0, 256, st);        // the masks are rebuilt: the workspace need not be the forward's
-    adj_mask_kernel<<<agg_grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(a->adj, masks, flag, a->mb, N);
+    adj_mask_kernel<<<agg_grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(a->adj, a->mol_index, a->adj_u8, masks, flag, a->mb, N);
     count_launch();
     if ((rc = check_launch("adj_mask_kernel"))) return rc;
     for (int t = T - 1; t >= 0; --t) {
@@ -1010,7 +1049,8 @@ int bmp_ggnn_backward_x3(const bmp_ggnn_bwd_t *a, void *stream) {
             }
         ga.njobs = nj;
         if ((rc = launch_gemm(ga, st))) return rc;
-        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, dm, a->Ps + (size_t)t * 4 * RH, nullptr, a->mb, N, H, nullptr);
+        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, a->mol_index, a->adj_u8, dm, a->Ps + (size_t)t * 4 * RH, nullptr,
+                                                          a->mb, N, H, nullptr);
         count_launch();
         if ((rc = check_launch("agg_kernel"))) return rc;
         // ---- dHs[t] += dh_x + sum_e P_e W_e
@@ -1189,7 +1229,7 @@ static int relgcn_adjacency(const float *adj, int mb, int N, bool scale, uint8_t
     int *flag = reinterpret_cast<int *>(ws + R.mask_off);
     const int grid = mb < 8 * sm_count() ? mb : 8 * sm_count();
     cudaMemsetAsync(flag, 0, 256, st);
-    adj_mask_kernel<<<grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(adj, reinterpret_cast<unsigned long long *>(ws + R.mask_off + 256),
+    adj_mask_kernel<<<grid, 256, (size_t)32 * N * ((N + 63) / 64), st>>>(adj, nullptr, 0, reinterpret_cast<unsigned long long *>(ws + R.mask_off + 256),
                                                                          flag, mb, N);
     count_launch();
     int rc;
@@ -1215,11 +1255,6 @@ static int relgcn_pack(const float *const *Ws, const float *const *bs, const flo
         count_launch();
     }
     return check_launch("pack_relgcn_kernel");
-}
-
-static int pointwise_grid(long n) {
-    const long g = (n + 255) / 256;
-    return (int)(g < 16L * sm_count() ? g : 16L * sm_count());
 }
 
 }  // namespace x3
@@ -1285,7 +1320,7 @@ int bmp_relgcn_forward_x3(const bmp_relgcn_fwd_t *a, void *stream) {
     size_t hs_off = (size_t)rows * a->ch[0];
     for (int l = 0; l < L; ++l) {
         float *h = X[l & 1], *hn = X[(l + 1) & 1];
-        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, h, AH, l == 0 ? deg : nullptr, a->mb, N, Cp, cs);
+        agg_kernel<false><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, nullptr, 0, h, AH, l == 0 ? deg : nullptr, a->mb, N, Cp, cs);
         count_launch();
         if ((rc = check_launch("agg_kernel"))) return rc;
         const uint8_t *img = ws + (size_t)l * R.layer_img;
@@ -1352,7 +1387,7 @@ int bmp_relgcn_backward_x3(const bmp_relgcn_bwd_t *a, void *stream) {
                                                                              Cp, a->act);
         count_launch();
         if ((rc = check_launch("relgcn_delta_kernel"))) return rc;
-        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, D, P, nullptr, a->mb, N, Cp, cs);
+        agg_kernel<true><<<agg_grid, 256, agg_smem, st>>>(masks, flag, a->adj, nullptr, 0, D, P, nullptr, a->mb, N, Cp, cs);
         count_launch();
         if ((rc = check_launch("agg_kernel"))) return rc;
         const float *Hl = a->Hs + hs_off[l];

@@ -120,7 +120,11 @@ extern "C" int bmp_pair_forward_backward(const bmp_pair_t *a, void *stream) {
     const int N[2] = {a->n1, a->n2};
     const int32_t *atoms[2] = {a->atoms_1, a->atoms_2};
     const void *adj[2] = {a->adj_1, a->adj_2};
-    if (a->adj_u8 && !bf16) { set_error("bmp_pair_forward_backward: a byte / bit-packed adjacency needs BMP_MODE_BF16"); return BMP_EINVAL; }
+    if (a->adj_u8 && !bf16 && !pl.x3_ws) {
+        set_error("bmp_pair_forward_backward: adj_u8=%d in BMP_MODE_F32 needs both encoders on the tensor-core row path (hidden "
+                  "64/128/256, mb * n_atoms >= 128 on each side)", a->adj_u8);
+        return BMP_EINVAL;
+    }
     const float *hT[2];
     float *d_hT[2];
     int rc;

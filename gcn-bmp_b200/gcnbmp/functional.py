@@ -51,13 +51,15 @@ def unpack_adjacency(bits, n_atoms=None):
     return x[..., :n].to(torch.float32).contiguous()
 
 
-def _adj(t, mode):
-    """Adjacency as the kernels take it: fp32, or -- BF16 mode only -- the caller's uint8 / bool / bit-packed array as is
-    (exact for 0/1 bonds; 1/4 resp. 1/32 of the PCIe and HBM traffic).  Returns (tensor, storage code)."""
+def _adj(t, mode, keep=False):
+    """Adjacency as the kernels take it: fp32, or -- BF16 mode, or `keep` (the fp32 tensor-core row path) -- the caller's
+    uint8 / bool / bit-packed array as is (exact for 0/1 bonds; 1/4 resp. 1/32 of the PCIe and HBM traffic).  Returns
+    (tensor, storage code)."""
     fmt = adj_format(t)
-    if fmt == 2 and mode != K.MODE_BF16:
+    keep = keep or mode == K.MODE_BF16
+    if fmt == 2 and not keep:
         return unpack_adjacency(t), 0
-    if mode == K.MODE_BF16 and fmt:
+    if keep and fmt:
         t = t.contiguous()
         return (t.view(torch.uint8) if t.dtype == torch.bool else t), fmt
     return _f32(t), 0
@@ -134,6 +136,13 @@ def _tc_images(kind, nbytes, dev, params):
 F32_TENSOR_CORES = True     # MODE_F32: run the encoder's contractions on tcgen05 with a bf16 hi/lo split (fp32-grade); False = FFMA kernels
 
 
+def x3_row_path(a, inference):
+    """MODE_F32: does the encoder call `a` (a GgnnFwd with its shape, state and parameter pointers filled in) take the tensor-core
+    row path?  The library decides (bmp_ggnn_x3_forward_bytes, the test bmp_ggnn_forward applies).  Only that path reads a drug
+    table through `mol_index` and byte / bit-packed adjacency in place; the FFMA kernels get gathered fp32 rows."""
+    return F32_TENSOR_CORES and int(K.lib.bmp_ggnn_x3_forward_bytes(C.byref(a), int(inference))) > 0
+
+
 def _x3_workspace(a, mb, N, H, E, T, dev, params, inference):
     """MODE_F32 on the tensor cores: hand the call a workspace (weight images + temporaries) when the shape is covered."""
     if not F32_TENSOR_CORES:
@@ -186,35 +195,39 @@ class GGNNEncode(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, adj, state_in, plan, n_msg, n_gru, mode, want_stash, keep_steps, mol_index, *params):
         _need_cuda(x, adj)
-        if mol_index is not None and (mode != K.MODE_BF16 or x.dtype not in (torch.int32, torch.int64)):
-            # table indirection is read inside the tcgen05 kernels only; elsewhere gather the rows (a device-side copy)
-            x, adj, mol_index = x.index_select(0, mol_index.long()), adj.index_select(0, mol_index.long()), None
-        adj, adj_u8 = _adj(adj, mode)
-        mb, E, N, _ = adj.shape
-        if mol_index is not None:
-            mol_index = mol_index.to(torch.int32).contiguous()
-            mb = mol_index.shape[0]
+        is_ids = x.dtype in (torch.int32, torch.int64)
         embed_W = params[0]
         msg = [(params[1 + 2 * i], params[2 + 2 * i]) for i in range(n_msg)]
         base = 1 + 2 * n_msg
         gru = [params[base + 12 * i: base + 12 * (i + 1)] for i in range(n_gru)]
         H = msg[0][0].shape[1]
         T = len(plan)
+        _, E, N = adj.shape[:3]
+        mb = adj.shape[0] if mol_index is None else mol_index.shape[0]
+        state_in = _f32(state_in)
         a = K.GgnnFwd()
         a.mb, a.n_atoms, a.hidden, a.n_edge, a.n_steps, a.mode = mb, N, H, E, T, mode
-        is_ids = x.dtype in (torch.int32, torch.int64)
+        a.state_in = _p(state_in)
+        for t, (mi, gi, st) in enumerate(plan):
+            a.msg_W[t], a.msg_b[t] = _p(msg[mi][0]), _p(msg[mi][1])
+            _fill_gru(a.gru[t], gru[gi])
+            a.stateful[t] = int(st)
+        # MODE_F32: the row path reads a table row and the table's own storage in its adjacency kernels; the FFMA kernels
+        # need gathered, widened rows
+        row = mode == K.MODE_F32 and x3_row_path(a, not want_stash)
+        if mol_index is not None and not (is_ids and (mode == K.MODE_BF16 or row)):
+            # table indirection is read inside the kernels on those paths only; elsewhere gather the rows (a device-side copy)
+            x, adj, mol_index = x.index_select(0, mol_index.long()), adj.index_select(0, mol_index.long()), None
+        adj, adj_u8 = _adj(adj, mode, keep=row)
+        if mol_index is not None:
+            mol_index = mol_index.to(torch.int32).contiguous()
         if is_ids:
             x = x.to(torch.int32).contiguous()
             a.atoms, a.embed_W, a.n_atom_types = _p(x), _p(embed_W), embed_W.shape[0]
         else:
             x = _f32(x)
             a.h_in = _p(x)
-        state_in = _f32(state_in)
-        a.adj, a.state_in, a.adj_u8, a.mol_index = _p(adj), _p(state_in), adj_u8, _p(mol_index)
-        for t, (mi, gi, st) in enumerate(plan):
-            a.msg_W[t], a.msg_b[t] = _p(msg[mi][0]), _p(msg[mi][1])
-            _fill_gru(a.gru[t], gru[gi])
-            a.stateful[t] = int(st)
+        a.adj, a.adj_u8, a.mol_index = _p(adj), adj_u8, _p(mol_index)
         dev = adj.device
         rows = mb * N
         if mode == K.MODE_BF16:
@@ -242,7 +255,7 @@ class GGNNEncode(torch.autograd.Function):
             ctx.meta = (plan, n_msg, n_gru, mode, is_ids, keep_steps)
             return out
         x3ws = None
-        if mode == K.MODE_F32 and state_in is None and mol_index is None and not adj_u8:
+        if row:
             x3ws = _x3_workspace(a, mb, N, H, E, T, dev, params, not want_stash)
         if want_stash:
             Hs = torch.empty((T + 1, mb, N, H), device=dev, dtype=torch.float32)

@@ -64,14 +64,15 @@ def _as_device(x, dtype=None):
     return x
 
 
-def _adj_device(adj, mode):
+def _adj_device(adj, mode, table=False):
     """Adjacency to the device: fp32 as in the reference; a uint8 / bool / bit-packed (functional.pack_adjacency) adjacency is
     kept as is in BF16 mode (the tcgen05 kernels stage it directly -- exact for 0/1 bonds, 1/4 resp. 1/32 of the bytes) and
-    widened to fp32 otherwise."""
+    for a drug table read through `mol_index` (the encoder gathers and widens only the rows it needs when its kernels cannot
+    read the table in place), and widened to fp32 otherwise."""
     dt = adj.dtype if isinstance(adj, torch.Tensor) else torch.from_numpy(np.empty(0, np.asarray(adj).dtype)).dtype
     if dt in (torch.uint8, torch.bool):
         t = _as_device(adj)
-        if mode == K.MODE_BF16:
+        if mode == K.MODE_BF16 or table:
             return t
         return Fn.unpack_adjacency(t) if Fn.adj_format(t) == 2 else t.to(torch.float32)
     return _as_device(adj, torch.float32)
@@ -318,11 +319,12 @@ def _encode(x, adj, state, plan, msgs, grus, embed_W, mode, keep_steps=False, mo
     `keep_steps` (or in fp32 mode with a tape) -- BF16 mode trains on a bf16 panel stash it keeps internally."""
     want = torch.is_grad_enabled()
     H = msgs[0][0].shape[1]
-    if mode == K.MODE_BF16 and adj.shape[-1] > Fn.MAX_KERNEL_ATOMS and mol_index is None:
+    if mode == K.MODE_BF16 and adj.shape[-2] > Fn.MAX_KERNEL_ATOMS:
         # molecules with more than 64 atoms: the fused tcgen05 encoders hold a two-molecule tile of 64-atom molecules; such batches take
-        # the fp32 tensor-core path (row GEMMs, any N up to 256) -- more accurate, slower, same interface
+        # the fp32 tensor-core path (row GEMMs, any N up to 256) -- more accurate, slower, same interface.  A drug table keeps its
+        # index and storage: that path reads the rows in place (GGNNEncode gathers them when it cannot)
         mode = K.MODE_F32
-        if adj.dtype != torch.float32:
+        if adj.dtype != torch.float32 and mol_index is None:
             adj = Fn.unpack_adjacency(adj) if Fn.adj_format(adj) == 2 else adj.to(torch.float32)
     if mode == K.MODE_BF16 and H not in (64, 128, 256) and H < 128 and state is None and msgs[0][0].shape[0] == 4 * H:
         # The tcgen05 encoders exist for hidden 64 / 128 (256 forward only); any other hidden size <= 128 (the paper's 32, the
@@ -456,7 +458,7 @@ class GGNN(Link):
     def __call__(self, atom_array, adj, is_real_node=None, mol_index=None):
         """`mol_index` (extension): rows of a device-resident drug table, as in GGNNMono.__call__."""
         self.reset_state()
-        adj = _adj_device(adj, self.__dict__.get("mode", K.MODE_F32))
+        adj = _adj_device(adj, self.__dict__.get("mode", K.MODE_F32), table=mol_index is not None)
         if mol_index is not None:
             mol_index = _as_device(mol_index, torch.int32)
         ids = _is_ids(atom_array) and getattr(atom_array, "ndim", 2) <= 2
@@ -520,9 +522,10 @@ class GGNNMono(Link):
 
     def __call__(self, atom_array, adj, mol_index=None):
         """`mol_index` (extension, SURVEY 8 f-1): int (mb,) -- `atom_array` (U,N) / `adj` (U,E,N,N) are a device-resident drug
-        table and molecule b of the batch is its row mol_index[b] (read inside the tcgen05 kernels, no gather copy)."""
+        table and molecule b of the batch is its row mol_index[b], read inside the kernels with no gather copy (BF16 mode, and
+        fp32 mode on the tensor-core row path: mb * N >= 128, hidden 64/128/256; elsewhere the rows are gathered)."""
         self.update_layer.reset_state()
-        adj = _adj_device(adj, self.__dict__.get("mode", K.MODE_F32))
+        adj = _adj_device(adj, self.__dict__.get("mode", K.MODE_F32), table=mol_index is not None)
         if mol_index is not None:
             mol_index = _as_device(mol_index, torch.int32)
         ids = _is_ids(atom_array)
@@ -1231,10 +1234,11 @@ class GraphConvPredictorForPair(Link):
         return self.head(g1, g2)
 
     def encode_rows(self, table_atoms, table_adjs, rows):
-        """Encoder over rows of a device-resident drug table -> (graph vectors, atom states).  GGNN encoders in BF16 mode read
-        the table through the index inside the kernels; every other encoder gets a gathered copy of the rows."""
+        """Encoder over rows of a device-resident drug table -> (graph vectors, atom states).  GGNN encoders take the index
+        (read inside the kernels in BF16 mode and on the fp32 tensor-core row path; gathered by the encoder elsewhere); every other
+        encoder gets a gathered copy of the rows."""
         enc = self.graph_conv
-        if isinstance(enc, (GGNN, GGNNMono)) and enc.__dict__.get("mode", K.MODE_F32) == K.MODE_BF16 and _is_ids(table_atoms):
+        if isinstance(enc, (GGNN, GGNNMono)) and _is_ids(table_atoms):
             g = enc(table_atoms, table_adjs, mol_index=rows)
         else:
             rows = rows.long()

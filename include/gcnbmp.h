@@ -81,7 +81,7 @@ typedef struct {
     const int32_t *atoms;        /* (mb,N) or NULL when h_in is given              */
     const float   *h_in;         /* (mb,N,H) or NULL                                */
     const float   *embed_W;      /* (n_atom_types,H); used when atoms != NULL       */
-    const float   *adj;          /* (mb,E,N,N)                                      */
+    const float   *adj;          /* (mb,E,N,N), or the drug table (U,E,N,N) with mol_index; storage per adj_u8 */
     const float   *state_in;     /* (mb,N,H) or NULL (= after reset_state)          */
     const float   *msg_W[BMP_MAX_STEPS];   /* (E*H,H) */
     const float   *msg_b[BMP_MAX_STEPS];   /* (E*H)   */
@@ -96,12 +96,16 @@ typedef struct {
                                  /* bmp_ggnn_stash2_bytes() bytes, the only tape     */
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
-    int    adj_u8;               /* BMP_MODE_BF16 only, storage of `adj`: 0 = fp32 (mb,E,N,N) as the reference; 1 = the same
-                                   array as bytes (exact for 0/1 bonds; 1/4 of the PCIe / HBM traffic); 2 = bit-packed rows
-                                   (mb,E,N,ceil(N/8)), bit j&7 of byte j>>3 = adj[i][j] (numpy.packbits little; 1/32)  */
-    const int32_t *mol_index;    /* BMP_MODE_BF16 only, or NULL.  (mb,) int32: `atoms` (U,N) and `adj` (U,E,N,N) are a device-resident
-                                   drug TABLE and molecule b of this call is its row mol_index[b] (train_binary.py:285-294 builds the
-                                   per-pair copies this replaces); read inside the kernels, no gather copy              */
+    int    adj_u8;               /* storage of `adj`: 0 = fp32 (mb,E,N,N) as the reference; 1 = the same array as bytes (exact
+                                   for 0/1 bonds; 1/4 of the PCIe / HBM traffic; in BMP_MODE_F32 a byte other than 0/1 is a
+                                   general weight); 2 = bit-packed rows (mb,E,N,ceil(N/8)), bit j&7 of byte j>>3 = adj[i][j]
+                                   (numpy.packbits little; 1/32).  BMP_MODE_F32 takes 1 / 2 on the tensor-core row path only
+                                   (tc_workspace >= bmp_ggnn_x3_workspace_bytes(), no state_in): else BMP_EINVAL      */
+    const int32_t *mol_index;    /* or NULL.  (mb,) int32: `atoms` (U,N) and `adj` (U,E,N,N) are a device-resident drug TABLE and
+                                   molecule b of this call is its row mol_index[b] (train_binary.py:285-294 builds the per-pair
+                                   copies this replaces); read inside the kernels, no gather copy.  Needs `atoms` (not h_in).
+                                   BMP_MODE_F32: on the tensor-core row path only (as adj_u8; else BMP_ESHAPE); mb is the
+                                   length of the index, and h_out / h0_out / Hs / Ms / Gs / RSs stay indexed by b        */
 } bmp_ggnn_fwd_t;
 
 int bmp_ggnn_forward(const bmp_ggnn_fwd_t *a, void *stream);
@@ -114,6 +118,10 @@ size_t bmp_ggnn_tc_workspace_bytes(int hidden, int n_steps);
  * stash to the workspace).  The backward must be given a workspace sized with inference = 0; dHs[t] is then updated in
  * place for every t (the FFMA path only writes dHs[0]).  0 = shape not covered (hidden 64/128/256, 4 bond types).          */
 size_t bmp_ggnn_x3_workspace_bytes(int mb, int n_atoms, int hidden, int n_edge, int n_steps, int inference);
+/* The same for one filled-in forward struct (shape, n_steps, state_in, msg_b and the GRU bias pointers are read; tc_workspace is
+ * not): the tc_workspace bytes with which bmp_ggnn_forward runs this call on the tensor-core row path, 0 = it runs the FFMA
+ * kernels (then mol_index and adj_u8 = 1 / 2 are refused).  `inference` as above.  Host-only.                                  */
+size_t bmp_ggnn_x3_forward_bytes(const bmp_ggnn_fwd_t *a, int inference);
 /* Bytes of the bf16 panel stash (forward operand panels + gate values + backward delta/P panels). */
 size_t bmp_ggnn_stash2_bytes(int mb, int hidden, int n_steps);
 
@@ -142,10 +150,11 @@ typedef struct {
                                     unused and dHs is laid out as dHs_every_step says                          */
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
-    int    adj_u8;               /* BMP_MODE_BF16 only, storage of `adj`: 0 = fp32 (mb,E,N,N) as the reference; 1 = the same
-                                   array as bytes (exact for 0/1 bonds; 1/4 of the PCIe / HBM traffic); 2 = bit-packed rows
-                                   (mb,E,N,ceil(N/8)), bit j&7 of byte j>>3 = adj[i][j] (numpy.packbits little; 1/32)  */
-    const int32_t *mol_index;    /* the forward's mol_index: adjacency table rows, or NULL                          */
+    int    adj_u8;               /* storage of `adj` as in the forward; BMP_MODE_F32 takes 1 / 2 on the tensor-core row path only,
+                                   i.e. with a tc_workspace of bmp_ggnn_x3_workspace_bytes(.., inference = 0), else BMP_EINVAL */
+    const int32_t *mol_index;    /* the forward's mol_index: adjacency table rows, or NULL (BMP_MODE_F32: row path only, else
+                                   BMP_ESHAPE; Hs / Ms / Gs / RSs / Ps / dHs stay indexed by b; the embedding gradient is
+                                   the caller's, over the gathered ids)                                                   */
     int    dHs_every_step;       /* BMP_MODE_BF16 only.  0: dHs has TWO slices, [0] = gradient w.r.t. h_0, [1] = gradient
                                     w.r.t. h_T.  Nonzero: dHs (T+1, mb*N, H) as in BMP_MODE_F32, an external gradient for
                                     every h_t.  Either way dHs[0] holds the total gradient w.r.t. h_0 on exit    */
@@ -372,7 +381,7 @@ typedef struct {
     int mb, n1, n2, hidden, out_dim, head, n_classes, n_steps, n_atom_types, mode;
     int coattn_variant, coattn_act;
     const int32_t *atoms_1, *atoms_2;      /* (mb,N1), (mb,N2) */
-    const void    *adj_1, *adj_2;          /* (mb,4,N1,N1), (mb,4,N2,N2): fp32, or the storage `adj_u8` names (BMP_MODE_BF16 only) */
+    const void    *adj_1, *adj_2;          /* (mb,4,N1,N1), (mb,4,N2,N2): fp32, or the storage `adj_u8` names */
     const int32_t *labels;                 /* (mb,n_classes), -1 = ignored */
     float count;                           /* what the loss mean divides by (the GLOBAL count of labels != -1 under data parallelism) */
     const float *embed_W;
@@ -389,7 +398,9 @@ typedef struct {
     float *logits, *loss;
     void  *workspace;
     size_t workspace_bytes;
-    int    adj_u8;                         /* storage of adj_1 / adj_2 as in bmp_ggnn_fwd_t: 0 fp32, 1 bytes, 2 bit-packed rows (BF16 mode) */
+    int    adj_u8;                         /* storage of adj_1 / adj_2 as in bmp_ggnn_fwd_t: 0 fp32, 1 bytes, 2 bit-packed rows.
+                                              BMP_MODE_F32 takes 1 / 2 when both encoders run on the tensor-core row path
+                                              (bmp_ggnn_x3_workspace_bytes(mb, n, ..) > 0 for n1 and n2), else BMP_EINVAL */
 } bmp_pair_t;
 
 size_t bmp_pair_workspace_bytes(int mb, int n1, int n2, int hidden, int out_dim, int head, int n_classes, int n_steps, int mode);
