@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "gcnbmp", "libgcnbmp.so")
-SOURCES = ["misc.cu", "gemm.cu", "heads.cu", "ggnn.cu", "ggnn_x3.cu", "ggnn_tc.cu", "ggnn_tc256.cu", "ggnn_tc_bwd.cu", "wgrad_tc.cu", "wgrad_tc2.cu", "relgcn.cu", "relgcn_tc.cu", "readout.cu", "readout_tc.cu", "coattn.cu", "coattn_big.cu", "coattn_tc.cu", "bimpm.cu", "pair.cu"]
+SOURCES = ["misc.cu", "gemm.cu", "heads.cu", "ggnn.cu", "ggnn_x3.cu", "ggnn_tc.cu", "ggnn_tc256.cu", "ggnn_tc_bwd.cu", "wgrad_tc.cu", "wgrad_tc2.cu", "relgcn.cu", "relgcn_tc.cu", "readout.cu", "readout_tc.cu", "coattn.cu", "coattn_big.cu", "coattn_tc.cu", "bimpm.cu", "pair.cu", "det.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 FLAGS = [f for f in FLAGS if f != "--use_fast_math=false"]

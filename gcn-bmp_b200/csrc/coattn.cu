@@ -6,7 +6,7 @@
 // the reference's two F.tile copies of (mb*N2*N1, H) never exist.  Row/column
 // softmaxes, the head projections and the attended pooling follow in the same CTA.
 // compact_k = j_layer(sum_n attn_k[n] atoms_k[n]) because sum_n attn_k[n] = 1.
-#include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -254,6 +254,7 @@ struct CoBwd {
     const float *dc1, *dc2;
     float *R, *P1, *P2, *DL1, *DL2, *d_a1, *d_a2;
     float *d_V1, *d_V2, *d_b, *d_wa_1, *d_wa_2;
+    CoDet det;          // deterministic mode: per-CTA slots of the vector gradients (det.cuh)
 };
 
 __global__ void __launch_bounds__(NTHREADS, 1) coattn_bwd_kernel(const CoArgs A, const CoBwd B) {
@@ -505,14 +506,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) coattn_bwd_kernel(const CoArgs A,
     }
     __syncthreads();
     for (int h = tid; h < H; h += NTHREADS) {
-        if (B.d_V1) atomicAdd(B.d_V1 + h, gV1[h]);
-        if (B.d_V2) atomicAdd(B.d_V2 + h, gV2[h]);
+        if (B.d_V1) det_put(B.d_V1 + h, B.det.slot(B.det.v(0) + h), gV1[h]);
+        if (B.d_V2) det_put(B.d_V2 + h, B.det.slot(B.det.v(1) + h), gV2[h]);
     }
     if (tid < hd && A.variant == BMP_COATTN_FINE) {
-        if (B.d_wa_1) atomicAdd(B.d_wa_1 + tid, gwa1[tid]);
-        if (B.d_wa_2) atomicAdd(B.d_wa_2 + tid, gwa2[tid]);
+        if (B.d_wa_1) det_put(B.d_wa_1 + tid, B.det.slot(B.det.wa(0) + tid), gwa1[tid]);
+        if (B.d_wa_2) det_put(B.d_wa_2 + tid, B.det.slot(B.det.wa(1) + tid), gwa2[tid]);
     }
-    if (tid == 0 && B.d_b) atomicAdd(B.d_b, gb[0]);
+    if (tid == 0 && B.d_b) det_put(B.d_b, B.det.slot(B.det.b()), gb[0]);
 }
 
 static int co_check(int mb, int n1, int n2, int H, int O, int head, int variant, const void *ws, size_t ws_bytes) {
@@ -592,7 +593,7 @@ extern "C" int bmp_coattn_forward(const bmp_coattn_fwd_t *a, void *stream) {
     return check_launch("coattn_fwd_kernel");
 }
 
-extern "C" int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream) {
+static int coattn_backward_impl(const bmp_coattn_bwd_t *a, void *stream) {
     if (!a || !a->atoms_1 || !a->atoms_2 || !a->W || !a->V1 || !a->V2 || !a->b || !a->W_j || !a->b_j ||
         !a->d_compact_1 || !a->d_compact_2 || !a->R || !a->P1 || !a->P2 || !a->d_atoms_1 || !a->d_atoms_2) {
         set_error("bmp_coattn_backward: null argument");
@@ -622,10 +623,15 @@ extern "C" int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream) {
         B.d_V1 = a->d_V1; B.d_V2 = a->d_V2; B.d_b = a->d_b; B.d_wa_1 = a->d_wa_1; B.d_wa_2 = a->d_wa_2;
         size_t smem = co_smem_floats(A.H, A.head) * sizeof(float);
         int grid = a->mb < 148 ? a->mb : 148;
+        Partials pt((cudaStream_t)stream);
+        if ((rc = co_det_begin(pt, B.det, A.H, grid))) return rc;
         cudaFuncSetAttribute(coattn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         coattn_bwd_kernel<<<grid, NTHREADS, smem, (cudaStream_t)stream>>>(A, B);
         count_launch();
         if ((rc = check_launch("coattn_bwd_kernel"))) return rc;
+        if ((rc = co_det_end(pt, B.det, grid, fine ? a->head : 0, nullptr, nullptr, nullptr, a->d_V1, a->d_V2, a->d_wa_1, a->d_wa_2,
+                             a->d_b, false, "det_reduce_kernel (coattn_bwd)")))
+            return rc;
     }
     const int H = a->hidden, O = a->out_dim, hd = a->head;
     const long rows1 = (long)a->mb * a->n1, rows2 = (long)a->mb * a->n2;
@@ -649,4 +655,20 @@ extern "C" int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream) {
         if (a->d_lt_2 && (rc = bmp_wgrad(a->DL2, hd, a->atoms_2, H, a->d_lt_2, H, rows2, hd, H, stream))) return rc;
     }
     return BMP_OK;
+}
+
+// Bytes of det_scratch (deterministic mode, det.cuh) that bmp_coattn_backward needs for this filled-in struct; 0 = no shape to cover.
+extern "C" size_t bmp_coattn_backward_det_bytes(const bmp_coattn_bwd_t *a) {
+    if (!a) return 0;
+    if (a->mb <= 0 || a->n1 <= 0 || a->n2 <= 0 || a->hidden <= 0 || a->out_dim <= 0) return 0;
+    const int H = a->hidden, O = a->out_dim, M = H > O ? (H > a->head ? H : a->head) : (O > a->head ? O : a->head);
+    return det_max({det_coattn_bytes(a->mb, H), det_wgrad_bytes(M, H), det_wgrad_tc_bytes(M, H), det_colsum_bytes(O)});
+}
+extern "C" int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream) {
+    if (a && a->det_scratch) {
+        int rc = det_check("bmp_coattn_backward", a->det_scratch, a->det_scratch_bytes, bmp_coattn_backward_det_bytes(a));
+        if (rc) return rc;
+    }
+    DetScope ds(a ? a->det_scratch : nullptr, a ? a->det_scratch_bytes : 0);
+    return coattn_backward_impl(a, stream);
 }

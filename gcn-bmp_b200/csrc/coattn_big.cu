@@ -9,7 +9,7 @@
 // The backward recomputes the forward into the same slice, overwrites C^T with dC^T and writes R, P1/P2, DL1/DL2 and d_atoms_k
 // with the meanings of bmp_coattn_bwd_t, so the parameter-gradient calls of bmp_coattn_backward are shared with coattn.cu.
 #include <cstring>
-#include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 namespace big {
@@ -71,6 +71,7 @@ struct Args {
     const float *dc1, *dc2;                     // backward
     float *R, *P1, *P2, *DL1, *DL2, *d_a1, *d_a2;
     float *d_V1, *d_V2, *d_b, *d_wa_1, *d_wa_2;
+    CoDet det;                                  // deterministic mode: per-CTA slots of the vector gradients (det.cuh)
 };
 
 __device__ __forceinline__ float wsum(float v) {
@@ -462,14 +463,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) coattn_big_bwd_kernel(const Args 
     }
     __syncthreads();
     for (int h = tid; h < H; h += NTHREADS) {
-        if (A.d_V1) atomicAdd(A.d_V1 + h, gV1[h]);
-        if (A.d_V2) atomicAdd(A.d_V2 + h, gV2[h]);
+        if (A.d_V1) det_put(A.d_V1 + h, A.det.slot(A.det.v(0) + h), gV1[h]);
+        if (A.d_V2) det_put(A.d_V2 + h, A.det.slot(A.det.v(1) + h), gV2[h]);
     }
     if (tid < hd && fine) {
-        if (A.d_wa_1) atomicAdd(A.d_wa_1 + tid, gwa1[tid]);
-        if (A.d_wa_2) atomicAdd(A.d_wa_2 + tid, gwa2[tid]);
+        if (A.d_wa_1) det_put(A.d_wa_1 + tid, A.det.slot(A.det.wa(0) + tid), gwa1[tid]);
+        if (A.d_wa_2) det_put(A.d_wa_2 + tid, A.det.slot(A.det.wa(1) + tid), gwa2[tid]);
     }
-    if (tid == 0 && A.d_b) atomicAdd(A.d_b, gb);
+    if (tid == 0 && A.d_b) det_put(A.d_b, A.det.slot(A.det.b()), gb);
 }
 
 }  // namespace big
@@ -509,9 +510,16 @@ int bmp_coattn_big(const bmp_coattn_fwd_t *f, const bmp_coattn_bwd_t *bw, void *
     const size_t smem = smem_floats(A.H, A.head) * sizeof(float);
     const int grid = A.mb < CTAS ? A.mb : CTAS;
     const cudaStream_t st = (cudaStream_t)stream;
+    Partials pt(st);
     if (bw) {
+        if (co_det_begin(pt, A.det, A.H, grid)) return BMP_EINVAL;
         cudaFuncSetAttribute(coattn_big_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         coattn_big_bwd_kernel<<<grid, NTHREADS, smem, st>>>(A);
+        count_launch();
+        int rc = check_launch("coattn_big_bwd_kernel");
+        if (rc) return rc;
+        return co_det_end(pt, A.det, grid, A.variant == BMP_COATTN_FINE ? A.head : 0, nullptr, nullptr, nullptr, A.d_V1, A.d_V2,
+                          A.d_wa_1, A.d_wa_2, A.d_b, false, "det_reduce_kernel (coattn_big)");
     } else {
         cudaFuncSetAttribute(coattn_big_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         coattn_big_fwd_kernel<<<grid, NTHREADS, smem, st>>>(A);

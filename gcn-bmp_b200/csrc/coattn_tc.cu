@@ -14,6 +14,7 @@
 // Weights stream from L2 as pre-packed bf16 tiles (cp.async.bulk + mbarrier ring); warp 16 produces, warp 17
 // issues the MMAs, warps 0-15 own TMEM lane quarter (warp % 4) and column group (warp / 4).
 #include "tc_common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 namespace ctc {
@@ -37,6 +38,7 @@ struct Args {
     const float *dc1, *dc2;
     float *R, *P1, *P2, *DL1, *DL2, *d_a1, *d_a2;
     float *d_W, *d_lt_1, *d_lt_2, *d_V1, *d_V2, *d_b, *d_wa_1, *d_wa_2;
+    CoDet det;                   // deterministic mode: this CTA's slot takes the flush below instead of the atomics
     long long *dbg;              // optional phase timestamps of CTA 0, second pair (tools/co_timeline.py)
 };
 
@@ -839,11 +841,11 @@ __global__ void __launch_bounds__(NT, 1) coattn_tc_kernel(const Args a) {
                 uint32_t v[32];
                 tc_ld32(t_lane + C::COL_DW + cg * 32, v);
                 tc_wait_ld();
-                float *dst = a.d_W + (long)row * H + cg * 32;
+                float *dst = a.d_W + (long)row * H + cg * 32, *sp = a.det.slot(a.det.w() + (long)row * H + cg * 32);
 #pragma unroll
                 for (int x = 0; x < 32; x += 4)
-                    atomicAdd(reinterpret_cast<float4 *>(dst + x),
-                              make_float4(__uint_as_float(v[x]), __uint_as_float(v[x + 1]), __uint_as_float(v[x + 2]), __uint_as_float(v[x + 3])));
+                    det_put4(dst + x, sp ? sp + x : nullptr,
+                             make_float4(__uint_as_float(v[x]), __uint_as_float(v[x + 1]), __uint_as_float(v[x + 2]), __uint_as_float(v[x + 3])));
             }
             if (row < H && cg >= 2) {                         // [d lt_k | d V_k]^T: lane = feature, column = head (15: V)
                 const int k2 = cg - 2;
@@ -853,16 +855,16 @@ __global__ void __launch_bounds__(NT, 1) coattn_tc_kernel(const Args a) {
                 float *dlt = k2 ? a.d_lt_2 : a.d_lt_1, *dV = k2 ? a.d_V2 : a.d_V1;
 #pragma unroll
                 for (int d = 0; d < MAXHD; ++d)
-                    if (d < hd && dlt) atomicAdd(dlt + (long)d * H + row, __uint_as_float(w[d]));
-                if (dV) atomicAdd(dV + row, __uint_as_float(w[15]));
+                    if (d < hd && dlt) det_put(dlt + (long)d * H + row, a.det.slot(a.det.lt(k2) + (long)d * H + row), __uint_as_float(w[d]));
+                if (dV) det_put(dV + row, a.det.slot(a.det.v(k2) + row), __uint_as_float(w[15]));
             }
             tc_fence_before();
             EPI_SYNC();
             if (tid < hd) {
-                if (a.d_wa_1) atomicAdd(a.d_wa_1 + tid, gwa1[tid]);
-                if (a.d_wa_2) atomicAdd(a.d_wa_2 + tid, gwa2[tid]);
+                if (a.d_wa_1) det_put(a.d_wa_1 + tid, a.det.slot(a.det.wa(0) + tid), gwa1[tid]);
+                if (a.d_wa_2) det_put(a.d_wa_2 + tid, a.det.slot(a.det.wa(1) + tid), gwa2[tid]);
             }
-            if (tid == 0 && a.d_b) atomicAdd(a.d_b, gb[0]);
+            if (tid == 0 && a.d_b) det_put(a.d_b, a.det.slot(a.det.b()), gb[0]);
         }
     }
     tc_fence_before();
@@ -950,11 +952,19 @@ static int launch_ctc_hp(const ctc::Args &k, int head, cudaStream_t st) {
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int grid = k.mb < sms ? k.mb : sms;
     const size_t smem = ctc::smem_bytes<H, BWD>(head);
+    Partials pt(st);
+    ctc::Args kk = k;
+    if (BWD && co_det_begin(pt, kk.det, H, grid)) return BMP_EINVAL;
     cudaFuncSetAttribute(ctc::coattn_tc_kernel<H, BWD, HP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    ProfScope prof(BWD ? BMP_PROF_COATTN_BWD : BMP_PROF_COATTN_FWD, st);
-    ctc::coattn_tc_kernel<H, BWD, HP><<<grid, ctc::NT, smem, st>>>(k);
+    {
+        ProfScope prof(BWD ? BMP_PROF_COATTN_BWD : BMP_PROF_COATTN_FWD, st);
+        ctc::coattn_tc_kernel<H, BWD, HP><<<grid, ctc::NT, smem, st>>>(kk);
+    }
     count_launch();
-    return check_launch("coattn_tc_kernel");
+    int rc = check_launch("coattn_tc_kernel");
+    if (rc || !BWD) return rc;
+    return co_det_end(pt, kk.det, grid, head, k.d_W, k.d_lt_1, k.d_lt_2, k.d_V1, k.d_V2, k.d_wa_1, k.d_wa_2, k.d_b, true,
+                      "det_reduce_kernel (coattn_tc)");
 }
 
 template <int H, bool BWD>

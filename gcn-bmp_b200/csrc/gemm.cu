@@ -1,7 +1,7 @@
 // gemm.cu -- the dense pieces that are not per-molecule: parameter-gradient
 // contractions over all atoms of a batch (C += A^T B), column sums for bias
 // gradients, and the links.Linear layers of the heads (hole.py:21-26).
-#include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -14,7 +14,7 @@ __global__ void __launch_bounds__(NTHREADS) wgrad_kernel(const float *__restrict
                                                          const float *__restrict__ B, int ldb,
                                                          float *__restrict__ C, int ldc,
                                                          long rows, int M, int N, int tilesN, long rows_per_cta,
-                                                         int vec) {
+                                                         int vec, float *__restrict__ part) {
     __shared__ __align__(16) float As[2][RT][WLD];
     __shared__ __align__(16) float Bs[2][RT][WLD];
     const int tid = threadIdx.x;
@@ -76,13 +76,15 @@ __global__ void __launch_bounds__(NTHREADS) wgrad_kernel(const float *__restrict
     for (int a = 0; a < 4; ++a)
 #pragma unroll
         for (int b = 0; b < 4; ++b)
-            if (tm + m0 + a < M && tn + n0 + b < N) atomicAdd(C + (long)(tm + m0 + a) * ldc + tn + n0 + b, acc[a][b]);
+            if (tm + m0 + a < M && tn + n0 + b < N)       // deterministic mode: slot blockIdx.y of the (M,N) partials
+                det_put(C + (long)(tm + m0 + a) * ldc + tn + n0 + b,
+                        part ? part + ((long)blockIdx.y * M + tm + m0 + a) * N + tn + n0 + b : nullptr, acc[a][b]);
 }
 
 // out[n*ostride] += sum_r B[r*ldb + n]
 __global__ void __launch_bounds__(NTHREADS) colsum_kernel(const float *__restrict__ B, int ldb,
                                                           float *__restrict__ out, int ostride, long rows, int N,
-                                                          long rows_per_cta) {
+                                                          long rows_per_cta, float *__restrict__ part) {
     __shared__ float red[4][64];
     const int col = blockIdx.x * 64 + (threadIdx.x & 63), rg = threadIdx.x >> 6;
     const long r_begin = (long)blockIdx.y * rows_per_cta;
@@ -94,7 +96,7 @@ __global__ void __launch_bounds__(NTHREADS) colsum_kernel(const float *__restric
     __syncthreads();
     if (rg == 0 && col < N) {
         s = red[0][threadIdx.x] + red[1][threadIdx.x] + red[2][threadIdx.x] + red[3][threadIdx.x];
-        atomicAdd(out + (long)col * ostride, s);
+        det_put(out + (long)col * ostride, part ? part + (long)blockIdx.y * N + col : nullptr, s);
     }
 }
 
@@ -229,9 +231,15 @@ extern "C" int bmp_wgrad(const float *A, int lda, const float *B, int ldb, float
     rpc = (rpc + RT - 1) / RT * RT;
     split = (rows + rpc - 1) / rpc;
     dim3 grid(tiles, (unsigned)split);
-    wgrad_kernel<<<grid, NTHREADS, 0, (cudaStream_t)stream>>>(A, lda, B, ldb, C, ldc, rows, M, N, tilesN, rpc, vec);
+    Partials pt((cudaStream_t)stream);
+    float *part = det_on() ? pt.take(split * M * N) : nullptr;
+    if (det_on() && !part) return BMP_EINVAL;
+    wgrad_kernel<<<grid, NTHREADS, 0, (cudaStream_t)stream>>>(A, lda, B, ldb, C, ldc, rows, M, N, tilesN, rpc, vec, part);
     count_launch();
-    return check_launch("wgrad_kernel");
+    int rc = check_launch("wgrad_kernel");
+    if (rc || !part) return rc;
+    pt.add(C, ldc, M, N, part, (int)split, (long)M * N);
+    return pt.reduce("det_reduce_kernel (bmp_wgrad)");
 }
 
 extern "C" int bmp_colsum(const float *B, int ldb, float *out, int out_stride, int64_t rows, int N, void *stream) {
@@ -246,9 +254,15 @@ extern "C" int bmp_colsum(const float *B, int ldb, float *out, int out_stride, i
     long rpc = (rows + split - 1) / split;
     split = (rows + rpc - 1) / rpc;
     dim3 grid(tiles, (unsigned)split);
-    colsum_kernel<<<grid, NTHREADS, 0, (cudaStream_t)stream>>>(B, ldb, out, out_stride, rows, N, rpc);
+    Partials pt((cudaStream_t)stream);
+    float *part = det_on() ? pt.take(split * N) : nullptr;
+    if (det_on() && !part) return BMP_EINVAL;
+    colsum_kernel<<<grid, NTHREADS, 0, (cudaStream_t)stream>>>(B, ldb, out, out_stride, rows, N, rpc, part);
     count_launch();
-    return check_launch("colsum_kernel");
+    int rc = check_launch("colsum_kernel");
+    if (rc || !part) return rc;
+    pt.add(out, out_stride, N, 1, part, (int)split, N);
+    return pt.reduce("det_reduce_kernel (bmp_colsum)");
 }
 
 extern "C" int bmp_linear_forward(const float *x, const float *W, const float *b, float *y,
@@ -287,4 +301,19 @@ extern "C" int bmp_linear_backward(const float *x, const float *W, const float *
     }
     if (db && (rc = bmp_colsum(dy, out_dim, db, 1, rows, out_dim, stream))) return rc;
     return BMP_OK;
+}
+
+// Deterministic sibling (det.cuh): dW / db summed over the row split in fixed order in `scratch`.
+extern "C" size_t bmp_linear_backward_det_bytes(int rows, int in_dim, int out_dim) {
+    if (rows <= 0 || in_dim <= 0 || out_dim <= 0) return 0;
+    const size_t a = det_wgrad_bytes(out_dim, in_dim), b = det_colsum_bytes(out_dim);
+    return a > b ? a : b;
+}
+extern "C" int bmp_linear_backward_det(const float *x, const float *W, const float *y, float *dy, float *dx, float *dW, float *db,
+                                       int rows, int in_dim, int out_dim, int act, void *stream, void *scratch, size_t scratch_bytes) {
+    if (!scratch) { set_error("bmp_linear_backward_det: NULL scratch"); return BMP_EINVAL; }
+    int rc = det_check("bmp_linear_backward_det", scratch, scratch_bytes, bmp_linear_backward_det_bytes(rows, in_dim, out_dim));
+    if (rc) return rc;
+    DetScope ds(scratch, scratch_bytes);
+    return bmp_linear_backward(x, W, y, dy, dx, dW, db, rows, in_dim, out_dim, act, stream);
 }

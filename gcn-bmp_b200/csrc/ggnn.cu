@@ -10,6 +10,7 @@
 // W_e = W_m[e::E] (the c*E+e interleave of ggnn_update.py:35-39 becomes a row
 // stride), so the (mb,E,N,H) tensors of the reference never exist.
 #include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -646,7 +647,7 @@ extern "C" int bmp_ggnn_forward(const bmp_ggnn_fwd_t *a, void *stream) {
     return check_launch("ggnn_fwd_kernel");
 }
 
-extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
+static int ggnn_backward_impl(const bmp_ggnn_bwd_t *a, void *stream) {
     if (a && (a->stash2 || a->mode == BMP_MODE_BF16)) {
         if (!a->stash2 || a->mode != BMP_MODE_BF16) {
             set_error("bmp_ggnn_backward: BMP_MODE_BF16 trains on the bf16 panel stash: stash2 (written by the forward) is required, "
@@ -774,4 +775,21 @@ extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
         t0 = t1 + 1;
     }
     return BMP_OK;
+}
+
+// Bytes of det_scratch (deterministic mode, det.cuh) that bmp_ggnn_backward needs for this filled-in struct; 0 = no shape to cover.
+extern "C" size_t bmp_ggnn_backward_det_bytes(const bmp_ggnn_bwd_t *a) {
+    if (!a) return 0;
+    const int H = a->hidden;
+    if (a->mb <= 0 || a->n_atoms <= 0 || H <= 0 || a->n_steps <= 0) return 0;
+    size_t n = det_max({det_wgrad_bytes(H, H), det_wgrad_tc_bytes(H, H), det_colsum_bytes(H)});
+    return a->mode == BMP_MODE_BF16 ? det_max({n, det_panels_bytes()}) : n;
+}
+extern "C" int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream) {
+    if (a && a->det_scratch) {
+        int rc = det_check("bmp_ggnn_backward", a->det_scratch, a->det_scratch_bytes, bmp_ggnn_backward_det_bytes(a));
+        if (rc) return rc;
+    }
+    DetScope ds(a ? a->det_scratch : nullptr, a ? a->det_scratch_bytes : 0);
+    return ggnn_backward_impl(a, stream);
 }

@@ -6,7 +6,7 @@
 //                   rank-R reduction -- Chainer's (B, L, R) outer product is never materialised
 //   gradient hooks  GradientClipping -> WeightDecay -> Lasso in the order train_binary.py:537-543 adds them
 // HBM-bound elementwise / reduction work: grid-stride loops, float4 where the shapes allow.
-#include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -289,7 +289,7 @@ __global__ void embed_fwd_kernel(const int32_t *__restrict__ ids, const float *_
 }
 
 // ---------------------------------------------------------------- optimizer hooks
-__global__ void sumsq_kernel(const float *__restrict__ g, long n, float *__restrict__ out) {
+__global__ void sumsq_kernel(const float *__restrict__ g, long n, float *__restrict__ out, float *__restrict__ part) {
     float s = 0.f;
     for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) s = fmaf(g[i], g[i], s);
 #pragma unroll
@@ -300,7 +300,7 @@ __global__ void sumsq_kernel(const float *__restrict__ g, long n, float *__restr
     if (threadIdx.x == 0) {
         float tot = 0.f;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += red[w];
-        atomicAdd(out, tot);
+        det_put(out, part ? part + blockIdx.x : nullptr, tot);     // deterministic mode: slot blockIdx.x
     }
 }
 __global__ void hooks_kernel(float *__restrict__ g, const float *__restrict__ p, long n, float clip, float l2, float l1,
@@ -508,11 +508,46 @@ extern "C" int bmp_grad_hooks(float *grad, const float *param, int n, float clip
     if (clip_threshold > 0.f) {
         if (!norm_ws) { set_error("bmp_grad_hooks: GradientClipping needs one float of device scratch (norm_ws)"); return BMP_EINVAL; }
         if (cudaMemsetAsync(norm_ws, 0, sizeof(float), st) != cudaSuccess) { set_error("bmp_grad_hooks: memset failed"); return BMP_ECUDA; }
-        sumsq_kernel<<<grid_for(n), 256, 0, st>>>(grad, n, norm_ws);
+        Partials pt(st);
+        float *part = det_on() ? pt.take(grid_for(n)) : nullptr;
+        if (det_on() && !part) return BMP_EINVAL;
+        sumsq_kernel<<<grid_for(n), 256, 0, st>>>(grad, n, norm_ws, part);
         count_launch();
         if ((rc = check_launch("sumsq_kernel"))) return rc;
+        if (part) {
+            pt.add(norm_ws, 1, 1, 1, part, grid_for(n), 1);
+            if ((rc = pt.reduce("det_reduce_kernel (bmp_grad_hooks)"))) return rc;
+        }
     }
     hooks_kernel<<<grid_for(n), 256, 0, st>>>(grad, param, n, clip_threshold, l2_rate, l1_rate, norm_ws);
     count_launch();
     return check_launch("hooks_kernel");
+}
+
+// Deterministic sibling (det.cuh): the clipping norm is summed in block order in `scratch`.
+extern "C" size_t bmp_grad_hooks_det_bytes(int n) { return n > 0 ? (size_t)grid_for(n) * sizeof(float) + 512 : 0; }
+extern "C" int bmp_grad_hooks_det(float *grad, const float *param, int n, float clip_threshold, float l2_rate, float l1_rate,
+                                  float *norm_ws, void *stream, void *scratch, size_t scratch_bytes) {
+    if (!scratch) { set_error("bmp_grad_hooks_det: NULL scratch"); return BMP_EINVAL; }
+    int rc = det_check("bmp_grad_hooks_det", scratch, scratch_bytes, bmp_grad_hooks_det_bytes(n));
+    if (rc) return rc;
+    DetScope ds(scratch, scratch_bytes);
+    return bmp_grad_hooks(grad, param, n, clip_threshold, l2_rate, l1_rate, norm_ws, stream);
+}
+
+// Deterministic sibling (det.cuh): dW, dV1, dV2, db summed over the row split in fixed order in `scratch`.
+extern "C" size_t bmp_bilinear_backward_det_bytes(int rows, int left, int right, int out) {
+    if (rows <= 0 || left <= 0 || right <= 0 || out <= 0) return 0;
+    const int M = left > right ? left : right;
+    return det_max({det_wgrad_bytes(M, right * out), det_colsum_bytes(out)});
+}
+extern "C" int bmp_bilinear_backward_det(const float *e1, const float *e2, const float *W, const float *V1, const float *V2,
+                                         const float *u, const float *dy, float *du, float *de1, float *de2, float *dW, float *dV1,
+                                         float *dV2, float *db, int rows, int left, int right, int out, void *stream, void *scratch,
+                                         size_t scratch_bytes) {
+    if (!scratch) { set_error("bmp_bilinear_backward_det: NULL scratch"); return BMP_EINVAL; }
+    int rc = det_check("bmp_bilinear_backward_det", scratch, scratch_bytes, bmp_bilinear_backward_det_bytes(rows, left, right, out));
+    if (rc) return rc;
+    DetScope ds(scratch, scratch_bytes);
+    return bmp_bilinear_backward(e1, e2, W, V1, V2, u, dy, du, de1, de2, dW, dV1, dV2, db, rows, left, right, out, stream);
 }

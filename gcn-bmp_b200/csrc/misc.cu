@@ -6,7 +6,7 @@
 #include <atomic>
 #include <mutex>
 #include <vector>
-#include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -132,6 +132,7 @@ __global__ void __launch_bounds__(256) embed_bwd_kernel(const int32_t *__restric
     }
 }
 
+// (ldh = row stride of dh: H, or the full width when a deterministic call runs one column tile of a wide table.)
 // Atomic-free variant: a CTA owns a contiguous block of rows; its 256 threads form two row partitions of 128
 // column owners.  A thread is the only writer of "its" columns of its partition's private table, so the
 // scatter-add is a plain shared-memory read-modify-write in row order; the two tables are merged on the way out.
@@ -139,7 +140,7 @@ __global__ void __launch_bounds__(256) embed_bwd_kernel(const int32_t *__restric
 constexpr int EMB_U = 16;
 __global__ void __launch_bounds__(256) embed_bwd_owner_kernel(const int32_t *__restrict__ ids, const float *__restrict__ dh,
                                                               float *__restrict__ dW, long rows, int H, int n_types,
-                                                              long rows_per_cta) {
+                                                              long rows_per_cta, float *__restrict__ slots, long ldh) {
     extern __shared__ float tab[];   // [2][n_types][H]
     const int n = n_types * H;
     for (int i = threadIdx.x; i < 2 * n; i += blockDim.x) tab[i] = 0.f;
@@ -157,7 +158,7 @@ __global__ void __launch_bounds__(256) embed_bwd_owner_kernel(const int32_t *__r
                 const bool ok = r + u < r1;
                 const int x = ok ? __ldg(ids + r + u) : 0;
                 id[b][u] = x < 0 ? 0 : (x >= n_types ? n_types - 1 : x);
-                v[b][u] = ok ? __ldg(dh + (r + u) * H + c) : 0.f;
+                v[b][u] = ok ? __ldg(dh + (r + u) * ldh + c) : 0.f;
             }
         };
         long r = r0 + part * EMB_U;
@@ -175,13 +176,15 @@ __global__ void __launch_bounds__(256) embed_bwd_owner_kernel(const int32_t *__r
     __syncthreads();
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
         const float v = tab[i] + tab[n + i];
-        if (v != 0.f) atomicAdd(dW + i, v);
+        if (slots) slots[(long)blockIdx.x * n + i] = v;       // deterministic mode: slot blockIdx.x
+        else if (v != 0.f) atomicAdd(dW + i, v);
     }
 }
 
 // ---- sigmoid cross entropy ------------------------------------------------------
 __global__ void __launch_bounds__(256) sce_kernel(const float *__restrict__ x, const int32_t *__restrict__ t,
-                                                  float *__restrict__ loss, float *__restrict__ dx, long n, float inv_count) {
+                                                  float *__restrict__ loss, float *__restrict__ dx, long n, float inv_count,
+                                                  float *__restrict__ part) {
     __shared__ float red[8];
     float s = 0.f;
     for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) {
@@ -198,7 +201,7 @@ __global__ void __launch_bounds__(256) sce_kernel(const float *__restrict__ x, c
     if (threadIdx.x < 8) {
         s = red[threadIdx.x];
         for (int o = 4; o; o >>= 1) s += __shfl_xor_sync(0xffu, s, o);
-        if (threadIdx.x == 0 && loss) atomicAdd(loss, s * inv_count);
+        if (threadIdx.x == 0 && loss) det_put(loss, part ? part + blockIdx.x : nullptr, s * inv_count);
     }
 }
 
@@ -221,7 +224,7 @@ __global__ void adam_kernel(float *__restrict__ p, const float *__restrict__ g, 
 using namespace bmp;
 
 extern "C" const char *bmp_last_error(void) { return g_err; }
-extern "C" int bmp_version(void) { return 100; }
+extern "C" int bmp_version(void) { return 101; }
 extern "C" uint64_t bmp_launch_count(void) { return g_launches.load(); }
 extern "C" void bmp_reset_launch_count(void) { g_launches.store(0); }
 
@@ -278,20 +281,55 @@ extern "C" int bmp_hole_corr_backward(const float *left, const float *right, con
     return check_launch("hole_bwd_kernel");
 }
 
+// Columns per launch of the owner kernel: its two [n_types][cols] tables fit 200 KB of shared memory.  The default path runs it
+// when the whole table fits; the deterministic path also runs wider tables as column tiles (the fallback kernel below
+// scatters with shared-memory atomics, whose order is not fixed).
+static int embed_tile_cols(int hidden, int n_atom_types) {
+    const long c = 200L * 1024 / (2 * sizeof(float)) / (n_atom_types > 0 ? n_atom_types : 1);
+    return c >= hidden ? hidden : (int)(c & ~3L);
+}
+static size_t embed_det_bytes(int rows, int hidden, int n_atom_types) {
+    const int tc = embed_tile_cols(hidden, n_atom_types);
+    if (rows <= 0 || hidden <= 0 || n_atom_types <= 0 || tc < 4) return 0;
+    return 148 * (size_t)n_atom_types * tc * sizeof(float) + 512;
+}
+
+// One owner-kernel launch over columns [c0, c0 + cols) of the table (all of it when cols == hidden).
+static int embed_owner(const int32_t *atoms, const float *dh, float *d_embed_W, int rows, int hidden, int c0, int cols,
+                       int n_atom_types, cudaStream_t st) {
+    const size_t smem = (size_t)n_atom_types * cols * sizeof(float);
+    const int ctas = 148;
+    long rpc = ((long)rows + ctas - 1) / ctas;
+    rpc = (rpc + 2 * EMB_U - 1) / (2 * EMB_U) * (2 * EMB_U);
+    const int grid = (int)(((long)rows + rpc - 1) / rpc);
+    Partials pt(st);
+    const long n = (long)n_atom_types * cols;
+    float *part = det_on() ? pt.take(grid * n) : nullptr;
+    if (det_on() && !part) return BMP_EINVAL;
+    cudaFuncSetAttribute(embed_bwd_owner_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * smem));
+    embed_bwd_owner_kernel<<<grid, 256, 2 * smem, st>>>(atoms, dh + c0, d_embed_W + c0, rows, cols, n_atom_types, rpc, part, hidden);
+    count_launch();
+    int rc = check_launch("embed_bwd_owner_kernel");
+    if (rc || !part) return rc;
+    pt.add(d_embed_W + c0, hidden, n_atom_types, cols, part, grid, n);
+    return pt.reduce("det_reduce_kernel (bmp_embed_backward)");
+}
+
 extern "C" int bmp_embed_backward(const int32_t *atoms, const float *dh, float *d_embed_W,
                                   int rows, int hidden, int n_atom_types, void *stream) {
     if (!atoms || !dh || !d_embed_W) { set_error("bmp_embed_backward: null pointer"); return BMP_EINVAL; }
     if (rows <= 0) return BMP_OK;
     size_t smem = (size_t)n_atom_types * hidden * sizeof(float);
-    if (2 * smem <= 200 * 1024) {
-        const int ctas = 148;
-        long rpc = ((long)rows + ctas - 1) / ctas;
-        rpc = (rpc + 2 * EMB_U - 1) / (2 * EMB_U) * (2 * EMB_U);
-        const int grid = (int)(((long)rows + rpc - 1) / rpc);
-        cudaFuncSetAttribute(embed_bwd_owner_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * smem));
-        embed_bwd_owner_kernel<<<grid, 256, 2 * smem, (cudaStream_t)stream>>>(atoms, dh, d_embed_W, rows, hidden, n_atom_types, rpc);
-        count_launch();
-        return check_launch("embed_bwd_owner_kernel");
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (2 * smem <= 200 * 1024) return embed_owner(atoms, dh, d_embed_W, rows, hidden, 0, hidden, n_atom_types, st);
+    if (det_on()) {
+        const int tc = embed_tile_cols(hidden, n_atom_types);
+        if (tc < 4) { set_error("bmp_embed_backward_det: %d atom types do not fit a 4-column tile", n_atom_types); return BMP_ESHAPE; }
+        for (int c0 = 0; c0 < hidden; c0 += tc) {
+            const int rc = embed_owner(atoms, dh, d_embed_W, rows, hidden, c0, hidden - c0 < tc ? hidden - c0 : tc, n_atom_types, st);
+            if (rc) return rc;
+        }
+        return BMP_OK;
     }
     if (smem > 200 * 1024) { set_error("bmp_embed_backward: table %d x %d does not fit shared memory", n_atom_types, hidden); return BMP_ESHAPE; }
     int grid = 148 * 2;
@@ -310,9 +348,41 @@ extern "C" int bmp_sigmoid_ce(const float *logits, const int32_t *labels, float 
     if (n <= 0) return BMP_OK;
     int grid = (n + 255) / 256;
     if (grid > 148 * 8) grid = 148 * 8;
-    sce_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(logits, labels, loss_sum, d_logits, n, 1.f / (count > 0.f ? count : 1.f));
+    Partials pt((cudaStream_t)stream);
+    float *part = det_on() && loss_sum ? pt.take(grid) : nullptr;
+    if (det_on() && loss_sum && !part) return BMP_EINVAL;
+    sce_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(logits, labels, loss_sum, d_logits, n, 1.f / (count > 0.f ? count : 1.f), part);
     count_launch();
-    return check_launch("sce_kernel");
+    int rc = check_launch("sce_kernel");
+    if (rc || !part) return rc;
+    pt.add(loss_sum, 1, 1, 1, part, grid, 1);
+    return pt.reduce("det_reduce_kernel (bmp_sigmoid_ce)");
+}
+
+// ---- deterministic siblings (det.cuh): the same work with fixed-order cross-CTA sums in `scratch`
+extern "C" size_t bmp_embed_backward_det_bytes(int rows, int hidden, int n_atom_types) {
+    return embed_det_bytes(rows, hidden, n_atom_types);
+}
+extern "C" int bmp_embed_backward_det(const int32_t *atoms, const float *dh, float *d_embed_W, int rows, int hidden,
+                                      int n_atom_types, void *stream, void *scratch, size_t scratch_bytes) {
+    if (!scratch) { set_error("bmp_embed_backward_det: NULL scratch"); return BMP_EINVAL; }
+    int rc = det_check("bmp_embed_backward_det", scratch, scratch_bytes, embed_det_bytes(rows, hidden, n_atom_types));
+    if (rc) return rc;
+    DetScope ds(scratch, scratch_bytes);
+    return bmp_embed_backward(atoms, dh, d_embed_W, rows, hidden, n_atom_types, stream);
+}
+extern "C" size_t bmp_sigmoid_ce_det_bytes(int n) {
+    if (n <= 0) return 0;
+    const long grid = (n + 255) / 256 > 148 * 8 ? 148 * 8 : (n + 255) / 256;
+    return (size_t)grid * sizeof(float) + 512;
+}
+extern "C" int bmp_sigmoid_ce_det(const float *logits, const int32_t *labels, float *loss_sum, float *d_logits, int n, float count,
+                                  void *stream, void *scratch, size_t scratch_bytes) {
+    if (!scratch) { set_error("bmp_sigmoid_ce_det: NULL scratch"); return BMP_EINVAL; }
+    int rc = det_check("bmp_sigmoid_ce_det", scratch, scratch_bytes, bmp_sigmoid_ce_det_bytes(n));
+    if (rc) return rc;
+    DetScope ds(scratch, scratch_bytes);
+    return bmp_sigmoid_ce(logits, labels, loss_sum, d_logits, n, count, stream);
 }
 
 extern "C" int bmp_adam_step(float *param, const float *grad, float *m, float *v, int n,

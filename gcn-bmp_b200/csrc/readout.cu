@@ -8,6 +8,7 @@
 // state (an atom's gradient depends on dg and its own row only).  Up to 64 atoms there
 // is one chunk and the arithmetic is that of the single-tile kernel.
 #include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -192,7 +193,7 @@ extern "C" int bmp_readout_forward(const bmp_readout_fwd_t *a, void *stream) {
     return check_launch("readout_kernel<fwd>");
 }
 
-extern "C" int bmp_readout_backward(const bmp_readout_bwd_t *a, void *stream) {
+static int readout_backward_impl(const bmp_readout_bwd_t *a, void *stream) {
     if (!a || !a->dg) { set_error("bmp_readout_backward: null argument"); return BMP_EINVAL; }
     int rc = readout_check(a->mb, a->n_atoms, a->hidden, a->out_dim, a->variant, a->h);
     if (rc) return rc;
@@ -250,4 +251,20 @@ extern "C" int bmp_readout_backward(const bmp_readout_bwd_t *a, void *stream) {
     if (a->d_b_i && !bi_done && (rc = bmp_colsum(a->DU, O, a->d_b_i, 1, rows, O, stream))) return rc;
     if (a->d_b_j && !bj_done && (rc = bmp_colsum(a->DV, O, a->d_b_j, 1, rows, O, stream))) return rc;
     return BMP_OK;
+}
+
+// Bytes of det_scratch (deterministic mode, det.cuh) that bmp_readout_backward needs for this filled-in struct; 0 = no shape to cover.
+extern "C" size_t bmp_readout_backward_det_bytes(const bmp_readout_bwd_t *a) {
+    if (!a) return 0;
+    if (a->mb <= 0 || a->n_atoms <= 0 || a->hidden <= 0 || a->out_dim <= 0) return 0;
+    const int O = a->out_dim, K = 2 * a->hidden;
+    return det_max({det_wgrad_bytes(O, K), det_wgrad_tc_bytes(O, K), det_colsum_bytes(O)});
+}
+extern "C" int bmp_readout_backward(const bmp_readout_bwd_t *a, void *stream) {
+    if (a && a->det_scratch) {
+        int rc = det_check("bmp_readout_backward", a->det_scratch, a->det_scratch_bytes, bmp_readout_backward_det_bytes(a));
+        if (rc) return rc;
+    }
+    DetScope ds(a ? a->det_scratch : nullptr, a ? a->det_scratch_bytes : 0);
+    return readout_backward_impl(a, stream);
 }

@@ -6,6 +6,7 @@
 // exactly like the GGNN message (ggnn.cu), with the column-degree normalisation
 // folded into the adjacency tile while it is staged.
 #include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 
@@ -254,7 +255,7 @@ extern "C" int bmp_relgcn_forward(const bmp_relgcn_fwd_t *a, void *stream) {
     return check_launch("relgcn_fwd_kernel");
 }
 
-extern "C" int bmp_relgcn_backward(const bmp_relgcn_bwd_t *a, void *stream) {
+static int relgcn_backward_impl(const bmp_relgcn_bwd_t *a, void *stream) {
     if (a && a->mode == BMP_MODE_BF16) {
         if (!a->adj) { set_error("bmp_relgcn_backward: null argument"); return BMP_EINVAL; }
         if (a->mb <= 0 || a->n_atoms <= 0 || a->n_atoms > BMP_MAX_ATOMS || !bmp_relgcn_tc_supported(a->ch, a->n_layers, a->n_edge)) {
@@ -318,4 +319,24 @@ extern "C" int bmp_relgcn_backward(const bmp_relgcn_bwd_t *a, void *stream) {
         ps_off += rows * E * Cout;
     }
     return BMP_OK;
+}
+
+// Bytes of det_scratch (deterministic mode, det.cuh) that bmp_relgcn_backward needs for this filled-in struct; 0 = no shape to cover.
+extern "C" size_t bmp_relgcn_backward_det_bytes(const bmp_relgcn_bwd_t *a) {
+    if (!a) return 0;
+    if (a->mb <= 0 || a->n_atoms <= 0 || a->n_layers <= 0 || a->n_layers > BMP_MAX_STEPS) return 0;
+    int c = 0;
+    for (int l = 0; l <= a->n_layers; ++l) c = a->ch[l] > c ? a->ch[l] : c;
+    if (c <= 0) return 0;
+    c = c <= 64 ? 64 : (c <= 128 ? 128 : 256 > c ? 256 : c);     // the tensor-core row path pads every layer
+    size_t n = det_max({det_wgrad_bytes(c, c), det_wgrad_tc_bytes(c, c), det_colsum_bytes(c)});
+    return a->mode == BMP_MODE_BF16 ? det_max({n, det_panels_bytes()}) : n;
+}
+extern "C" int bmp_relgcn_backward(const bmp_relgcn_bwd_t *a, void *stream) {
+    if (a && a->det_scratch) {
+        int rc = det_check("bmp_relgcn_backward", a->det_scratch, a->det_scratch_bytes, bmp_relgcn_backward_det_bytes(a));
+        if (rc) return rc;
+    }
+    DetScope ds(a ? a->det_scratch : nullptr, a ? a->det_scratch_bytes : 0);
+    return relgcn_backward_impl(a, stream);
 }

@@ -452,6 +452,8 @@ struct Multi {
     Args cls[MAX_CLASSES];
     int n;
     int cta0[MAX_CLASSES + 1];         // class c owns CTAs [cta0[c], cta0[c+1])
+    float *part[MAX_CLASSES];          // deterministic mode: class c's [CTAs][plen] partials (det.cuh), else nullptr
+    long plen[MAX_CLASSES];
 };
 }  // namespace w2
 }  // namespace bmp

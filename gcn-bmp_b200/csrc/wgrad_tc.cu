@@ -11,7 +11,7 @@
 // bf16 hi / lo pair (x = hi + lo up to 2^-17 relative) and each k-step issues three UMMAs, hi.hi + lo.hi + hi.lo, into the fp32
 // TMEM accumulator (the lo.lo term is below fp32 rounding of the sum).
 #include <cuda_bf16.h>
-#include "common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 namespace wtc {
@@ -59,6 +59,7 @@ struct Args {
     float *C, *dbias;
     int lda, ldb, ldc, M, N, bias_stride;
     long rows, rows_per_cta;
+    float *part, *bpart;     // deterministic mode: [split][M][N] and [split][M] partials (slot blockIdx.y), else nullptr
 };
 
 template <int N, bool SPLIT>
@@ -179,7 +180,7 @@ __global__ void __launch_bounds__(NTHR, SPLIT ? 1 : 2) wgrad_tc_kernel(const Arg
                 float t = 0.f;
 #pragma unroll
                 for (int w = 0; w < 8; ++w) t += cs_red[w * 128 + tid];
-                atomicAdd(a.dbias + (long)(tm + tid) * a.bias_stride, t);
+                det_put(a.dbias + (long)(tm + tid) * a.bias_stride, a.bpart ? a.bpart + (long)blockIdx.y * a.M + tm + tid : nullptr, t);
             }
         }
         // ---------------- epilogue: TMEM -> C (fp32 atomics) ----------------
@@ -203,7 +204,12 @@ __global__ void __launch_bounds__(NTHR, SPLIT ? 1 : 2) wgrad_tc_kernel(const Arg
             asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
             if (m < a.M) {
                 float *dst = a.C + (long)m * a.ldc + hf * (N / 2) + cc;
-                if ((((uintptr_t)dst) & 15) == 0) {
+                if (a.part) {                           // N % 64 == 0: the slot row is 16-byte aligned
+                    float *pp = a.part + ((long)blockIdx.y * a.M + m) * N + hf * (N / 2) + cc;
+#pragma unroll
+                    for (int x = 0; x < 32; x += 4)
+                        det_put4(nullptr, pp + x, make_float4(__uint_as_float(v[x]), __uint_as_float(v[x + 1]), __uint_as_float(v[x + 2]), __uint_as_float(v[x + 3])));
+                } else if ((((uintptr_t)dst) & 15) == 0) {
 #pragma unroll
                     for (int x = 0; x < 32; x += 4)      // 128-bit vector reductions: 4x fewer L2 atomic operations
                         atomicAdd(reinterpret_cast<float4 *>(dst + x),
@@ -234,10 +240,20 @@ static int launch(const Args &a, cudaStream_t st, int sms) {
     Args k = a;
     k.rows_per_cta = ((a.rows + split - 1) / split + KT - 1) / KT * KT;
     split = (a.rows + k.rows_per_cta - 1) / k.rows_per_cta;
+    Partials pt(st);
+    k.part = k.bpart = nullptr;
+    if (det_on()) {
+        if (!(k.part = pt.take(split * a.M * N))) return BMP_EINVAL;
+        if (a.dbias && !(k.bpart = pt.take(split * a.M))) return BMP_EINVAL;
+    }
     cudaFuncSetAttribute(wgrad_tc_kernel<N, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     wgrad_tc_kernel<N, SPLIT><<<dim3(mtiles, (unsigned)split), NTHR, smem, st>>>(k);
     count_launch();
-    return check_launch("wgrad_tc_kernel");
+    int rc = check_launch("wgrad_tc_kernel");
+    if (rc || !k.part) return rc;
+    pt.add(a.C, a.ldc, a.M, N, k.part, (int)split, (long)a.M * N);
+    if (k.bpart) pt.add(a.dbias, a.bias_stride, a.M, 1, k.bpart, (int)split, a.M);
+    return pt.reduce("det_reduce_kernel (bmp_wgrad_tc)");
 }
 
 }  // namespace wtc

@@ -12,6 +12,7 @@
 // A) come from one extra N=16 UMMA per M tile against a block of ones.
 #include <cstdlib>
 #include "tc_common.cuh"
+#include "det.cuh"
 
 namespace bmp {
 namespace w2 {
@@ -121,12 +122,16 @@ __global__ void __launch_bounds__(NTH, 1) wgrad2_kernel(const __grid_constant__ 
         if (k0 < total) {
             const int q = warp, blk = q >> 1, r = (q & 1) * 32 + lane;     // TMEM lane 32q+lane = A column = C row
             const uint32_t t_lane = tmem + ((uint32_t)(32 * q) << 16);
+            // deterministic mode: this CTA's slot; target (m, blk, j) at ((2m + blk) NB + j) 4096 + 64 r, bias row r of (m, blk)
+            // after the 2 NMT NB targets.  C and C2 of a target get the same partial, so they share it.
+            float *slot = mm.part[ci] ? mm.part[ci] + k0 * mm.plen[ci] : nullptr;
             for (int m = 0; m < NMT; ++m) {
                 if (a.a_panel[m][blk] < 0) continue;
                 for (int j = 0; j < NB; ++j) {
                     float *d1 = a.C[m][blk][j] ? a.C[m][blk][j] + (long)r * a.ldc[j] : nullptr;
                     float *d2 = a.C2[m][blk][j] ? a.C2[m][blk][j] + (long)r * a.ldc2[j] : nullptr;
                     if (!d1 && !d2) continue;
+                    float *sp = slot ? slot + ((long)(2 * m + blk) * NB + j) * 4096 + 64 * r : nullptr;
                     for (int cc = 0; cc < 64; cc += 32) {
                         uint32_t v[32];
                         tc_ld32(t_lane + col_of(m) + j * 64 + cc, v);
@@ -134,8 +139,12 @@ __global__ void __launch_bounds__(NTH, 1) wgrad2_kernel(const __grid_constant__ 
 #pragma unroll
                         for (int x = 0; x < 32; x += 4) {     // 128-bit vector reductions (sm_90+): 4x fewer L2 atomic operations
                             const float4 f = make_float4(__uint_as_float(v[x]), __uint_as_float(v[x + 1]), __uint_as_float(v[x + 2]), __uint_as_float(v[x + 3]));
-                            if (d1) atomicAdd(reinterpret_cast<float4 *>(d1 + cc + x), f);
-                            if (d2) atomicAdd(reinterpret_cast<float4 *>(d2 + cc + x), f);
+                            if (sp) {
+                                det_put4(nullptr, sp + cc + x, f);
+                            } else {
+                                if (d1) atomicAdd(reinterpret_cast<float4 *>(d1 + cc + x), f);
+                                if (d2) atomicAdd(reinterpret_cast<float4 *>(d2 + cc + x), f);
+                            }
                         }
                     }
                 }
@@ -143,8 +152,12 @@ __global__ void __launch_bounds__(NTH, 1) wgrad2_kernel(const __grid_constant__ 
                     uint32_t w[16];
                     tc_ld16(t_lane + bias_col(m), w);
                     tc_wait_ld();
-                    if (a.bias[m][blk]) atomicAdd(a.bias[m][blk] + (long)r * a.bias_stride, __uint_as_float(w[0]));
-                    if (a.bias2[m][blk]) atomicAdd(a.bias2[m][blk] + (long)r * a.bias_stride, __uint_as_float(w[0]));
+                    if (slot) {
+                        det_put(nullptr, slot + (long)NMT * 2 * NB * 4096 + (2 * m + blk) * 64 + r, __uint_as_float(w[0]));
+                    } else {
+                        if (a.bias[m][blk]) atomicAdd(a.bias[m][blk] + (long)r * a.bias_stride, __uint_as_float(w[0]));
+                        if (a.bias2[m][blk]) atomicAdd(a.bias2[m][blk] + (long)r * a.bias_stride, __uint_as_float(w[0]));
+                    }
                 }
             }
         }
@@ -226,6 +239,12 @@ int bmp_wgrad_panels_multi(w2::Args *list, int n, void *stream) {
         m.cls[c] = list[c];
     }
     m.cta0[n] = used;
+    Partials pt((cudaStream_t)stream);
+    if (det_on())
+        for (int c = 0; c < n; ++c) {
+            m.plen[c] = (long)list[c].n_mt * 2 * list[c].nb * 4096 + list[c].n_mt * 2 * 64;
+            if (!(m.part[c] = pt.take((m.cta0[c + 1] - m.cta0[c]) * m.plen[c]))) return BMP_EINVAL;
+        }
     static bool attr = false;
     if (!attr) {
         cudaFuncSetAttribute(w2::wgrad2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, w2::STAGES * 8 * w2::BLK + w2::BLK + 256 + 1024);
@@ -234,7 +253,25 @@ int bmp_wgrad_panels_multi(w2::Args *list, int n, void *stream) {
     ProfScope prof(BMP_PROF_WGRAD, (cudaStream_t)stream);
     w2::wgrad2_kernel<<<(unsigned)used, w2::NTH, smem, (cudaStream_t)stream>>>(m);
     count_launch();
-    return check_launch("wgrad2_kernel");
+    int rc = check_launch("wgrad2_kernel");
+    if (rc || !det_on()) return rc;
+    for (int c = 0; c < n; ++c) {
+        const w2::Args &k = list[c];
+        const int parts = m.cta0[c + 1] - m.cta0[c], NB = k.nb;
+        for (int mt = 0; mt < k.n_mt; ++mt)
+            for (int blk = 0; blk < 2; ++blk) {
+                if (k.a_panel[mt][blk] < 0) continue;
+                for (int j = 0; j < NB; ++j) {
+                    const float *src = m.part[c] + ((long)(2 * mt + blk) * NB + j) * 4096;
+                    pt.add(k.C[mt][blk][j], k.ldc[j], 64, 64, src, parts, m.plen[c]);
+                    pt.add(k.C2[mt][blk][j], k.ldc2[j], 64, 64, src, parts, m.plen[c]);
+                }
+                const float *bsrc = m.part[c] + (long)k.n_mt * 2 * NB * 4096 + (2 * mt + blk) * 64;
+                pt.add(k.bias[mt][blk], k.bias_stride, 64, 1, bsrc, parts, m.plen[c]);
+                pt.add(k.bias2[mt][blk], k.bias_stride, 64, 1, bsrc, parts, m.plen[c]);
+            }
+    }
+    return pt.reduce("det_reduce_kernel (bmp_wgrad_panels)");
 }
 
 int bmp_wgrad_panels(w2::Args &k, void *stream) { return bmp_wgrad_panels_multi(&k, 1, stream); }

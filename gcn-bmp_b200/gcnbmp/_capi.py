@@ -42,7 +42,7 @@ class GgnnBwd(C.Structure):
         ("stateful", C.c_int * MAX_STEPS), ("Hs", fp), ("Ms", fp), ("RSs", fp), ("Gs", fp), ("Ps", fp), ("dHs", fp),
         ("d_msg_W", _A()), ("d_msg_b", _A()), ("d_gru", GRU * MAX_STEPS), ("d_state_in", fp),
         ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("stash2", fp), ("tc_images_ready", C.c_int), ("adj_u8", C.c_int),
-        ("mol_index", fp), ("dHs_every_step", C.c_int)]
+        ("mol_index", fp), ("dHs_every_step", C.c_int), ("det_scratch", fp), ("det_scratch_bytes", C.c_size_t)]
 
 
 class Pair(C.Structure):
@@ -75,7 +75,7 @@ class RelgcnBwd(C.Structure):
         ("ch", C.c_int * (MAX_STEPS + 1)), ("adj", fp), ("self_W", _A()), ("edge_W", _A()), ("Hs", fp),
         ("d_h_out", fp), ("Ds", fp), ("Ps", fp), ("d_h0", fp),
         ("d_self_W", _A()), ("d_self_b", _A()), ("d_edge_W", _A()), ("d_edge_b", _A()),
-        ("mode", C.c_int), ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("stash2", fp), ("tc_images_ready", C.c_int), ("adj_u8", C.c_int)]
+        ("mode", C.c_int), ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("stash2", fp), ("tc_images_ready", C.c_int), ("adj_u8", C.c_int), ("det_scratch", fp), ("det_scratch_bytes", C.c_size_t)]
 
 
 class ReadoutFwd(C.Structure):
@@ -88,7 +88,7 @@ class ReadoutBwd(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("mb", "n_atoms", "hidden", "out_dim", "variant", "act", "act_agg")] + [
         (n, fp) for n in ("h", "h0", "is_real_node", "W_i", "b_i", "W_j", "b_j", "g", "dg",
                           "DU", "DV", "dh", "dh0", "d_W_i", "d_b_i", "d_W_j", "d_b_j")] + [
-        ("mode", C.c_int), ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("tc_images_ready", C.c_int)]
+        ("mode", C.c_int), ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("tc_images_ready", C.c_int), ("det_scratch", fp), ("det_scratch_bytes", C.c_size_t)]
 
 
 _CO_PARAMS = ("W", "V1", "V2", "b", "lt_1", "lt_2", "wa_1", "wa_2", "W_j", "b_j")
@@ -105,7 +105,7 @@ class CoattnBwd(C.Structure):
         (n, fp) for n in ("atoms_1", "atoms_2") + _CO_PARAMS + ("d_compact_1", "d_compact_2", "R", "P1", "P2",
                                                              "DL1", "DL2", "d_atoms_1", "d_atoms_2")
         + tuple("d_" + p for p in _CO_PARAMS)] + [
-        ("mode", C.c_int), ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("tc_images_ready", C.c_int)]
+        ("mode", C.c_int), ("tc_workspace", fp), ("tc_workspace_bytes", C.c_size_t), ("tc_images_ready", C.c_int), ("det_scratch", fp), ("det_scratch_bytes", C.c_size_t)]
 
 
 def _load():
@@ -152,6 +152,11 @@ def _load():
         "bmp_bimpm_forward": [C.POINTER(Bimpm), vp],
         "bmp_bimpm_backward": [C.POINTER(Bimpm), vp],
         "bmp_embed_forward": [fp, fp, fp, i, i, i, vp],
+        "bmp_linear_backward_det": [fp, fp, fp, fp, fp, fp, fp, i, i, i, i, vp, vp, C.c_size_t],
+        "bmp_embed_backward_det": [fp, fp, fp, i, i, i, vp, vp, C.c_size_t],
+        "bmp_sigmoid_ce_det": [fp, fp, fp, fp, i, f, vp, vp, C.c_size_t],
+        "bmp_grad_hooks_det": [fp, fp, i, f, f, f, fp, vp, vp, C.c_size_t],
+        "bmp_bilinear_backward_det": [fp] * 14 + [i, i, i, i, vp, vp, C.c_size_t],
     }
     for name, args in sig.items():
         fn = getattr(lib, name)
@@ -169,6 +174,14 @@ def _load():
     lib.bmp_relgcn_tc_workspace_bytes.argtypes, lib.bmp_relgcn_tc_workspace_bytes.restype = [i, i], C.c_size_t
     lib.bmp_relgcn_x3_workspace_bytes.argtypes, lib.bmp_relgcn_x3_workspace_bytes.restype = [i] * 5, C.c_size_t
     lib.bmp_bimpm_workspace_bytes.argtypes, lib.bmp_bimpm_workspace_bytes.restype = [i, i, i, i, i], C.c_size_t
+    for name in ("bmp_ggnn_backward_det_bytes", "bmp_relgcn_backward_det_bytes", "bmp_readout_backward_det_bytes",
+                 "bmp_coattn_backward_det_bytes"):
+        getattr(lib, name).argtypes, getattr(lib, name).restype = [C.c_void_p], C.c_size_t
+    lib.bmp_linear_backward_det_bytes.argtypes, lib.bmp_linear_backward_det_bytes.restype = [i, i, i], C.c_size_t
+    lib.bmp_embed_backward_det_bytes.argtypes, lib.bmp_embed_backward_det_bytes.restype = [i, i, i], C.c_size_t
+    lib.bmp_sigmoid_ce_det_bytes.argtypes, lib.bmp_sigmoid_ce_det_bytes.restype = [i], C.c_size_t
+    lib.bmp_grad_hooks_det_bytes.argtypes, lib.bmp_grad_hooks_det_bytes.restype = [i], C.c_size_t
+    lib.bmp_bilinear_backward_det_bytes.argtypes, lib.bmp_bilinear_backward_det_bytes.restype = [i, i, i, i], C.c_size_t
     lib.bmp_last_error.restype = C.c_char_p
     lib.bmp_version.restype = C.c_int
     lib.bmp_device_check.restype = C.c_int
@@ -188,7 +201,11 @@ EXPORTS = ["bmp_ggnn_forward", "bmp_ggnn_backward", "bmp_embed_backward", "bmp_r
            "bmp_atoms_bcast_add_act_forward", "bmp_atoms_bcast_add_act_backward", "bmp_atoms_softmax_forward", "bmp_atoms_softmax_backward",
            "bmp_atoms_pool_forward", "bmp_atoms_pool_backward", "bmp_gin_aggregate", "bmp_nfp_gather", "bmp_embed_forward", "bmp_bimpm_forward", "bmp_bimpm_backward", "bmp_bimpm_workspace_bytes",
            "bmp_last_error", "bmp_version", "bmp_device_check", "bmp_launch_count", "bmp_reset_launch_count",
-           "bmp_profile_enable", "bmp_profile_read"]
+           "bmp_profile_enable", "bmp_profile_read",
+           "bmp_ggnn_backward_det_bytes", "bmp_relgcn_backward_det_bytes", "bmp_readout_backward_det_bytes", "bmp_coattn_backward_det_bytes",
+           "bmp_linear_backward_det", "bmp_linear_backward_det_bytes", "bmp_embed_backward_det", "bmp_embed_backward_det_bytes",
+           "bmp_sigmoid_ce_det", "bmp_sigmoid_ce_det_bytes", "bmp_grad_hooks_det", "bmp_grad_hooks_det_bytes",
+           "bmp_bilinear_backward_det", "bmp_bilinear_backward_det_bytes"]
 
 
 class BmpError(RuntimeError):

@@ -17,6 +17,75 @@ def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+# ---- deterministic mode (torch.use_deterministic_algorithms): fixed-order cross-CTA sums, include/gcnbmp.h
+def deterministic():
+    """True when torch's deterministic switch is on: the backward calls then pass deterministic scratch to the kernels."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def no_deterministic(op):
+    """Refuse (warn under warn_only) an op whose kernels have no fixed-order reduction, as torch does for its own ops."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = "gcnbmp: %s does not have a deterministic implementation, but torch.use_deterministic_algorithms(True) is set" % op
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        import warnings
+        warnings.warn(msg)
+        return
+    raise RuntimeError(msg)
+
+
+FILL_INTERNAL = False     # tests: fill internal buffers with NaN / 0xFF to show that no kernel reads what it has not written
+
+
+def empty_internal(shape, device, dtype):
+    """torch.empty for buffers the kernels write before they read (stashes, workspaces, scratch).  Under the deterministic
+    switch torch fills every torch.empty with NaN (torch.utils.deterministic.fill_uninitialized_memory); for the bf16 panel
+    stash that is a memset of tens of GB per micro-batch, so it is skipped here.  Tensors the user sees keep torch's fill."""
+    # a bare storage from the caching allocator is never filled; no process-wide setting is touched
+    shape = tuple(shape)
+    n = 1
+    for d in shape:
+        n *= int(d)
+    itemsize = torch.empty((), dtype=dtype).element_size()
+    st = torch.UntypedStorage(max(n, 1) * itemsize, device=device)
+    t = torch.empty(0, device=device, dtype=dtype).set_(st, 0, shape)
+    if FILL_INTERNAL:
+        t.fill_(float("nan") if t.is_floating_point() else 255)
+    return t
+
+
+def _det_attach(a, query, dev):
+    """Deterministic mode: give a backward struct its det_scratch (sized by the header's query); returns the buffer."""
+    if not deterministic():
+        return None
+    n = int(getattr(K.lib, query)(C.byref(a)))
+    if n == 0:      # a call with work always has a size: 0 means the query does not cover it
+        no_deterministic("%s for this shape" % query[:-len("_det_bytes")])
+        return None
+    buf = empty_internal((n,), dev, torch.uint8)
+    a.det_scratch, a.det_scratch_bytes = _p(buf), n
+    return buf
+
+
+def _det_call(name, size_args, args, dev):
+    """Plain entry point, or in deterministic mode its _det sibling with scratch appended."""
+    if not deterministic():
+        return K.check(getattr(K.lib, name)(*args))
+    n = int(getattr(K.lib, name + "_det_bytes")(*size_args))
+    if n == 0:      # nothing to sum (no rows), or a shape the deterministic path does not cover
+        if any(isinstance(v, int) and v <= 0 for v in size_args):
+            return K.check(getattr(K.lib, name)(*args))
+        no_deterministic("%s for this shape" % name)
+        return K.check(getattr(K.lib, name)(*args))
+    buf = empty_internal((n,), dev, torch.uint8)
+    K.check(getattr(K.lib, name + "_det")(*(tuple(args) + (_p(buf), n))))
+
+
+def embed_backward(ids, dh, gW, rows, H):
+    _det_call("bmp_embed_backward", (rows, H, gW.shape[0]), (_p(ids), _p(dh), _p(gW), rows, H, gW.shape[0], _stream()), gW.device)
+
+
 def adj_format(t):
     """Storage code of an adjacency tensor (include/gcnbmp.h `adj_u8`): 0 = fp32 (mb,E,N,N), 1 = bytes (mb,E,N,N),
     2 = bit-packed rows (mb,E,N,ceil(N/8)) as produced by `pack_adjacency`."""
@@ -121,12 +190,12 @@ def params_changed():
 def _tc_images(kind, nbytes, dev, params):
     """Workspace for the packed weight images of one launch kind -> (uint8 tensor, ready flag)."""
     if not _WEIGHT_CACHE:
-        return torch.empty((nbytes,), device=dev, dtype=torch.uint8), 0
+        return empty_internal((nbytes,), dev, torch.uint8), 0
     key = (kind, nbytes, str(dev)) + tuple(p.data_ptr() if p is not None else 0 for p in params)
     ent = _IMAGES.get(key)
     if ent is not None and ent[1] == _PARAM_EPOCH:
         return ent[0], 1
-    ws = torch.empty((nbytes,), device=dev, dtype=torch.uint8)
+    ws = empty_internal((nbytes,), dev, torch.uint8)
     # the entry keeps the keyed tensors alive: while it exists the allocator cannot hand one of those addresses to a
     # different (derived, temporary) tensor, so an address match always means "the same values since params_changed()"
     _IMAGES[key] = (ws, _PARAM_EPOCH, tuple(params))
@@ -243,7 +312,7 @@ class GGNNEncode(torch.autograd.Function):
             # bf16 panel stash: the tape keeps operand panels + gate values; only [h_0, h_T] (every h_t with keep_steps) go
             # back as fp32
             out = torch.empty((T + 1 if keep_steps else 2, mb, N, H), device=dev, dtype=torch.float32)
-            stash2 = torch.empty((int(K.lib.bmp_ggnn_stash2_bytes(mb, H, T)),), device=dev, dtype=torch.uint8)
+            stash2 = empty_internal((int(K.lib.bmp_ggnn_stash2_bytes(mb, H, T)),), dev, torch.uint8)
             if keep_steps:
                 a.Hs = _p(out)
             else:
@@ -259,9 +328,9 @@ class GGNNEncode(torch.autograd.Function):
             x3ws = _x3_workspace(a, mb, N, H, E, T, dev, params, not want_stash)
         if want_stash:
             Hs = torch.empty((T + 1, mb, N, H), device=dev, dtype=torch.float32)
-            Ms = torch.empty((T, rows, H), device=dev, dtype=torch.float32)
-            Gs = torch.empty((T, rows, 3 * H), device=dev, dtype=torch.float32)
-            RSs = torch.empty((T, rows, H), device=dev, dtype=torch.float32)
+            Ms = empty_internal((T, rows, H), dev, torch.float32)
+            Gs = empty_internal((T, rows, 3 * H), dev, torch.float32)
+            RSs = empty_internal((T, rows, H), dev, torch.float32)
             a.Hs, a.Ms, a.Gs, a.RSs = _p(Hs), _p(Ms), _p(Gs), _p(RSs)
             K.check(K.lib.bmp_ggnn_forward(C.byref(a), _stream()))
             ctx.save_for_backward(x, adj, state_in, Hs, Ms, Gs, RSs, *params)
@@ -288,7 +357,7 @@ class GGNNEncode(torch.autograd.Function):
         rows = mb * N
         dHs = dHs.contiguous().clone()
         grads, rets = _grad_targets(params)
-        Ps = torch.empty((T, rows, E * H), device=adj.device, dtype=torch.float32) if stash2 is None else None
+        Ps = empty_internal((T, rows, E * H), adj.device, torch.float32) if stash2 is None else None
         a = K.GgnnBwd()
         a.mb, a.n_atoms, a.hidden, a.n_edge, a.n_steps, a.mode = mb, N, H, E, T, mode
         mol_index = ctx.mol_index
@@ -311,11 +380,12 @@ class GGNNEncode(torch.autograd.Function):
         if mode == K.MODE_F32 and getattr(ctx, "x3", False):
             # same kind and size as the forward's: the images packed there (same parameter values) are found ready
             _x3_workspace(a, mb, N, H, E, T, adj.device, params, False)
+        det = _det_attach(a, "bmp_ggnn_backward_det_bytes", adj.device)      # noqa: F841
         K.check(K.lib.bmp_ggnn_backward(C.byref(a), _stream()))
         dx = None
         if is_ids:
             ids = x if mol_index is None else x.index_select(0, mol_index.long()).contiguous()      # (mb, N) int32: tiny
-            K.check(K.lib.bmp_embed_backward(_p(ids), _p(dHs[0]), _p(grads[0]), rows, H, grads[0].shape[0], _stream()))
+            embed_backward(ids, dHs[0], grads[0], rows, H)
         else:
             dx = dHs[0]
             rets[0] = None
@@ -372,7 +442,7 @@ class RelGCNEncode(torch.autograd.Function):
             ws, a.tc_images_ready = _tc_images("relgcn_fwd", nbytes, adj.device, params)
             a.mode, a.tc_workspace, a.tc_workspace_bytes = K.MODE_BF16, _p(ws), nbytes
             if want_stash:       # bf16 panel tape (same layout as the GGNN encoder's)
-                Hs = torch.empty((int(K.lib.bmp_ggnn_stash2_bytes(mb, ch[0], L)),), device=adj.device, dtype=torch.uint8)
+                Hs = empty_internal((int(K.lib.bmp_ggnn_stash2_bytes(mb, ch[0], L)),), adj.device, torch.uint8)
                 a.stash2 = _p(Hs)
         elif want_stash:
             Hs = torch.empty((rows * sum(ch),), device=adj.device, dtype=torch.float32)
@@ -420,10 +490,11 @@ class RelGCNEncode(torch.autograd.Function):
             a.self_W[l], a.edge_W[l] = _p(Ws), _p(We)
             gWs, gbs, gWe, gbe = grads[1 + 4 * l: 5 + 4 * l]
             a.d_self_W[l], a.d_self_b[l], a.d_edge_W[l], a.d_edge_b[l] = _p(gWs), _p(gbs), _p(gWe), _p(gbe)
+        det = _det_attach(a, "bmp_relgcn_backward_det_bytes", dev)      # noqa: F841
         K.check(K.lib.bmp_relgcn_backward(C.byref(a), _stream()))
         dx = None
         if is_ids:
-            K.check(K.lib.bmp_embed_backward(_p(x), _p(d_h0), _p(grads[0]), rows, ch[0], grads[0].shape[0], _stream()))
+            embed_backward(x, d_h0, grads[0], rows, ch[0])
         else:
             dx = d_h0
             rets[0] = None
@@ -555,6 +626,7 @@ class Readout(torch.autograd.Function):
         a.dh, a.dh0 = _p(dh), _p(dh0)
         a.d_W_i, a.d_b_i, a.d_W_j, a.d_b_j = _p(gWi), _p(gbi), _p(gWj), _p(gbj)
         ws = _readout_ws(a, mode, H, O, variant, dev, (W_i, W_j))
+        det = _det_attach(a, "bmp_readout_backward_det_bytes", dev)      # noqa: F841
         K.check(K.lib.bmp_readout_backward(C.byref(a), _stream()))
         return (dh, dh0, None, None, None, None) + tuple(rets) + (None,)
 
@@ -633,6 +705,7 @@ class Coattention(torch.autograd.Function):
         a.d_atoms_1, a.d_atoms_2 = _p(da1), _p(da2)
         a.mode = mode
         ws = _coattn_workspace(a, mode, H, dev, ps)
+        det = _det_attach(a, "bmp_coattn_backward_det_bytes", dev)      # noqa: F841
         K.check(K.lib.bmp_coattn_backward(C.byref(a), _stream()))
         return (da1, da2, None, None) + tuple(rets) + (None,)
 
@@ -713,8 +786,9 @@ class Bilinear(torch.autograd.Function):
         du = torch.empty_like(u)
         de1, de2 = torch.empty_like(e1), torch.empty_like(e2)
         (dW, dV1, dV2, db), rets = _grad_targets([W, V1, V2, b])
-        K.check(K.lib.bmp_bilinear_backward(_p(e1), _p(e2), _p(W), _p(V1), _p(V2), _p(u), _p(dy), _p(du), _p(de1), _p(de2),
-                                            _p(dW), _p(dV1), _p(dV2), _p(db), mb, L, R, Ko, _stream()))
+        _det_call("bmp_bilinear_backward", (mb, L, R, Ko),
+                  (_p(e1), _p(e2), _p(W), _p(V1), _p(V2), _p(u), _p(dy), _p(du), _p(de1), _p(de2),
+                   _p(dW), _p(dV1), _p(dV2), _p(db), mb, L, R, Ko, _stream()), e1.device)
         return (de1, de2) + tuple(rets)
 
 
@@ -860,6 +934,7 @@ class BiMPMMatch(torch.autograd.Function):
         (gm, ga, gx), rets = _grad_targets([Wm, Wa, Wx])
         a.d_out_1, a.d_out_2, a.d_atoms_1, a.d_atoms_2 = _p(g1), _p(g2), _p(d1), _p(d2)
         a.d_max_pooling_W, a.d_att_mean_W, a.d_att_max_W = _p(gm), _p(ga), _p(gx)
+        no_deterministic("BiMPM (BiMPMMatch backward)")
         K.check(K.lib.bmp_bimpm_backward(C.byref(a), _stream()))
         return (d1, d2) + tuple(rets)
 
@@ -881,7 +956,7 @@ class EmbedID(torch.autograd.Function):
     def backward(ctx, d_out):
         ids, W = ctx.saved_tensors
         (gW,), rets = _grad_targets([W])
-        K.check(K.lib.bmp_embed_backward(_p(ids), _p(_f32(d_out)), _p(gW), ids.numel(), W.shape[1], W.shape[0], _stream()))
+        embed_backward(ids, _f32(d_out), gW, ids.numel(), W.shape[1])
         return None, rets[0]
 
 
@@ -935,8 +1010,8 @@ class Linear(torch.autograd.Function):
         dy = dy.contiguous().float().clone()
         dx = torch.empty_like(x)
         (dW, db), rets = _grad_targets([W, b])
-        K.check(K.lib.bmp_linear_backward(_p(x), _p(W), _p(y), _p(dy), _p(dx), _p(dW), _p(db),
-                                          rows, in_dim, out_dim, ctx.act, _stream()))
+        _det_call("bmp_linear_backward", (rows, in_dim, out_dim),
+                  (_p(x), _p(W), _p(y), _p(dy), _p(dx), _p(dW), _p(db), rows, in_dim, out_dim, ctx.act, _stream()), x.device)
         return dx, rets[0], rets[1], None
 
 
@@ -953,7 +1028,7 @@ class SigmoidCrossEntropy(torch.autograd.Function):
             count = float(max(int((t != -1).sum().item()), 1))
         loss = torch.zeros((), device=x.device, dtype=torch.float32)
         dx = torch.empty_like(x)
-        K.check(K.lib.bmp_sigmoid_ce(_p(x), _p(t), _p(loss), _p(dx), x.numel(), float(count), _stream()))
+        _det_call("bmp_sigmoid_ce", (x.numel(),), (_p(x), _p(t), _p(loss), _p(dx), x.numel(), float(count), _stream()), x.device)
         ctx.save_for_backward(dx)
         return loss
 

@@ -27,6 +27,7 @@ def supported(model):
 def pair_forward_backward(model, atoms_1, adj_1, atoms_2, adj_2, labels, count=None):
     """One fwd+bwd of the pair model in a single library call.  Adds every parameter gradient into `p.grad` (created as zeros
     when absent), returns (loss, logits).  `count`: what the loss mean divides by (default: this batch's labels != -1)."""
+    Fn.no_deterministic("gcnbmp.fused.pair_forward_backward (the one-call step reduces with atomics)")
     if not supported(model):
         raise ValueError("gcnbmp.fused: the one-call step covers GGNNMono + fine / pooling co-attention + HolE(hidden_dims=())")
     enc, attn, head = model.graph_conv, model.attn, model.mlp

@@ -52,9 +52,10 @@ class GradientHooks(object):
 
     def apply(self):
         p = lambda t: C.c_void_p(t.data_ptr())
-        K.check(K.lib.bmp_grad_hooks(p(self.gflat), p(self.flat), self.gflat.numel(), max(self.max_norm, 0.0),
-                                     max(self.l2_rate, 0.0), max(self.l1_rate, 0.0), p(self.norm_ws),
-                                     C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+        n = self.gflat.numel()
+        Fn._det_call("bmp_grad_hooks", (n,), (p(self.gflat), p(self.flat), n, max(self.max_norm, 0.0), max(self.l2_rate, 0.0),
+                                             max(self.l1_rate, 0.0), p(self.norm_ws), C.c_void_p(torch.cuda.current_stream().cuda_stream)),
+                    self.flat.device)
 
 
 class ExponentialShift(object):

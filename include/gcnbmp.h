@@ -158,6 +158,9 @@ typedef struct {
     int    dHs_every_step;       /* BMP_MODE_BF16 only.  0: dHs has TWO slices, [0] = gradient w.r.t. h_0, [1] = gradient
                                     w.r.t. h_T.  Nonzero: dHs (T+1, mb*N, H) as in BMP_MODE_F32, an external gradient for
                                     every h_t.  Either way dHs[0] holds the total gradient w.r.t. h_0 on exit    */
+    void  *det_scratch;          /* deterministic mode (see "Deterministic reductions" below): NULL = fp32 atomics, today's path
+                                   bit for bit; else >= bmp_ggnn_backward_det_bytes(this struct) bytes of device scratch, else BMP_EINVAL */
+    size_t det_scratch_bytes;
 } bmp_ggnn_bwd_t;
 
 int bmp_ggnn_backward(const bmp_ggnn_bwd_t *a, void *stream);
@@ -229,6 +232,9 @@ typedef struct {
     int    adj_u8;               /* BMP_MODE_BF16 only, storage of `adj`: 0 = fp32 (mb,E,N,N) as the reference; 1 = the same
                                    array as bytes (exact for 0/1 bonds; 1/4 of the PCIe / HBM traffic); 2 = bit-packed rows
                                    (mb,E,N,ceil(N/8)), bit j&7 of byte j>>3 = adj[i][j] (numpy.packbits little; 1/32)  */
+    void  *det_scratch;          /* deterministic mode (see "Deterministic reductions" below): NULL = fp32 atomics, today's path
+                                   bit for bit; else >= bmp_relgcn_backward_det_bytes(this struct) bytes of device scratch, else BMP_EINVAL */
+    size_t det_scratch_bytes;
 } bmp_relgcn_bwd_t;
 
 int bmp_relgcn_backward(const bmp_relgcn_bwd_t *a, void *stream);
@@ -269,6 +275,9 @@ typedef struct {
     size_t tc_workspace_bytes;
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
+    void  *det_scratch;          /* deterministic mode (see "Deterministic reductions" below): NULL = fp32 atomics, today's path
+                                   bit for bit; else >= bmp_readout_backward_det_bytes(this struct) bytes of device scratch, else BMP_EINVAL */
+    size_t det_scratch_bytes;
 } bmp_readout_bwd_t;
 
 int bmp_readout_backward(const bmp_readout_bwd_t *a, void *stream);
@@ -312,6 +321,9 @@ typedef struct {
     size_t tc_workspace_bytes;
     int    tc_images_ready;      /* nonzero: tc_workspace already holds the images packed by an earlier call of the same
                                    kind with exactly these parameter values -- skip packing             */
+    void  *det_scratch;          /* deterministic mode (see "Deterministic reductions" below): NULL = fp32 atomics, today's path
+                                   bit for bit; else >= bmp_coattn_backward_det_bytes(this struct) bytes of device scratch, else BMP_EINVAL */
+    size_t det_scratch_bytes;
 } bmp_coattn_bwd_t;
 
 int bmp_coattn_backward(const bmp_coattn_bwd_t *a, void *stream);
@@ -404,6 +416,8 @@ typedef struct {
 } bmp_pair_t;
 
 size_t bmp_pair_workspace_bytes(int mb, int n1, int n2, int hidden, int out_dim, int head, int n_classes, int n_steps, int mode);
+/* Always finishes its sums with fp32 atomics: there is no deterministic variant of the one-call step (see "Deterministic
+ * reductions"); compose the per-layer entry points with det_scratch for bitwise-reproducible training.                   */
 int bmp_pair_forward_backward(const bmp_pair_t *a, void *stream);
 
 /* ---- remaining link-prediction heads (SURVEY 8 f-4) --------------------------------
@@ -452,6 +466,42 @@ int bmp_gin_aggregate(const float *adj, const float *h, float *out, int mb, int 
  * (g += l2 * p), Lasso(l1_rate) (g += l1 * sign(p)).  norm_ws: one float of device scratch (needed when clipping).     */
 int bmp_grad_hooks(float *grad, const float *param, int n, float clip_threshold, float l2_rate, float l1_rate,
                    float *norm_ws, void *stream);
+
+/* ---- Deterministic reductions (bmp_version() >= 101) ---------------------------------------------------------------
+ * By default every cross-CTA sum -- parameter gradients, the loss sum, the clipping norm -- ends in fp32 atomics, so two
+ * identical calls can differ in the last bits.  Given device scratch, the same kernels write one partial per CTA into it
+ * instead and one shared reduce kernel adds the partials into the destination in CTA order, in fp32:
+ *   dst[i] += ((p_0 + p_1) + ...) + p_{P-1}.
+ * Same shapes, mode and device model then give the same bits run after run.  Nothing is promised across devices with a
+ * different SM count.  Struct entry points take `det_scratch` / `det_scratch_bytes` (NULL = atomics) sized by the queries
+ * below, which read the filled-in struct (host-only; 0 = nothing to cover).  Plain entry points have `_det` siblings with
+ * (scratch, scratch_bytes) appended and their own size queries.  Relaxations and limits:
+ *   - bmp_embed_backward_det runs a table wider than the shared-memory owner kernel (more than 25600 floats) as column tiles
+ *     of that kernel instead of the default large-table kernel, whose shared-memory atomics have no fixed order.
+ *   - A size query covers every call the entry point makes for that struct: it is the largest need over them.
+ *   - bmp_pair_forward_backward (the one-call step) and bmp_bimpm_backward have no deterministic path; they stay on atomics.
+ *   - The scratch is only touched between the first kernel of a call and its last reduce: it may be reused by the next call
+ *     on the same stream.                                                                                                   */
+size_t bmp_ggnn_backward_det_bytes(const bmp_ggnn_bwd_t *a);
+size_t bmp_relgcn_backward_det_bytes(const bmp_relgcn_bwd_t *a);
+size_t bmp_readout_backward_det_bytes(const bmp_readout_bwd_t *a);
+size_t bmp_coattn_backward_det_bytes(const bmp_coattn_bwd_t *a);
+size_t bmp_linear_backward_det_bytes(int rows, int in_dim, int out_dim);
+int bmp_linear_backward_det(const float *x, const float *W, const float *y, float *dy, float *dx, float *dW, float *db,
+                            int rows, int in_dim, int out_dim, int act, void *stream, void *scratch, size_t scratch_bytes);
+size_t bmp_embed_backward_det_bytes(int rows, int hidden, int n_atom_types);
+int bmp_embed_backward_det(const int32_t *atoms, const float *dh, float *d_embed_W, int rows, int hidden, int n_atom_types,
+                           void *stream, void *scratch, size_t scratch_bytes);
+size_t bmp_sigmoid_ce_det_bytes(int n);
+int bmp_sigmoid_ce_det(const float *logits, const int32_t *labels, float *loss_sum, float *d_logits, int n, float count,
+                       void *stream, void *scratch, size_t scratch_bytes);
+size_t bmp_bilinear_backward_det_bytes(int rows, int left, int right, int out);
+int bmp_bilinear_backward_det(const float *e1, const float *e2, const float *W, const float *V1, const float *V2, const float *u,
+                              const float *dy, float *du, float *de1, float *de2, float *dW, float *dV1, float *dV2, float *db,
+                              int rows, int left, int right, int out, void *stream, void *scratch, size_t scratch_bytes);
+size_t bmp_grad_hooks_det_bytes(int n);
+int bmp_grad_hooks_det(float *grad, const float *param, int n, float clip_threshold, float l2_rate, float l1_rate,
+                       float *norm_ws, void *stream, void *scratch, size_t scratch_bytes);
 
 /* ---- housekeeping ------------------------------------------------------------ */
 const char *bmp_last_error(void);
